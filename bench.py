@@ -3,6 +3,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo's CUDA path
     python bench.py --impl reference [--gpus N] --steps K ...    # the reference's own CPU path
     torchrun --nproc-per-node N bench.py --gpus N ...            # one rank per GPU (weak scaling)
+    python bench.py --steps K --warmup W --dump-outputs DIR      # also writes the last timed step's outputs as .npy
 
 Workload: BASELINE.json configs[3] -- 2 snakes on 19x19, classic rules, 1M envs sharded over 8
 GPUs, i.e. 131072 envs per GPU (weak scaling), uniform random actions from the Philox action
@@ -299,6 +300,29 @@ def rank_parity(env, rank, steps=16, n_blocks=4, count=256):
     return bool(ok), sum(c for _, c, _ in bo.blocks), steps
 
 
+DUMP_OBS_ENVS = 4096   # 4096 x 21 x 21 x 6 float32 = 43 MB of observations: with the [N] arrays the dump stays under 64 MB
+
+
+def dump_obs_envs(n):
+    """The envs whose observations the dump holds: DUMP_OBS_ENVS of n drawn with a fixed seed, in ascending order."""
+    import numpy as np
+    return np.sort(np.random.RandomState(0).choice(n, min(DUMP_OBS_ENVS, n), replace=False))
+
+
+def dump_outputs(path, env):
+    """Writes what the last timed step handed its caller as float32 .npy files in `path`: reward, done, num_snakes and
+    Monitor's episode return and length (where done; 0 elsewhere) of every env, and the observations of the envs
+    dump_obs_envs picks.  Two builds run with the same arguments can then be compared array by array."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    idx = dump_obs_envs(env.N)
+    arrays = {"obs": env.obs[torch.as_tensor(idx, device=env.device)], "reward": env.rewards, "done": env._done_u8,
+              "num_snakes": env.num_alive, "episode_return": env.episode_return, "episode_length": env.episode_len}
+    for name, x in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), x.cpu().numpy().astype(np.float32))
+
+
 def time_config(sb, torch, dev, peak, name, N, kw, steps, n_batches=16, warm=40):
     """One secondary configuration through the graph path: us per step, fraction of the HBM roofline, mean body length."""
     env = sb.SnakeVecEnv(N, seed=0, device=dev.index, **kw)
@@ -404,6 +428,8 @@ def run_ours(args):
     launches = env.launch_count() - l0
     ms = max_over_ranks(e0.elapsed_time(e1))
     stats_local = env.stats(reduce=False)
+    if args.dump_outputs and rank == 0:   # before anything else steps the env
+        dump_outputs(args.dump_outputs, env)
     collective = None
     if use_comm:
         barrier()                   # every rank has finished its K steps: all pushes / all-reduces have landed
@@ -668,7 +694,11 @@ def main():
     ap.add_argument("--no-collective", action="store_true", help="A/B: multi-GPU run without the in-loop all-reduce")
     ap.add_argument("--comm", default="p2p", choices=["p2p", "nccl"],
                     help="form of the per-step statistics reduction: fused peer-memory pushes (default) or ncclAllReduce on a side stream")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0's envs) into DIR as float32 .npy files")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to this repo's CUDA path only")
     if args.impl == "reference":
         run_reference(args)
         return
