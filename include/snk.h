@@ -83,7 +83,10 @@ typedef struct snk_config {
  * SubprocVecEnv.step_wait (subproc_vec_env.py:57-61) and Monitor's info['episode']
  * (baselines/bench/monitor.py:62-76). */
 typedef struct snk_buffers {
-  uint8_t* d_obs;          /* [N][H][W][3K] uint8 (H = W = V native, 84 atari); may be redirected */
+  uint8_t* d_obs;          /* [N][H][W][3K] uint8 (H = W = V native, 84 atari); may be redirected.  READ-ONLY for
+                            * callers: the step writes only the bytes that changed into the handle's own buffer (the
+                            * sectors a step can change, when the handle knows the buffer still shows the previous
+                            * frame), so anything written into it between steps may survive them.  Copy it instead. */
   float* d_reward;         /* [N]    reward of snake 0 (the reference's scalar reward) */
   float* d_reward_all;     /* [N][S] extension: per-snake reward */
   uint8_t* d_done;         /* [N]    1 = episode ended this step (obs is then the reset obs if auto_reset) */

@@ -120,7 +120,7 @@ static int gcd(int a, int b) { return b ? gcd(b, a % b) : a; }
 // ---- experiment switches.  ONE string of comma-separated key=value pairs, given explicitly to snk_create_ex or, for
 // snk_create, read from the single environment variable SNK_DEBUG.  None changes results (all are parity-tested); an
 // unset / empty string is the production configuration.  Keys: force_kernel=lane|tile|rows|dense, lane=fused|ws|split,
-// store=stg, restore=tma, l2=<bits>, pdl=0, restore_thr=<n>, logic_warps=<n>, rows_kb=<n>, rows_block=<n>, extra_smem=<bytes>.
+// store=stg, restore=tma, l2=<bits>, pdl=0, delta=0|1, restore_thr=<n>, logic_warps=<n>, rows_kb=<n>, rows_block=<n>, extra_smem=<bytes>.
 static bool dbg_get(const std::string& opts, const char* key, std::string* out) {
   size_t pos = 0;
   const size_t klen = strlen(key);
@@ -522,6 +522,19 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   if (cfg->rules != SNK_RULES_CLASSIC && p.family == 1) TRY(dev_alloc(h, &p.gbits, (size_t)N * p.GBW, true));
   TRY(dev_alloc(h, &h->d_obs_own, (size_t)N * p.E, true));
   p.obs = h->d_obs_own;
+  if (p.family == 1) {
+    // frame_ok[e] = 1 <=> d_obs_own holds exactly the image of env e's record (cleared here and by snk_load_state, written
+    // by every lane-family kernel that writes a record).  With it the fused kernel's classic step stores only the sectors
+    // a step changes; delta=0 always stores whole images.  Sectors never cross env boundaries because the first and last
+    // (V+1)*C bytes of an env image are border (needs >= 32) and the buffer is 32-byte aligned.  Default: 32-env batches
+    // only.  A small shard (smaller batches, §4.10 of DESIGN.md) is bound by one warp's serial chain, not by the stream,
+    // and there the sector loop is longer than one bulk-store issue (2x10x10, 4 096 envs on B200: 10.39 vs 9.86 us per
+    // step); the headline shard gains 64.5 -> 52.7 us.  delta=0 / delta=1 turn it off / on regardless.
+    TRY(dev_alloc(h, &p.frame_ok, (size_t)N, true));
+    const int dm = dbg_int(dbg, "delta", -1);
+    p.delta = cfg->rules == SNK_RULES_CLASSIC && (V + 1) * p.C >= 32 && ((uintptr_t)h->d_obs_own & 31) == 0 &&
+              (dm < 0 ? p.EPW == 32 : dm != 0);
+  }
   h->d_obs84_own = nullptr;
   h->obs_out_env_bytes = (size_t)p.E;
   h->d_obs_user = h->d_obs_own;
@@ -648,6 +661,8 @@ static int launch(snk_handle* h, int mode, const int8_t* d_actions, const uint8_
     }
   }
   p.mode = mode; p.actions = d_actions; p.mask = d_mask;
+  p.frame_own = p.obs == h->d_obs_own;  // the step kernels write every env's image into p.obs
+  p.delta = p.delta && p.frame_own && mode == MODE_STEP;
   p.tape_vals = h->d_tape_vals; p.tape_bounds = h->d_tape_bounds; p.tape_off = h->d_tape_off;
   if (p.rng_mode == SNK_RNG_TAPE && !p.tape_vals) return fail(SNK_EINVAL, "rng_mode is TAPE but no tape was set");
   const bool reduce = h->comm && h->reduce_enabled && mode == MODE_STEP;   // NCCL form: snapshot + all-reduce on the side stream
@@ -1119,6 +1134,7 @@ extern "C" int snk_load_state(snk_handle* h, const void* h_src, size_t bytes) {
   CUDA_TRY(cudaDeviceSynchronize());
   CUDA_TRY(cudaMemcpy(h->d_blob, h_src, h->lay.total_bytes, cudaMemcpyHostToDevice));
   h->obs_current = nullptr;
+  if (h->p.frame_ok) CUDA_TRY(cudaMemset(h->p.frame_ok, 0, (size_t)h->p.N));  // the own buffer no longer shows the records
   CUDA_TRY(snk_launch_load(h->p, h->d_blob, h->lay, 0));
   h->launches++;
   CUDA_TRY(cudaDeviceSynchronize());

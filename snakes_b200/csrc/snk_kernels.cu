@@ -674,6 +674,7 @@ __global__ void __launch_bounds__(160, 5) k_step_lane_ws(const Params p) {
 
 // k_step_lane: see snk_lane.cuh.  A warp is an independent worker: 32 envs of logic (one per lane),
 // then 32/TE rounds of paint -> TMA bulk store -> un-paint on its private image.  No __syncthreads.
+// With Params::delta an image whose envs all qualify (delta_eligible) goes out as its changed sectors instead (delta_store).
 template <int S, int RULES, int K>
 __global__ void __launch_bounds__(64) k_step_lane(const Params p) {
   extern __shared__ __align__(128) u8 smem[];
@@ -702,6 +703,8 @@ __global__ void __launch_bounds__(64) k_step_lane(const Params p) {
   const long long n_batches = (p.N + EPW - 1) / EPW;
   const long long stride = (long long)gridDim.x * wpc;
   const bool stepping = p.mode == MODE_STEP;
+  const bool delta = RULES == SNK_RULES_CLASSIC && stepping && p.delta;
+  const u32 tile_mask = TE == 32 ? ~0u : (1u << TE) - 1u;
   long long b = (long long)blockIdx.x * wpc + warp;
   LaneRaw<S> raw;
   // Programmatic dependent launch: everything above (shared-memory carve-up, mbarrier, border image
@@ -737,6 +740,13 @@ __global__ void __launch_bounds__(64) k_step_lane(const Params p) {
       }
       if (valid && p.mode != MODE_OBSERVE) lane_store<S>(p, e, env);
     }
+    // delta store: the old state's paint items, and the lanes whose env must go out as a whole image
+    DeltaOld<S> old;
+    u32 whole = ~0u;
+    if (delta) {
+      old = delta_old<S>(raw);
+      whole = __ballot_sync(FULL, valid && !delta_eligible<S>(old, raw.frame, env));
+    }
     // records + actions of this warp's NEXT batch: in flight while the current one is painted
     if (b + stride < n_batches && lane < EPW && (b + stride) * EPW + lane < p.N) raw = lane_fetch<S>(p, (b + stride) * EPW + lane, stepping);
     const bool restore = lane_wants_restore<S>(p, env.len, LPE);  // one decision for the batch's 32/TE images
@@ -755,7 +765,12 @@ __global__ void __launch_bounds__(64) k_step_lane(const Params p) {
 #ifdef SNK_PHASE_TIMING
       { const long long t1 = clock64(); tB += t1 - t0; t0 = t1; }
 #endif
-      store_image(p, tile, tile_bytes, e0, lane);
+      if (((whole >> (q * TE)) & tile_mask) == 0) {
+        const DeltaOld<S> po = delta_old_from_lane<S>(old, q * TE + slot);
+        delta_store<S, K>(p, pe, po, slot, sub, LPE, tile, (int)min((long long)TE, p.N - e0) * E, e0);
+      } else {
+        store_image(p, tile, tile_bytes, e0, lane);
+      }
       __syncwarp();
 #ifdef SNK_PHASE_TIMING
       { const long long t1 = clock64(); tC += t1 - t0; t0 = t1; }

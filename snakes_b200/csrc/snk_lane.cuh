@@ -88,6 +88,13 @@ __device__ __forceinline__ u32 lane_draw(const Params& p, long long e, LaneEnv<S
   return __umulhi(x, n);
 }
 
+// Displacement from segment 0 to segment r (0..16) of the codes in word w: V * (#(+V) - #(-V)) + (#(+1) - #(-1)).
+__device__ __forceinline__ int codes_disp(u32 w, int V, int r) {
+  const u32 m = r >= 16 ? 0x55555555u : ((1u << (2 * r)) - 1u) & 0x55555555u;
+  const u32 lo = w & m, hi = (w >> 1) & m;
+  return V * (r - __popc(lo | hi) - __popc(hi & ~lo)) + (__popc(lo & ~hi) - __popc(lo & hi));
+}
+
 // Position of segment i without walking: the 2-bit codes before it are counted per direction with
 // popcounts, pid_i = head - V*(#(+V) - #(-V)) - (#(+1) - #(-1)).
 template <bool AT_L2 = false>  // AT_L2: the chain words were written by another lane a moment ago -- read them at the L2
@@ -101,12 +108,7 @@ __device__ __forceinline__ int chain_pos(int head, u32 c0, const u32* __restrict
     n1 += __popc(lo & ~hi) - __popc(lo & hi);
     w = AT_L2 ? __ldcg(ch + k + 1) : ch[k + 1];
   }
-  const int r = i - 16 * k;  // 0..16 codes of word k
-  const u32 m = r >= 16 ? 0x55555555u : ((1u << (2 * r)) - 1u) & 0x55555555u;
-  const u32 lo = w & m, hi = (w >> 1) & m;
-  nV += r - __popc(lo | hi) - __popc(hi & ~lo);
-  n1 += __popc(lo & ~hi) - __popc(lo & hi);
-  return head - V * nV - n1;
+  return head - V * nV - n1 - codes_disp(w, V, i - 16 * k);
 }
 
 // chain_pos for a lane that visits segments in increasing order (i, i + LPE, ...): the whole words before the current
@@ -122,10 +124,7 @@ struct ChainCursor {
       w = ch[k + 1];
       ++k;
     }
-    const int r = i - 16 * k;  // 0..16 codes of word k
-    const u32 m = r >= 16 ? 0x55555555u : ((1u << (2 * r)) - 1u) & 0x55555555u;
-    const u32 lo = w & m, hi = (w >> 1) & m;
-    return base - V * (r - __popc(lo | hi) - __popc(hi & ~lo)) - (__popc(lo & ~hi) - __popc(lo & hi));
+    return base - codes_disp(w, V, i - 16 * k);  // 0..16 codes of word k
   }
 };
 
@@ -568,7 +567,8 @@ __device__ __forceinline__ void lane_step(const Params& p, long long e, bool val
 template <int S>
 struct LaneRaw {
   uint4 v[LaneRec<S>::RW / 4];
-  u32 act;  // S int8 actions, little-endian
+  u32 act;     // S int8 actions, little-endian
+  bool frame;  // frame_ok: the own observation buffer holds this record's image
 };
 
 template <int S>
@@ -587,6 +587,7 @@ __device__ __forceinline__ LaneRaw<S> lane_fetch(const Params& p, long long e, b
 #pragma unroll
     for (int i = 0; i < RW / 4; ++i) raw.v[i] = g[i];
   }
+  raw.frame = p.frame_ok[e] != 0;
   raw.act = 0;
   if (with_actions) {
     const int8_t* a = p.actions + e * S;
@@ -641,6 +642,7 @@ __device__ __forceinline__ void lane_store(const Params& p, long long e, const L
   r[REC_SNAKE0 + 2 * S] = (u32)env.fruit[0] | ((u32)env.fruit[1] << 16);
   r[REC_SNAKE0 + 2 * S + 1] = (u32)env.fruit[2] | ((u32)env.fruit[3] << 16);
   uint4* g = reinterpret_cast<uint4*>(p.rec + e * RW);
+  p.frame_ok[e] = (u8)p.frame_own;
   if (p.rec_evict_last) {
     u64 pol;
     asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
@@ -811,4 +813,127 @@ __device__ __forceinline__ void lane_unpaint(const Params& p, const PaintEnv<S>&
                                              u8* img, int lane, bool restore) {
   if (restore) lane_restore<K>(tile, tile_bytes >> 4, img, p.V, sub, LPE, lane);
   else lane_paint<S, RULES, K>(p, pe, e_owner, sub, LPE, img, false);
+}
+
+// ---- Delta store (Params::delta): the fused kernel's image store when the own observation buffer already holds the
+// previous frame.  Both frames of an env are the border over a black interior with fruits and bodies painted on top, so
+// a pixel painted in neither the old frame nor the new one is the same in both: writing every 32-byte sector that holds a
+// pixel of the OLD state's classic fruits and bodies or of the NEW state's turns the old image into the new one.  The
+// bytes come from the new image the warp has painted in shared memory; painting and un-painting stay as they are.
+// The first and last (V+1)*C >= 32 bytes of an env image are border (the planner checks it), so a sector holding an
+// interior pixel lies inside its own env and no two warps ever write the same sector.  Bodies of up to
+// DELTA_MAX_LEN segments: the whole chain is in the record's first chain word.
+#define DELTA_MAX_LEN 17
+
+template <int S>
+struct DeltaOld {  // the paint items of the state the record held before the step (= what the old frame shows)
+  u32 hl[S], c0[S];  // head | len << 16, first chain word
+  u32 fr[2];         // classic fruit ids, two u16 per word
+};
+
+template <int S>
+__device__ __forceinline__ DeltaOld<S> delta_old(const LaneRaw<S>& raw) {
+  constexpr int RW = LaneRec<S>::RW;
+  u32 r[RW];
+#pragma unroll
+  for (int i = 0; i < RW / 4; ++i) { r[4 * i] = raw.v[i].x; r[4 * i + 1] = raw.v[i].y; r[4 * i + 2] = raw.v[i].z; r[4 * i + 3] = raw.v[i].w; }
+  DeltaOld<S> o;
+#pragma unroll
+  for (int s = 0; s < S; ++s) { o.hl[s] = r[REC_SNAKE0 + 2 * s]; o.c0[s] = r[LaneRec<S>::c0_word(s)]; }
+  o.fr[0] = r[REC_SNAKE0 + 2 * S]; o.fr[1] = r[REC_SNAKE0 + 2 * S + 1];
+  return o;
+}
+
+// the owner lane's verdict: the old frame is in the buffer and every old and new body fits the first chain word
+template <int S>
+__device__ __forceinline__ bool delta_eligible(const DeltaOld<S>& o, bool frame, const LaneEnv<S>& env) {
+  bool ok = frame;
+#pragma unroll
+  for (int s = 0; s < S; ++s) ok = ok && (o.hl[s] >> 16) <= DELTA_MAX_LEN && env.len[s] <= DELTA_MAX_LEN;
+  return ok;
+}
+
+template <int S>
+__device__ __forceinline__ DeltaOld<S> delta_old_from_lane(const DeltaOld<S>& o, int owner) {
+  DeltaOld<S> d;
+#pragma unroll
+  for (int s = 0; s < S; ++s) { d.hl[s] = __shfl_sync(FULL, o.hl[s], owner); d.c0[s] = __shfl_sync(FULL, o.c0[s], owner); }
+  d.fr[0] = __shfl_sync(FULL, o.fr[0], owner); d.fr[1] = __shfl_sync(FULL, o.fr[1], owner);
+  return d;
+}
+
+// One sector: two 16-byte shared loads (an image starts 16-byte aligned in HBM, so a sector is 16-byte aligned in
+// shared memory), one 32-byte global store (STG.E.ENL2.256).  The data is in registers before the store issues, so the
+// image may be un-painted right after.
+__device__ __forceinline__ void store_sector(u8* g, const u8* s, bool hint, u64 pol) {
+  const uint4 a = *reinterpret_cast<const uint4*>(s), b = *reinterpret_cast<const uint4*>(s + 16);
+  if (hint)
+    asm volatile("st.global.L2::cache_hint.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8}, %9;" ::"l"(g), "r"(a.x), "r"(a.y), "r"(a.z),
+                 "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w), "l"(pol) : "memory");
+  else
+    asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(g), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w), "r"(b.x),
+                 "r"(b.y), "r"(b.z), "r"(b.w) : "memory");
+}
+
+// the one or two sectors of the C-byte pixel at byte `off` of the image; `a` = the image's HBM address mod 32.  A sector
+// outside [0, bytes) is skipped: only a border cell could produce one, and those are never painted.
+template <int C>
+__device__ __forceinline__ void delta_pixel(u8* g, const u8* tile, int bytes, int a, int off, bool hint, u64 pol) {
+  const int r0 = ((off + a) & ~31) - a, r1 = ((off + C - 1 + a) & ~31) - a;
+  if ((u32)r0 <= (u32)(bytes - 32)) store_sector(g + r0, tile + r0, hint, pol);
+  if (r1 != r0 && (u32)r1 <= (u32)(bytes - 32)) store_sector(g + r1, tile + r1, hint, pol);
+}
+
+// Store the sectors of one env of the image.  Its paint items -- the new and the old classic fruits, then per snake the
+// segments of the new and of the old body -- are dealt round-robin to the env's LPE lanes; one loop with one store site
+// keeps the code small (the kernel lives off the instruction cache, see lane_reset).  `bytes` = bytes of the image that
+// belong to valid envs.
+template <int S, int K>
+__device__ __forceinline__ void delta_store(const Params& p, const PaintEnv<S>& pe, const DeltaOld<S>& po, int slot, int sub, int LPE,
+                                            const u8* tile, int bytes, long long e0) {
+  constexpr int C = 3 * K;
+  if (!pe.valid) return;
+  const int V = p.V, F = p.F;
+  const long long t0 = e0 * (long long)p.E;
+  u8* g = p.obs + t0;
+  const int a = (int)(t0 & 31), base = slot * p.E;
+  const bool hint = p.obs_evict_first;
+  u64 pol = 0;
+  if (hint) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
+  // A snake that moved (and was neither killed nor reset) has old segment i = new segment i + 1: of its old body only the
+  // segments from new length - 1 on (the popped tail) are not in the new one.  `skip[s]` old segments are left out.
+  int n = 2 * F, skip[S];
+#pragma unroll
+  for (int s = 0; s < S; ++s) {
+    const int nl = pe.len[s], oh = (int)(po.hl[s] & 0xffffu), ol = (int)(po.hl[s] >> 16);
+    const u32 m = ol >= 17 ? ~0u : (1u << (2 * max(ol - 1, 0))) - 1u;  // the codes of the old body
+    const bool shifted = nl >= 1 && pe.head[s] - codes_disp(pe.c0[s], V, 1) == oh && (((pe.c0[s] >> 2) ^ po.c0[s]) & m) == 0;
+    skip[s] = shifted ? min(ol, nl - 1) : 0;
+    n += nl + ol - skip[s];
+  }
+  for (int j = sub; j < n; j += LPE) {
+    int pid = 0;
+    if (j < 2 * F) {
+#pragma unroll
+      for (int f = 0; f < 4; ++f) {
+        const int of = (int)((po.fr[f >> 1] >> (16 * (f & 1))) & 0xffffu);
+        if (f < F && j == f) pid = pe.fruit[f];
+        if (f < F && j == F + f) pid = of == pe.fruit[f] ? -1 : of;  // a fruit that stayed is one of the new items
+      }
+    } else {
+      int i = j - 2 * F, head = 0;
+      u32 w = 0;
+      bool found = false;
+#pragma unroll
+      for (int s = 0; s < S; ++s) {
+        const int nl = pe.len[s], ol = (int)(po.hl[s] >> 16) - skip[s];
+        if (!found && i < nl) { head = pe.head[s]; w = pe.c0[s]; found = true; }
+        else if (!found) i -= nl;
+        if (!found && i < ol) { head = (int)(po.hl[s] & 0xffffu); w = po.c0[s]; i += skip[s]; found = true; }
+        else if (!found) i -= ol;
+      }
+      pid = head - codes_disp(w, V, i);
+    }
+    if (pid >= 0) delta_pixel<C>(g, tile, bytes, a, base + pid * C, hint, pol);
+  }
 }

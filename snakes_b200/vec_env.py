@@ -175,6 +175,9 @@ class SnakeVecEnv(object):
     `host_copy` (default True: fresh arrays every step like np.stack; False: views of the pinned,
     NUMA-local staging buffers).  `debug`: experiment switches, a "key=value,..." string
     (include/snk.h, snk_create_ex); None reads the SNK_DEBUG environment variable.
+    `obs` (device tensor [N, H, W, 3K]) is the handle's own observation buffer and is read-only for callers: a step
+    rewrites only the 32-byte pieces of it that can have changed since the previous frame, so whatever is written into
+    it between steps may survive them.  Copy it (or use set_obs_target / rollout buffers) to modify observations.
     """
 
     def __init__(self, num_envs, size=(10, 10), n_snakes=2, n_fruits=None, n_views=None, rules="classic",
