@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SNK_VERSION 200 /* 0.2.0 */
+#define SNK_VERSION 300 /* 0.3.0 */
 
 /* error codes */
 #define SNK_OK 0
@@ -44,7 +44,8 @@ extern "C" {
 #define SNK_DEVERR_TAPE_BOUND 2u      /* replayed draw was recorded with another bound */
 #define SNK_DEVERR_FRUIT_OVERFLOW 4u  /* >255 fruits on one cell (adversarial / cut grid) */
 #define SNK_DEVERR_BODY_OVERFLOW 8u   /* ring capacity exceeded (cannot happen for cap = D*D+1) */
-#define SNK_DEVERR_BAD_STATE 16u      /* snk_load_state: a body whose consecutive segments are not adjacent cells */
+#define SNK_DEVERR_BAD_STATE 16u      /* a rejected state (snk_load_state, snk_restore_envs: see there) or an env index outside
+                                       * [0, N) given to snk_save_envs / snk_restore_envs / snk_copy_envs (entry skipped) */
 
 /* rule-sets */
 #define SNK_RULES_CLASSIC 0      /* gym_snake/envs/snake_multiple_test.py  (SnakeEnv) */
@@ -253,7 +254,7 @@ int snk_gae(const float* d_rewards, const float* d_values, const uint8_t* d_done
 int snk_set_draw_tape(snk_handle* h, const uint32_t* h_vals, const uint32_t* h_bounds,
                       const uint64_t* h_offsets);
 
-/* Canonical state (parity tests, checkpoint / resume).  Synchronous. */
+/* Canonical state (parity tests, checkpoint / resume) through HOST memory.  Synchronous. */
 int snk_state_layout_of(const snk_config* cfg, snk_state_layout* out);
 int snk_dump_state(snk_handle* h, void* h_dst, size_t bytes);
 /* Envs [first, first + count) only, as the blob of a `count`-env configuration (snk_state_layout_of with num_envs =
@@ -262,6 +263,32 @@ int snk_dump_state_range(snk_handle* h, int64_t first, int64_t count, void* h_ds
 /* Rejects (SNK_ESTATE, offending snakes left empty) bodies longer than the board, cell ids outside the padded grid,
  * velocity codes above 4 and consecutive segments that are not adjacent cells. */
 int snk_load_state(snk_handle* h, const void* h_src, size_t bytes);
+
+/* Per-env state on the device: start episodes from stored states, paired evaluation from the same start states, search by
+ * cloning one env into many slots.  None of the three synchronises, allocates or touches host memory; all work is
+ * stream-ordered on `stream`, so they can be recorded into a CUDA graph.  Indices are int64 device arrays (the dtype of a
+ * PyTorch index tensor).  An index outside [0, N) raises SNK_DEVERR_BAD_STATE (read it with snk_check_errors) and nothing is written for
+ * that entry; the launch itself still runs.  Device blobs must be 16-byte aligned.
+ *   What moves: all of the canonical state -- t, spare, draw_ctr, Monitor's running ep_ret / ep_len, bodies, grow_to, vel
+ *   and fruits.  What does not: the per-step outputs (d_reward, d_done, d_num_alive, d_episode_*), the running d_stats
+ *   sums, and the RNG key, which stays (seed, global id of the DESTINATION env).  A restored or copied env continues with
+ *   the source's draw_ctr on its own Philox stream, so a clone is identical to its source only until the next random
+ *   draw (a fruit respawn, an auto-reset).  In tape mode draw_ctr indexes the destination env's tape.
+ *   Observations are not re-encoded (as after snk_load_state): restored / copied envs are marked so that the next step
+ *   writes their images whole; call snk_reset with an all-zero mask to re-encode every env's observation at once. */
+/* Canonical state of envs d_idx[0..count) (NULL: envs [0, count)) into the DEVICE buffer d_blob, laid out as the blob of a
+ * `count`-env configuration (snk_state_layout_of with num_envs = count): byte-identical to what snk_dump_state_range
+ * writes for the same envs.  Indices may repeat. */
+int snk_save_envs(snk_handle* h, const int64_t* d_idx, int64_t count, void* d_blob, size_t bytes, void* stream);
+/* Env d_idx[j] (NULL: env j) <- entry j of the device blob d_blob (a `count`-env blob).  Validates exactly what
+ * snk_load_state validates; a rejected snake is left empty and SNK_DEVERR_BAD_STATE is raised.  Destination indices must
+ * be distinct.  The blob may come from a handle of another num_envs / seed / env_id_base, as long as size, n_snakes,
+ * n_fruits and rules are the same. */
+int snk_restore_envs(snk_handle* h, const int64_t* d_idx, int64_t count, const void* d_blob, size_t bytes, void* stream);
+/* Env d_dst[j] <- env d_src[j], private layout to private layout (record, chain words / ring row, fruit grid + bitmap):
+ * about 1/12 of the bytes of a save + restore through a blob at 2 snakes on 19x19.  d_src may repeat (1 -> many); d_dst
+ * must be distinct and disjoint from d_src. */
+int snk_copy_envs(snk_handle* h, const int64_t* d_src, const int64_t* d_dst, int64_t count, void* stream);
 
 /* Episode statistics (Monitor's aggregate role).  snk_get_stats synchronises `stream`. */
 int snk_get_stats(snk_handle* h, double* h_stats /*[SNK_NSTATS]*/, void* stream);

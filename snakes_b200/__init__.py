@@ -8,9 +8,9 @@ from ._lib import SnkError  # noqa: F401
 
 _lib.lib()  # no CPU fallback: a missing extension is an import error
 
-from .vec_env import Infos, MonitorCSV, SnakeVecEnv, StepGraph, split_state  # noqa: E402,F401
+from .vec_env import EnvStates, Infos, MonitorCSV, SnakeVecEnv, StepGraph, split_state  # noqa: E402,F401
 from .sharding import all_reduce_stats, make_sharded_env, shard_range  # noqa: E402,F401
 from .rollout import gae  # noqa: E402,F401
 from .registration import ENV_IDS, SnakeGymEnv, make, make_basic_env, register  # noqa: E402,F401
 
-__version__ = "0.2.0"
+__version__ = "0.3.0"

@@ -15,7 +15,7 @@ RNG_PHILOX, RNG_TAPE = 0, 1
 NSTATS = 8
 STAT_NAMES = ("env_steps", "episodes", "return_sum", "length_sum", "fruits", "deaths", "body_cells", "draws")
 DEVERR = {1: "draw tape underrun", 2: "draw tape bound mismatch", 4: "fruit count overflow", 8: "body ring overflow",
-          16: "bad state blob (non-adjacent segments, cell id or length out of range)"}
+          16: "bad state (non-adjacent segments, cell id or length out of range) or env index out of range"}
 GRAPH_SYNC_BACK = 1
 
 
@@ -71,6 +71,9 @@ _SIGNATURES = {
     "snk_dump_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t]),
     "snk_dump_state_range": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_size_t]),
     "snk_load_state": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t]),
+    "snk_save_envs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "snk_restore_envs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "snk_copy_envs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "snk_get_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "snk_reset_stats": (C.c_int, [C.c_void_p, C.c_void_p]),
     "snk_check_errors": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint32), C.c_void_p]),

@@ -523,7 +523,7 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   TRY(dev_alloc(h, &h->d_obs_own, (size_t)N * p.E, true));
   p.obs = h->d_obs_own;
   if (p.family == 1) {
-    // frame_ok[e] = 1 <=> d_obs_own holds exactly the image of env e's record (cleared here and by snk_load_state, written
+    // frame_ok[e] = 1 <=> d_obs_own holds exactly the image of env e's record (cleared here and by every restore / copy, written
     // by every lane-family kernel that writes a record).  With it the fused kernel's classic step stores only the sectors
     // a step changes; delta=0 always stores whole images.  Sectors never cross env boundaries because the first and last
     // (V+1)*C bytes of an env image are border (needs >= 32) and the buffer is 32-byte aligned.  Default: 32-env batches
@@ -1100,21 +1100,25 @@ static int ensure_blob(snk_handle* h, size_t bytes) {
   return rc;
 }
 
+// the blob layout of a `count`-env configuration of this handle's geometry
+static int sub_layout(const snk_handle* h, int64_t count, snk_state_layout* lay) {
+  snk_config sub = h->cfg;
+  sub.num_envs = count; sub.env_id_base = 0;
+  return snk_state_layout_of(&sub, lay);
+}
+
 extern "C" int snk_dump_state_range(snk_handle* h, int64_t first, int64_t count, void* h_dst, size_t bytes) {
   if (!h || !h_dst) return fail(SNK_EINVAL, "NULL argument");
   if (first < 0 || count < 1 || first + count > h->p.N) return fail(SNK_EINVAL, "env range [%lld, %lld) outside [0, %lld)",
                                                                     (long long)first, (long long)(first + count), h->p.N);
-  snk_config sub = h->cfg;
-  sub.num_envs = count; sub.env_id_base = h->cfg.env_id_base + first;
   snk_state_layout lay;
-  int rc = snk_state_layout_of(&sub, &lay);
+  int rc = sub_layout(h, count, &lay);
   if (rc) return rc;
   if (bytes < lay.total_bytes) return fail(SNK_EINVAL, "buffer too small: %zu < %zu", bytes, lay.total_bytes);
   CUDA_TRY(cudaSetDevice(h->cfg.device));
   if ((rc = ensure_blob(h, lay.total_bytes))) return rc;
   CUDA_TRY(cudaDeviceSynchronize());
-  CUDA_TRY(cudaMemset(h->d_blob, 0, lay.total_bytes));
-  CUDA_TRY(snk_launch_dump(h->p, h->d_blob, lay, first, count, 0));
+  CUDA_TRY(snk_launch_save(h->p, nullptr, first, count, h->d_blob, lay, 0));  // writes every byte of the blob
   h->launches++;
   CUDA_TRY(cudaMemcpy(h_dst, h->d_blob, lay.total_bytes, cudaMemcpyDeviceToHost));
   return SNK_OK;
@@ -1134,8 +1138,7 @@ extern "C" int snk_load_state(snk_handle* h, const void* h_src, size_t bytes) {
   CUDA_TRY(cudaDeviceSynchronize());
   CUDA_TRY(cudaMemcpy(h->d_blob, h_src, h->lay.total_bytes, cudaMemcpyHostToDevice));
   h->obs_current = nullptr;
-  if (h->p.frame_ok) CUDA_TRY(cudaMemset(h->p.frame_ok, 0, (size_t)h->p.N));  // the own buffer no longer shows the records
-  CUDA_TRY(snk_launch_load(h->p, h->d_blob, h->lay, 0));
+  CUDA_TRY(snk_launch_restore(h->p, nullptr, h->p.N, h->d_blob, h->lay, 0));  // clears frame_ok: the own buffer no longer shows the records
   h->launches++;
   CUDA_TRY(cudaDeviceSynchronize());
   uint32_t flags = 0;
@@ -1146,6 +1149,60 @@ extern "C" int snk_load_state(snk_handle* h, const void* h_src, size_t bytes) {
     return fail(SNK_ESTATE, "state blob rejected: a body that is too long, leaves the padded grid, has a velocity code above 4 "
                             "or whose consecutive segments are not adjacent cells (those snakes were left empty)");
   }
+  return SNK_OK;
+}
+
+// A state change the host did not see while a graph is being recorded on `stream`: the recorded work has not run, so the
+// host-side view of the state (obs_current) stays as it is, the way launch() treats a captured step.
+static bool stream_capturing(cudaStream_t stream) {
+  cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(stream, &st) != cudaSuccess) {
+    cudaGetLastError();
+    return true;  // the legacy stream while another stream captures globally: a capture is under way
+  }
+  return st != cudaStreamCaptureStatusNone;
+}
+
+static int envs_check(const snk_handle* h, const void* d_blob, int64_t count, size_t bytes, bool idx_null, snk_state_layout* lay) {
+  if (!h || !d_blob) return fail(SNK_EINVAL, "NULL argument");
+  if (count < 1) return fail(SNK_EINVAL, "count must be >= 1, got %lld", (long long)count);
+  if (idx_null && count > h->p.N) return fail(SNK_EINVAL, "count %lld > num_envs %lld without indices", (long long)count, h->p.N);
+  if (((uintptr_t)d_blob & 15) != 0) return fail(SNK_EINVAL, "device blob must be 16-byte aligned");
+  int rc = sub_layout(h, count, lay);
+  if (rc) return rc;
+  if (bytes < lay->total_bytes) return fail(SNK_EINVAL, "blob too small: %zu < %zu bytes for %lld envs", bytes, lay->total_bytes,
+                                            (long long)count);
+  return SNK_OK;
+}
+
+extern "C" int snk_save_envs(snk_handle* h, const int64_t* d_idx, int64_t count, void* d_blob, size_t bytes, void* stream) {
+  snk_state_layout lay;
+  int rc = envs_check(h, d_blob, count, bytes, d_idx == nullptr, &lay);
+  if (rc) return rc;
+  CUDA_TRY(cudaSetDevice(h->cfg.device));
+  CUDA_TRY(snk_launch_save(h->p, d_idx, 0, count, (uint8_t*)d_blob, lay, (cudaStream_t)stream));
+  h->launches++;
+  return SNK_OK;
+}
+
+extern "C" int snk_restore_envs(snk_handle* h, const int64_t* d_idx, int64_t count, const void* d_blob, size_t bytes, void* stream) {
+  snk_state_layout lay;
+  int rc = envs_check(h, d_blob, count, bytes, d_idx == nullptr, &lay);
+  if (rc) return rc;
+  CUDA_TRY(cudaSetDevice(h->cfg.device));
+  CUDA_TRY(snk_launch_restore(h->p, d_idx, count, (const uint8_t*)d_blob, lay, (cudaStream_t)stream));
+  h->launches++;
+  if (!stream_capturing((cudaStream_t)stream)) h->obs_current = nullptr;
+  return SNK_OK;
+}
+
+extern "C" int snk_copy_envs(snk_handle* h, const int64_t* d_src, const int64_t* d_dst, int64_t count, void* stream) {
+  if (!h || !d_src || !d_dst) return fail(SNK_EINVAL, "NULL argument");
+  if (count < 1) return fail(SNK_EINVAL, "count must be >= 1, got %lld", (long long)count);
+  CUDA_TRY(cudaSetDevice(h->cfg.device));
+  CUDA_TRY(snk_launch_copy(h->p, d_src, d_dst, count, (cudaStream_t)stream));
+  h->launches++;
+  if (!stream_capturing((cudaStream_t)stream)) h->obs_current = nullptr;
   return SNK_OK;
 }
 

@@ -1325,114 +1325,248 @@ __global__ void k_gae(const float* __restrict__ rewards, const float* __restrict
   }
 }
 
-// ------------------------------------------------------------------ state dump / load, action stream
-// canonical blob <-> private layout; one thread per (env, snake); not on the hot path
-__global__ void k_dump(const Params p, u8* blob, snk_state_layout lay, long long first, long long count) {
-  // `lay` is the layout of a blob of `count` envs; local env el of the blob is env first + el of the handle
-  const long long il = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-  const int S = p.S, cap = p.cap;
-  if (il >= count * S) return;
-  const long long el = il / S, e = first + el;
-  const int s = (int)(il - el * S);
-  const long long i = e * S + s;
+// ------------------------------------------------------------------ env state: canonical blob <-> private layout
+// snk_save_envs / snk_restore_envs / snk_copy_envs, and through them snk_dump_state(_range) / snk_load_state.  One warp
+// per entry: its snakes one after the other, then the entry's scalars and fruits.  Entry j of a launch is env idx[j]
+// of the handle (idx == NULL: env first + j) and row j of a `count`-env blob.  An index outside [0, N) raises
+// SNK_DEVERR_BAD_STATE and nothing is written for that entry.  Body rows move as 16-byte vectors by consecutive lanes.
+__device__ __forceinline__ bool entry_env(const Params& p, const int64_t* idx, long long first, long long j, bool report,
+                                          long long& e) {
+  e = idx ? (long long)idx[j] : first + j;
+  if (e >= 0 && e < p.N) return true;
+  if (report) atomicOr(p.err, SNK_DEVERR_BAD_STATE);
+  return false;
+}
+
+// the alignment gaps between the arrays of a blob (zero in every blob, so two blobs are byte-comparable)
+__device__ __noinline__ void blob_zero_gaps(u8* blob, const snk_state_layout lay, long long n, int S, int F, int VV) {
+  const size_t end[10] = {lay.off_t + 4 * n, lay.off_spare + 4 * n, lay.off_draw_ctr + 4 * n, lay.off_ep_ret + 4 * n,
+                          lay.off_ep_len + 4 * n, lay.off_len + 2 * n * S, lay.off_grow_to + 2 * n * S, lay.off_vel + n * S,
+                          lay.off_body + 2 * n * S * lay.cap, lay.off_fruit + (lay.fruit_is_grid ? n * VV : 2 * n * F)};
+  const size_t next[10] = {lay.off_spare, lay.off_draw_ctr, lay.off_ep_ret, lay.off_ep_len, lay.off_len, lay.off_grow_to,
+                           lay.off_vel, lay.off_body, lay.off_fruit, lay.total_bytes};
+#pragma unroll
+  for (int k = 0; k < 10; ++k)
+    for (size_t b = end[k]; b < next[k]; ++b) blob[b] = 0;
+}
+
+// private -> canonical.  Lane family: lane w expands chain word w (16 segments, two 16-byte stores of the row); the id of
+// its first segment is the head minus the displacement of all earlier words, an exclusive warp scan of the per-word
+// displacements (codes_disp).  Word 0 is the record's c0 word; words >= 1 are read only where the body reaches them.
+// Ring family: lane l takes 8 consecutive segments (ring_at) per 16-byte store.  Padding zeros are stored too.
+__global__ void __launch_bounds__(256) k_save_envs(const Params p, const int64_t* __restrict__ idx, long long first,
+                                                   long long count, u8* __restrict__ blob, const snk_state_layout lay) {
+  const int lane = threadIdx.x & 31, S = p.S, cap = p.cap, V = p.V;
+  if (blockIdx.x == 0 && threadIdx.x == 0) blob_zero_gaps(blob, lay, count, S, p.F, p.VV);
+  const long long j = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;  // entry j
+  if (j >= count) return;
+  long long e;
+  if (!entry_env(p, idx, first, j, lane == 0, e)) return;
   const u32* r = p.rec + e * p.RW;
-  const u32 a = r[REC_SNAKE0 + 2 * s], b = r[REC_SNAKE0 + 2 * s + 1];
-  const int len = a >> 16, hs = a & 0xffff;
-  reinterpret_cast<u16*>(blob + lay.off_len)[il] = (u16)len;
-  reinterpret_cast<u16*>(blob + lay.off_grow_to)[il] = (u16)(b & 0xffff);
-  (blob + lay.off_vel)[il] = (u8)(b >> 16);
-  u16* dst = reinterpret_cast<u16*>(blob + lay.off_body) + il * cap;
-  if (p.family == 1) {  // chain code: hs is the head id
-    const u32* ch = p.chain + i * p.CW;
-    const u32 c0 = r[s < 3 ? 5 + s : p.RW - 2];  // LaneRec::c0_word
-    for (int k = 0; k < cap; ++k) dst[k] = 0;
-    chain_walk(hs, len, c0, ch, p.V, [&](int k, int pid) { dst[k] = (u16)pid; });
-  } else {
-    const u16* ring = p.body + i * cap;
-    for (int k = 0; k < cap; ++k) dst[k] = k < len ? (u16)ring_at(ring, hs, k, cap) : (u16)0;
-  }
-  if (s == 0) {
-    reinterpret_cast<int32_t*>(blob + lay.off_t)[el] = (int32_t)r[REC_T];
-    reinterpret_cast<u32*>(blob + lay.off_spare)[el] = r[REC_SPARE];
-    reinterpret_cast<u32*>(blob + lay.off_draw_ctr)[el] = r[REC_DRAW_CTR];
-    reinterpret_cast<u32*>(blob + lay.off_ep_ret)[el] = r[REC_EP_RET];
-    reinterpret_cast<int32_t*>(blob + lay.off_ep_len)[el] = (int32_t)r[REC_EP_LEN];
-    if (lay.fruit_is_grid && p.family == 1) {
-      for (int k = 0; k < p.VV; ++k)
-        (blob + lay.off_fruit)[el * p.VV + k] = ((p.gbits[e * p.GBW + (k >> 5)] >> (k & 31)) & 1) ? p.grid[e * p.grid_stride + k] : (u8)0;
-    } else if (lay.fruit_is_grid) {
-      for (int k = 0; k < p.VV; ++k) (blob + lay.off_fruit)[el * p.VV + k] = p.grid[e * p.grid_stride + k];
-    } else {
-      const u16* fr = reinterpret_cast<const u16*>(r + REC_SNAKE0 + 2 * S);
-      for (int k = 0; k < p.F; ++k) reinterpret_cast<u16*>(blob + lay.off_fruit)[el * p.F + k] = fr[k];
+  for (int s = 0; s < S; ++s) {
+    const long long u = j * S + s;
+    const u32 a = r[REC_SNAKE0 + 2 * s], b = r[REC_SNAKE0 + 2 * s + 1];
+    const int len = a >> 16, hs = a & 0xffff;
+    if (lane == 0) {
+      reinterpret_cast<u16*>(blob + lay.off_len)[u] = (u16)len;
+      reinterpret_cast<u16*>(blob + lay.off_grow_to)[u] = (u16)(b & 0xffff);
+      (blob + lay.off_vel)[u] = (u8)(b >> 16);
     }
-  }
-}
-
-// snk_load_state trusts nothing: a body longer than the board, a cell id outside the padded grid, a velocity code above 4
-// or two consecutive segments that are not adjacent cells raise SNK_DEVERR_BAD_STATE and leave that snake empty.
-__global__ void k_load(const Params p, const u8* blob, snk_state_layout lay) {
-  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-  const int S = p.S, cap = p.cap;
-  if (i >= p.N * S) return;
-  const long long e = i / S;
-  const int s = (int)(i - e * S);
-  u32* r = p.rec + e * p.RW;
-  u32 len = reinterpret_cast<const u16*>(blob + lay.off_len)[i];
-  const u32 grow = reinterpret_cast<const u16*>(blob + lay.off_grow_to)[i];
-  u32 vel = (blob + lay.off_vel)[i];
-  const u16* src = reinterpret_cast<const u16*>(blob + lay.off_body) + i * cap;
-  bool bad = len > (u32)(p.D * p.D + 1) || len > (u32)cap || vel > 4u;
-  for (u32 k = 0; k < len && !bad; ++k) bad = src[k] >= (u32)p.VV;
-  if (p.family == 1) {
-    for (u32 k = 0; k + 1 < len && !bad; ++k) {
-      const int diff = (int)src[k] - (int)src[k + 1];
-      bad = !(diff == p.V || diff == 1 || diff == -p.V || diff == -1);
-    }
-  }
-  if (bad) { atomicOr(p.err, SNK_DEVERR_BAD_STATE); len = 0; vel = 0; }
-  r[REC_SNAKE0 + 2 * s + 1] = grow | (vel << 16);
-  if (p.family == 1) {  // chain code: direction of segment k+1 -> k, 16 per word
-    r[REC_SNAKE0 + 2 * s] = (len ? (u32)src[0] : 0u) | (len << 16);
-    u32* ch = p.chain + i * p.CW;
-    for (int k = 0; k < p.CW; ++k) ch[k] = 0;
-    for (int k = 0; k + 1 < (int)len; ++k) {
-      const int diff = (int)src[k] - (int)src[k + 1];
-      const u32 d = diff == p.V ? 0u : diff == 1 ? 1u : diff == -p.V ? 2u : 3u;
-      ch[k >> 4] |= d << (2 * (k & 15));
-    }
-    r[s < 3 ? 5 + s : p.RW - 2] = ch[0];  // LaneRec::c0_word
-  } else {
-    r[REC_SNAKE0 + 2 * s] = 0u | (len << 16);
-    u16* ring = p.body + i * cap;
-    for (int k = 0; k < cap; ++k) ring[k] = k < (int)len ? src[k] : (u16)0;
-  }
-  if (s == 0) {
-    r[REC_T] = (u32) reinterpret_cast<const int32_t*>(blob + lay.off_t)[e];
-    r[REC_SPARE] = reinterpret_cast<const u32*>(blob + lay.off_spare)[e];
-    r[REC_DRAW_CTR] = reinterpret_cast<const u32*>(blob + lay.off_draw_ctr)[e];
-    r[REC_EP_RET] = reinterpret_cast<const u32*>(blob + lay.off_ep_ret)[e];
-    r[REC_EP_LEN] = (u32) reinterpret_cast<const int32_t*>(blob + lay.off_ep_len)[e];
-    if (p.family == 0) r[5] = r[6] = r[7] = 0;
-    if (lay.fruit_is_grid) {
-      for (int k = 0; k < p.VV; ++k) p.grid[e * p.grid_stride + k] = (blob + lay.off_fruit)[e * p.VV + k];
-      if (p.family == 1) {
-        for (int w = 0; w < p.GBW; ++w) {
-          u32 bits = 0;
-          for (int k = 32 * w; k < min(32 * w + 32, p.VV); ++k) if (p.grid[e * p.grid_stride + k]) bits |= 1u << (k & 31);
-          p.gbits[e * p.GBW + w] = bits;
+    uint4* dst = reinterpret_cast<uint4*>(blob + lay.off_body + (size_t)u * cap * 2);
+    if (p.family == 1) {  // chain code: hs is the head id
+      const u32 c0 = r[s < 3 ? 5 + s : p.RW - 2];  // LaneRec::c0_word
+      const u32* ch = p.chain + (e * S + s) * p.CW;
+      int base = hs;  // id of the first segment of the current 32 words
+      for (int w0 = 0; 16 * w0 < cap; w0 += 32) {
+        const int w = w0 + lane, k0 = 16 * w;
+        const u32 word = k0 < len ? (w == 0 ? c0 : ch[w]) : 0u;
+        const int disp = k0 < len ? codes_disp(word, V, 16) : 0;
+        const int incl = warp_incl_scan(disp, lane);
+        int pid = base - (incl - disp);
+        base -= __shfl_sync(FULL, incl, 31);
+        u32 o[8];
+  #pragma unroll
+        for (int q = 0; q < 16; ++q) {
+          const u32 v = k0 + q < len ? (u32)pid : 0u;
+          o[q >> 1] = (q & 1) ? (o[q >> 1] | (v << 16)) : v;
+          pid -= chain_delta((word >> (2 * q)) & 3, V);
         }
+        if (k0 + 8 <= cap) dst[2 * w] = make_uint4(o[0], o[1], o[2], o[3]);
+        if (k0 + 16 <= cap) dst[2 * w + 1] = make_uint4(o[4], o[5], o[6], o[7]);
       }
     } else {
-      u16* fr = reinterpret_cast<u16*>(r + REC_SNAKE0 + 2 * S);
-      for (int k = 0; k < p.F; ++k) {
-        const u16 f = reinterpret_cast<const u16*>(blob + lay.off_fruit)[e * p.F + k];
-        if (f >= (u32)p.VV) { atomicOr(p.err, SNK_DEVERR_BAD_STATE); fr[k] = (u16)(p.V + 1); } else fr[k] = f;
+      const u16* ring = p.body + (e * S + s) * cap;
+      for (int k0 = 8 * lane; k0 < cap; k0 += 256) {
+        u32 o[4];
+  #pragma unroll
+        for (int q = 0; q < 8; ++q) {
+          const u32 v = k0 + q < len ? (u32)ring_at(ring, hs, k0 + q, cap) : 0u;
+          o[q >> 1] = (q & 1) ? (o[q >> 1] | (v << 16)) : v;
+        }
+        dst[k0 >> 3] = make_uint4(o[0], o[1], o[2], o[3]);
       }
     }
   }
+  if (lane == 0) {
+    reinterpret_cast<u32*>(blob + lay.off_t)[j] = r[REC_T];
+    reinterpret_cast<u32*>(blob + lay.off_spare)[j] = r[REC_SPARE];
+    reinterpret_cast<u32*>(blob + lay.off_draw_ctr)[j] = r[REC_DRAW_CTR];
+    reinterpret_cast<u32*>(blob + lay.off_ep_ret)[j] = r[REC_EP_RET];
+    reinterpret_cast<u32*>(blob + lay.off_ep_len)[j] = r[REC_EP_LEN];
+  }
+  if (lay.fruit_is_grid) {  // lane family: a count is valid only where its gbits bit is set
+    const u8* g = p.grid + e * p.grid_stride;
+    const u32* gb = p.family == 1 ? p.gbits + e * p.GBW : nullptr;
+    u8* out = blob + lay.off_fruit + (size_t)j * p.VV;
+    for (int k = lane; k < p.VV; k += 32) out[k] = (!gb || ((gb[k >> 5] >> (k & 31)) & 1)) ? g[k] : (u8)0;
+  } else if (lane < p.F) {
+    reinterpret_cast<u16*>(blob + lay.off_fruit)[j * p.F + lane] = reinterpret_cast<const u16*>(r + REC_SNAKE0 + 2 * S)[lane];
+  }
 }
 
+// canonical -> private, trusting nothing: a body longer than the board, a cell id outside the padded grid, a velocity code
+// above 4 or (lane family) two consecutive segments that are not adjacent cells raise SNK_DEVERR_BAD_STATE and leave that
+// snake empty; a classic fruit id outside the grid is flagged and replaced by cell (0, 0).  Lane family: lane w reads
+// segments 16w .. 16w+16 (two 16-byte loads and its neighbour's first id), builds chain word w and checks its part of the
+// body; a warp vote collects the verdict.  Chain words the body does not reach are not written (nothing reads them).
+// Clears frame_ok: the own observation buffer no longer shows the env.
+__global__ void __launch_bounds__(256) k_restore_envs(const Params p, const int64_t* __restrict__ idx, long long count,
+                                                      const u8* __restrict__ blob, const snk_state_layout lay) {
+  const int lane = threadIdx.x & 31, S = p.S, cap = p.cap, V = p.V;
+  const long long j = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+  if (j >= count) return;
+  long long e;
+  if (!entry_env(p, idx, 0, j, lane == 0, e)) return;
+  u32* r = p.rec + e * p.RW;
+  for (int s = 0; s < S; ++s) {
+    const long long u = j * S + s;
+    u32 len = reinterpret_cast<const u16*>(blob + lay.off_len)[u];
+    const u32 grow = reinterpret_cast<const u16*>(blob + lay.off_grow_to)[u];
+    u32 vel = (blob + lay.off_vel)[u];
+    const uint4* src = reinterpret_cast<const uint4*>(blob + lay.off_body + (size_t)u * cap * 2);
+    bool bad = len > (u32)(p.D * p.D + 1) || len > (u32)cap || vel > 4u;
+    const int n = bad ? 0 : (int)len;
+    u32 c0 = 0, head = 0;
+    if (p.family == 1) {
+      u32* ch = p.chain + (e * S + s) * p.CW;
+      for (int w0 = 0; w0 == 0 || 16 * w0 < n; w0 += 32) {
+        const int w = w0 + lane, k0 = 16 * w;
+        u32 v[8];
+  #pragma unroll
+        for (int q = 0; q < 8; ++q) v[q] = 0;
+        if (k0 < n || w == 0) {  // word 0 without waiting for len: most bodies fit it
+          const uint4 x = src[2 * w];
+          v[0] = x.x; v[1] = x.y; v[2] = x.z; v[3] = x.w;
+          if (k0 + 8 < n || (w == 0 && cap >= 16)) { const uint4 y = src[2 * w + 1]; v[4] = y.x; v[5] = y.y; v[6] = y.z; v[7] = y.w; }
+        }
+        int nxt = __shfl_down_sync(FULL, (int)(v[0] & 0xffff), 1);
+        if (lane == 31 && k0 + 16 < n) nxt = reinterpret_cast<const u16*>(src)[k0 + 16];
+        u32 word = 0;
+        bool lbad = false;
+  #pragma unroll
+        for (int q = 0; q < 16; ++q) {
+          const int cur = (int)((v[q >> 1] >> (16 * (q & 1))) & 0xffff);
+          const int nx = q < 15 ? (int)((v[(q + 1) >> 1] >> (16 * ((q + 1) & 1))) & 0xffff) : nxt;
+          if (k0 + q < n) lbad |= cur >= p.VV;
+          if (k0 + q + 1 < n) {
+            const int diff = cur - nx;
+            lbad |= !(diff == V || diff == 1 || diff == -V || diff == -1);
+            word |= (diff == V ? 0u : diff == 1 ? 1u : diff == -V ? 2u : 3u) << (2 * q);
+          }
+        }
+        bad |= __any_sync(FULL, lbad);
+        if (w0 == 0) { c0 = __shfl_sync(FULL, word, 0); head = __shfl_sync(FULL, v[0] & 0xffff, 0); }
+        if (w >= 1 && k0 + 1 < n) ch[w] = word;  // words holding at least one code
+      }
+    } else {  // the whole ring row, zeros past the body (as snk_load_state has always written it), head at slot 0
+      u16* ring = p.body + (e * S + s) * cap;
+      bool lbad = false;
+      for (int k0 = 8 * lane; k0 < cap; k0 += 256) {
+        u32 v[4] = {0u, 0u, 0u, 0u};
+        if (k0 < n) { const uint4 x = src[k0 >> 3]; v[0] = x.x; v[1] = x.y; v[2] = x.z; v[3] = x.w; }
+  #pragma unroll
+        for (int q = 0; q < 8; ++q) {
+          const u32 id = (v[q >> 1] >> (16 * (q & 1))) & 0xffff;
+          if (k0 + q >= n) v[q >> 1] &= (q & 1) ? 0x0000ffffu : 0xffff0000u;
+          else lbad |= id >= (u32)p.VV;
+        }
+        reinterpret_cast<uint4*>(ring)[k0 >> 3] = make_uint4(v[0], v[1], v[2], v[3]);
+      }
+      bad |= __any_sync(FULL, lbad);
+    }
+    if (bad) { len = 0; vel = 0; c0 = 0; }
+    if (lane == 0) {
+      if (bad) atomicOr(p.err, SNK_DEVERR_BAD_STATE);
+      r[REC_SNAKE0 + 2 * s] = (p.family == 1 && len ? head : 0u) | (len << 16);
+      r[REC_SNAKE0 + 2 * s + 1] = grow | (vel << 16);
+      if (p.family == 1) r[s < 3 ? 5 + s : p.RW - 2] = c0;  // LaneRec::c0_word
+    }
+  }
+  if (lane == 0) {
+    r[REC_T] = reinterpret_cast<const u32*>(blob + lay.off_t)[j];
+    r[REC_SPARE] = reinterpret_cast<const u32*>(blob + lay.off_spare)[j];
+    r[REC_DRAW_CTR] = reinterpret_cast<const u32*>(blob + lay.off_draw_ctr)[j];
+    r[REC_EP_RET] = reinterpret_cast<const u32*>(blob + lay.off_ep_ret)[j];
+    r[REC_EP_LEN] = reinterpret_cast<const u32*>(blob + lay.off_ep_len)[j];
+    if (p.family == 0) r[5] = r[6] = r[7] = 0;
+    if (p.frame_ok) p.frame_ok[e] = 0;
+  }
+  if (lay.fruit_is_grid) {  // counts, and the lane family's bitmap of the cells whose count is > 0 (one vote per word)
+    u8* g = p.grid + e * p.grid_stride;
+    const u8* in = blob + lay.off_fruit + (size_t)j * p.VV;
+    for (int c = 0; 32 * c < p.VV; ++c) {
+      const int k = 32 * c + lane;
+      const u8 v = k < p.VV ? in[k] : (u8)0;
+      if (k < p.VV) g[k] = v;
+      const u32 bits = __ballot_sync(FULL, v != 0);
+      if (p.family == 1 && lane == 0) p.gbits[e * p.GBW + c] = bits;
+    }
+  } else if (lane < p.F) {
+    u16 f = reinterpret_cast<const u16*>(blob + lay.off_fruit)[j * p.F + lane];
+    if (f >= (u32)p.VV) { atomicOr(p.err, SNK_DEVERR_BAD_STATE); f = (u16)(p.V + 1); }
+    reinterpret_cast<u16*>(r + REC_SNAKE0 + 2 * S)[lane] = f;
+  }
+}
+
+// private -> private, one warp per (src, dst) pair: the record, the chain words >= 1 each body reaches (lane family) or the
+// whole ring row (ring family), the fruit count grid and the lane family's fruit bitmap; clears frame_ok[dst].
+__global__ void k_copy_envs(const Params p, const int64_t* __restrict__ src,
+                            const int64_t* __restrict__ dst, long long count) {
+  const int lane = threadIdx.x & 31, S = p.S;
+  const long long j = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+  if (j >= count) return;
+  const long long es = src[j], ed = dst[j];
+  if (es < 0 || es >= p.N || ed < 0 || ed >= p.N) {
+    if (lane == 0) atomicOr(p.err, SNK_DEVERR_BAD_STATE);
+    return;
+  }
+  const u32* rs = p.rec + es * p.RW;
+  u32* rd = p.rec + ed * p.RW;
+  for (int w = lane; w < p.RW; w += 32) rd[w] = rs[w];
+  if (p.family == 1) {
+    for (int s = 0; s < S; ++s) {
+      const int len = rs[REC_SNAKE0 + 2 * s] >> 16;
+      const int nw = len >= 2 ? ((len - 2) >> 4) + 1 : 0;  // words holding codes 0 .. len-2; word 0 is in the record
+      const u32* cs = p.chain + (es * S + s) * p.CW;
+      u32* cd = p.chain + (ed * S + s) * p.CW;
+      for (int w = 1 + lane; w < nw; w += 32) cd[w] = cs[w];
+    }
+    if (lane == 0) p.frame_ok[ed] = 0;
+  } else {
+    const uint4* bs = reinterpret_cast<const uint4*>(p.body + es * S * p.cap);
+    uint4* bd = reinterpret_cast<uint4*>(p.body + ed * S * p.cap);
+    for (int k = lane; k < S * p.cap / 8; k += 32) bd[k] = bs[k];
+  }
+  if (p.grid) {
+    const uint4* gs = reinterpret_cast<const uint4*>(p.grid + es * p.grid_stride);
+    uint4* gd = reinterpret_cast<uint4*>(p.grid + ed * p.grid_stride);
+    for (int k = lane; k < p.grid_stride / 16; k += 32) gd[k] = gs[k];
+    if (p.gbits)
+      for (int w = lane; w < p.GBW; w += 32) p.gbits[ed * p.GBW + w] = p.gbits[es * p.GBW + w];
+  }
+}
+
+// ------------------------------------------------------------------ action stream, views
 // The first n_out views of every pixel, packed: [pixels][3K] -> [pixels][3 n_out].  Used by the host-buffer step when
 // the caller only keeps the main snake's view (ppo_multi_agent_new.py:181 stores obs[..., 0:3] alone: the D2H copy then
 // carries n_out / K of the bytes) and by snk_set_main_view_target (the learner's rollout slot).
@@ -1672,9 +1806,20 @@ cudaError_t snk_launch_upscale84(const uint8_t* native, uint8_t* out, long long 
   return launch_upscale<0, 0>(native, out, N, V, C, n_sm, stream);
 }
 
-cudaError_t snk_launch_dump(const Params& p, u8* blob, const snk_state_layout& lay, long long first, long long count, cudaStream_t stream) {
-  const long long n = count * p.S;
-  k_dump<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(p, blob, lay, first, count);
+cudaError_t snk_launch_save(const Params& p, const int64_t* idx, long long first, long long count, u8* blob,
+                            const snk_state_layout& lay, cudaStream_t stream) {
+  k_save_envs<<<(unsigned)((count + 7) / 8), 256, 0, stream>>>(p, idx, first, count, blob, lay);
+  return cudaGetLastError();
+}
+
+cudaError_t snk_launch_restore(const Params& p, const int64_t* idx, long long count, const u8* blob, const snk_state_layout& lay,
+                               cudaStream_t stream) {
+  k_restore_envs<<<(unsigned)((count + 7) / 8), 256, 0, stream>>>(p, idx, count, blob, lay);
+  return cudaGetLastError();
+}
+
+cudaError_t snk_launch_copy(const Params& p, const int64_t* src, const int64_t* dst, long long count, cudaStream_t stream) {
+  k_copy_envs<<<(unsigned)((count + 7) / 8), 256, 0, stream>>>(p, src, dst, count);
   return cudaGetLastError();
 }
 
@@ -1701,12 +1846,6 @@ cudaError_t snk_launch_extract_views(const uint8_t* src, uint8_t* dst, long long
   }
   const long long n = (n_pixels - done + 3) / 4;
   k_extract_views<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(src, dst, done, n_pixels, C, n_out);
-  return cudaGetLastError();
-}
-
-cudaError_t snk_launch_load(const Params& p, const u8* blob, const snk_state_layout& lay, cudaStream_t stream) {
-  const long long n = p.N * p.S;
-  k_load<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(p, blob, lay);
   return cudaGetLastError();
 }
 

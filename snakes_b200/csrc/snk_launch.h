@@ -25,10 +25,14 @@ cudaError_t snk_plan(int rules, LaunchPlan& plan, int n_sm, int S, int K);
 bool snk_lane_supported(int S, int K);
 cudaError_t snk_launch_step(const Params& p, int rules, const LaunchPlan& plan, cudaStream_t stream);
 cudaError_t snk_launch_upscale84(const uint8_t* native, uint8_t* out, long long N, int V, int C, int n_sm, cudaStream_t stream);
-cudaError_t snk_launch_dump(const Params& p, uint8_t* blob, const snk_state_layout& lay, long long first, long long count, cudaStream_t stream);
+// env state (k_save_envs / k_restore_envs / k_copy_envs): entry j is env idx[j], or env first + j when idx is NULL
+cudaError_t snk_launch_save(const Params& p, const int64_t* idx, long long first, long long count, uint8_t* blob,
+                            const snk_state_layout& lay, cudaStream_t stream);
+cudaError_t snk_launch_restore(const Params& p, const int64_t* idx, long long count, const uint8_t* blob, const snk_state_layout& lay,
+                               cudaStream_t stream);
+cudaError_t snk_launch_copy(const Params& p, const int64_t* src, const int64_t* dst, long long count, cudaStream_t stream);
 cudaError_t snk_launch_sum_inbox(const PeerArgs& a, const double* stats, double* glob, cudaStream_t stream);
 cudaError_t snk_launch_extract_views(const uint8_t* src, uint8_t* dst, long long n_pixels, int C, int n_out, cudaStream_t stream);
-cudaError_t snk_launch_load(const Params& p, const uint8_t* blob, const snk_state_layout& lay, cudaStream_t stream);
 cudaError_t snk_launch_scripted_actions(const Params& p, int8_t* actions, uint64_t step, uint64_t seed, int eps_permille,
                                         const uint8_t* occ_obs, cudaStream_t stream);
 cudaError_t snk_launch_gae(const float* rewards, const float* values, const uint8_t* dones, const float* last_values,

@@ -547,6 +547,117 @@ class SnakeVecEnv(object):
         _lib.check(self._L.snk_dump_state_range(self._h, int(first), int(count), blob.ctypes.data_as(C.c_void_p), blob.nbytes))
         return split_state(blob, lay, sub)
 
+    # ------------------------------------------------------------------ per-env state on the device
+    def _sub_config(self, count):
+        """This handle's geometry with `count` envs: the configuration of a `count`-env state blob."""
+        sub = _lib.SnkConfig.from_buffer_copy(self.cfg)
+        sub.num_envs, sub.env_id_base = int(count), 0
+        lay = _lib.SnkStateLayout()
+        _lib.check(self._L.snk_state_layout_of(C.byref(sub), C.byref(lay)))
+        return sub, lay
+
+    def _env_index(self, idx, distinct=False):
+        """(int64 CUDA tensor, count) for an index argument.  A CUDA integer tensor is used as is (trusted: an index
+        outside [0, N) only raises the device error flag, duplicates are not detected); host ints / numpy are checked."""
+        if isinstance(idx, torch.Tensor) and idx.is_cuda:
+            if idx.dtype.is_floating_point or idx.dtype == torch.bool:
+                raise TypeError("env indices must be integers, got %s" % idx.dtype)
+            t = idx.reshape(-1)
+            if t.dtype != torch.int64:
+                t = t.to(torch.int64)
+            return t.contiguous(), int(t.numel()), None
+        a = np.asarray(idx.cpu() if isinstance(idx, torch.Tensor) else idx)
+        if a.dtype.kind not in "iu" and a.size:
+            raise TypeError("env indices must be integers, got %s" % a.dtype)
+        a = a.astype(np.int64).reshape(-1)
+        if a.size == 0:
+            raise ValueError("no env indices given")
+        if a.min() < 0 or a.max() >= self.N:
+            raise IndexError("env index out of range [0, %d)" % self.N)
+        if distinct and len(np.unique(a)) != a.size:
+            raise ValueError("destination env indices must be distinct")
+        return torch.from_numpy(a).to(self.device), int(a.size), a
+
+    def _check_geometry(self, cfg):
+        mine = (self.cfg.size, self.cfg.n_snakes, self.cfg.n_fruits, self.cfg.rules)
+        theirs = (cfg.size, cfg.n_snakes, cfg.n_fruits, cfg.rules)
+        if mine != theirs:
+            raise ValueError("env states of geometry (size, n_snakes, n_fruits, rules) = %r do not fit this env's %r" % (theirs, mine))
+
+    def _observe(self):
+        """Re-encode every env's observation from its state (snk_reset with an all-zero mask), as SnakeVecEnv.load does."""
+        if getattr(self, "_no_reset_mask", None) is None:
+            self._no_reset_mask = torch.zeros(self.N, dtype=torch.uint8, device=self.device)
+        _lib.check(self._L.snk_reset(self._h, C.c_void_p(self._no_reset_mask.data_ptr()), self._stream()))
+
+    def save_envs(self, idx=None, out=None):
+        """Canonical state of envs `idx` (default: all) into a device blob, stream-ordered, no host round trip
+        (snk_save_envs).  Returns an EnvStates; `out` (an EnvStates of len(idx) envs of this geometry) is reused instead
+        of allocating, so the call can be recorded into a CUDA graph.  Indices may repeat."""
+        i, n, _ = (None, self.N, None) if idx is None else self._env_index(idx)
+        if out is None:
+            out = EnvStates.empty(self, n)
+        else:
+            if not isinstance(out, EnvStates):
+                raise TypeError("out must be an EnvStates")
+            self._check_geometry(out.cfg)
+            if out.count != n:
+                raise ValueError("out holds %d envs, %d are saved" % (out.count, n))
+        _lib.check(self._L.snk_save_envs(self._h, None if i is None else C.c_void_p(i.data_ptr()), n,
+                                         C.c_void_p(out.blob.data_ptr()), out.blob.numel(), self._stream()))
+        return out
+
+    def restore_envs(self, states, idx=None, observe=True):
+        """Env idx[j] (default: env j) <- entry j of `states` (snk_restore_envs): an EnvStates, or a uint8 torch / numpy
+        blob of a len(idx)-env layout.  The states may come from another handle of the same geometry (size, n_snakes,
+        n_fruits, rules); a rejected body raises the bad-state device flag (check_errors) and leaves that snake empty.
+        Everything else a step returns (rewards, dones, infos, statistics) is untouched and the RNG key stays the
+        destination env's.  observe=True re-encodes every env's observation from its state afterwards, as after a
+        reset; observe=False leaves the observation buffers as they were (the next step writes the restored envs'
+        images whole) and launches nothing but the restore."""
+        if isinstance(states, EnvStates):
+            self._check_geometry(states.cfg)
+            blob, count = states.blob, states.count
+        else:
+            blob, count = states, None
+        i, n, _ = (None, None, None) if idx is None else self._env_index(idx, distinct=True)
+        count = count if count is not None else (n if n is not None else self.N)
+        if n is not None and n != count:
+            raise ValueError("%d indices for %d saved envs" % (n, count))
+        if n is None and count > self.N:
+            raise ValueError("%d saved envs do not fit %d envs" % (count, self.N))
+        if not isinstance(states, EnvStates):
+            if isinstance(blob, torch.Tensor):
+                if blob.dtype != torch.uint8:
+                    raise TypeError("a state blob must be uint8")
+                blob = blob.reshape(-1).to(self.device).contiguous()
+            else:
+                blob = torch.from_numpy(np.ascontiguousarray(blob, dtype=np.uint8).reshape(-1)).to(self.device)
+            if blob.data_ptr() % 16:
+                blob = blob.clone()
+        if observe:
+            self._before_overwrite()
+        _lib.check(self._L.snk_restore_envs(self._h, None if i is None else C.c_void_p(i.data_ptr()), count,
+                                            C.c_void_p(blob.data_ptr()), blob.numel(), self._stream()))
+        if observe:
+            self._observe()
+
+    def copy_envs(self, src, dst, observe=True):
+        """Env dst[j] <- env src[j] on the device (snk_copy_envs): src may repeat (one env cloned into many slots),
+        dst must be distinct and disjoint from src.  A clone keeps its own RNG key, so it equals its source until the
+        next random draw.  `observe` as in restore_envs."""
+        s, ns, hs = self._env_index(src)
+        d, nd, hd = self._env_index(dst, distinct=True)
+        if ns != nd:
+            raise ValueError("%d sources for %d destinations" % (ns, nd))
+        if hs is not None and hd is not None and np.intersect1d(hs, hd).size:
+            raise ValueError("destination envs must not also be sources")
+        if observe:
+            self._before_overwrite()
+        _lib.check(self._L.snk_copy_envs(self._h, C.c_void_p(s.data_ptr()), C.c_void_p(d.data_ptr()), ns, self._stream()))
+        if observe:
+            self._observe()
+
     def save(self, path):
         """Checkpoint of the env state (the reference never checkpoints it; its learner only saves
         model parameters, ppo_multi_agent_new.py:104-106).  A .npz with the constructor arguments
@@ -691,6 +802,50 @@ class SnakeVecEnv(object):
         out = C.c_double(0)
         _lib.check(self._L.snk_algorithmic_bytes_per_step(C.byref(self.cfg), float(mean_sum_len), C.byref(out)))
         return out.value
+
+
+class EnvStates(object):
+    """Canonical states of `count` envs in a device uint8 blob (SnakeVecEnv.save_envs): the blob of a `count`-env
+    configuration of the env's geometry, byte for byte what dump_state_range writes for the same envs.  `cfg` is that
+    configuration and `lay` its SnkStateLayout.  States move between handles of the same size, n_snakes, n_fruits and
+    rules (another num_envs, seed or env_id_base is fine)."""
+
+    def __init__(self, blob, cfg, lay):
+        assert isinstance(blob, torch.Tensor) and blob.is_cuda and blob.dtype == torch.uint8 and blob.numel() >= lay.total_bytes
+        self.blob, self.cfg, self.lay = blob, cfg, lay
+        self.count = int(cfg.num_envs)
+
+    @classmethod
+    def empty(cls, env, count):
+        """An uninitialised buffer for `count` envs of `env`'s geometry (for save_envs(out=...))."""
+        cfg, lay = env._sub_config(count)
+        return cls(torch.empty(int(lay.total_bytes), dtype=torch.uint8, device=env.device), cfg, lay)
+
+    def __len__(self):
+        return self.count
+
+    def arrays(self):
+        """Named torch views of the blob, with the names and shapes of split_state."""
+        N, S, F, V, lay = self.count, self.cfg.n_snakes, self.cfg.n_fruits, self.cfg.size + 2, self.lay
+
+        def arr(off, dtype, shape):
+            n = int(np.prod(shape)) * torch.empty(0, dtype=dtype).element_size()
+            return self.blob[off:off + n].view(dtype).reshape(shape)
+
+        out = {"t": arr(lay.off_t, torch.int32, (N,)), "spare": arr(lay.off_spare, torch.uint32, (N,)),
+               "draw_ctr": arr(lay.off_draw_ctr, torch.uint32, (N,)), "ep_ret": arr(lay.off_ep_ret, torch.float32, (N,)),
+               "ep_len": arr(lay.off_ep_len, torch.int32, (N,)), "len": arr(lay.off_len, torch.uint16, (N, S)),
+               "grow_to": arr(lay.off_grow_to, torch.uint16, (N, S)), "vel": arr(lay.off_vel, torch.uint8, (N, S)),
+               "body": arr(lay.off_body, torch.uint16, (N, S, lay.cap))}
+        if lay.fruit_is_grid:
+            out["fruit_grid"] = arr(lay.off_fruit, torch.uint8, (N, V * V))
+        else:
+            out["fruit"] = arr(lay.off_fruit, torch.uint16, (N, F))
+        return out
+
+    def numpy(self):
+        """The blob on the host (synchronises), usable with split_state(blob, states.lay, states.cfg)."""
+        return self.blob[:self.lay.total_bytes].cpu().numpy()
 
 
 def split_state(blob, lay, cfg):
