@@ -137,8 +137,9 @@ const char* snk_last_error(void);
 
 /* gym.make(id) + env.__init__(**kwargs) + env.seed()  (utils.py:37-39), for N envs at once.
  * snk_create reads ONE environment variable, SNK_DEBUG: a comma-separated key=value list of experiment switches
- * (kernel family, lane-path form, L2 policies ...; DESIGN.md section 4.7).  None of them changes results; unset is the
- * production configuration.  snk_create_ex takes that string explicitly (NULL = production) and reads no environment. */
+ * (force_kernel, lane, adaptive, alt_hi, epw, delta, restore_thr; DESIGN.md section 4.7).  None of them changes results;
+ * unset is the production configuration.  An unknown key, or a force_kernel / lane value that is not listed there, is
+ * SNK_EINVAL.  snk_create_ex takes that string explicitly (NULL = production) and reads no environment. */
 int snk_create(const snk_config* cfg, snk_handle** out);
 int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_handle** out);
 /* VecEnv.close()  (subproc_vec_env.py:73-83). */
@@ -349,8 +350,8 @@ int snk_launch_count(const snk_handle* h, uint64_t* out);
  * dynamic shared memory bytes, resident CTAs per SM, envs per CTA. */
 int snk_launch_info(const snk_handle* h, int32_t* out /*[6]*/);
 /* Which form of the lane path the NEXT step will launch (it follows the body-length regime, DESIGN.md 4.8):
- * out[0] = 0 fused kernel, 1 warp-specialised kernel, 2 two kernels (k_lane_logic + k_lane_paint), 3 two kernels with
- * k_lane_paint2, -1 not a lane-family configuration; out[1] = envs stepped per warp batch of the fused kernel;
+ * out[0] = 0 fused kernel, 1 warp-specialised kernel, 3 two kernels (k_lane_logic + k_lane_paint2), -1 not a lane-family
+ * configuration (2 is no longer reported); out[1] = envs stepped per warp batch of the fused kernel;
  * out[2] = envs per shared-memory image; out[3] = 1 when the handle switches forms by itself. */
 int snk_launch_form(const snk_handle* h, int32_t* out /*[4]*/);
 

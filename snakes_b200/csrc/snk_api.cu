@@ -117,21 +117,27 @@ struct snk_handle {
 static size_t align16(size_t x) { return (x + 15) & ~(size_t)15; }
 static int gcd(int a, int b) { return b ? gcd(b, a % b) : a; }
 
-// ---- experiment switches.  ONE string of comma-separated key=value pairs, given explicitly to snk_create_ex or, for
-// snk_create, read from the single environment variable SNK_DEBUG.  None changes results (all are parity-tested); an
-// unset / empty string is the production configuration.  Keys: force_kernel=lane|tile|rows|dense, lane=fused|ws|split,
-// store=stg, restore=tma, l2=<bits>, pdl=0, delta=0|1, restore_thr=<n>, logic_warps=<n>, rows_kb=<n>, rows_block=<n>, extra_smem=<bytes>.
-static bool dbg_get(const std::string& opts, const char* key, std::string* out) {
-  size_t pos = 0;
-  const size_t klen = strlen(key);
-  while (pos < opts.size()) {
+// ---- experiment switches.  ONE string of key=value pairs separated by ',', ' ' or ';', given explicitly to snk_create_ex
+// or, for snk_create, read from the single environment variable SNK_DEBUG.  None changes results (all are parity-tested);
+// an unset / empty string is the production configuration.  Keys: force_kernel=lane|tile|rows|dense, lane=fused|ws|split,
+// adaptive=0, alt_hi=<body cells>, epw=<n>, delta=0|1, restore_thr=<n>.  dbg_check rejects anything else.
+static std::vector<std::string> dbg_tokens(const std::string& opts) {
+  std::vector<std::string> out;
+  for (size_t pos = 0; pos < opts.size();) {
     size_t end = opts.find_first_of(", ;", pos);
     if (end == std::string::npos) end = opts.size();
-    if (end - pos > klen && opts.compare(pos, klen, key) == 0 && opts[pos + klen] == '=') {
-      *out = opts.substr(pos + klen + 1, end - pos - klen - 1);
+    if (end > pos) out.push_back(opts.substr(pos, end - pos));
+    pos = end + 1;
+  }
+  return out;
+}
+static bool dbg_get(const std::string& opts, const char* key, std::string* out) {
+  const size_t klen = strlen(key);
+  for (const std::string& t : dbg_tokens(opts)) {
+    if (t.size() > klen && t.compare(0, klen, key) == 0 && t[klen] == '=') {
+      *out = t.substr(klen + 1);
       return true;
     }
-    pos = end + 1;
   }
   return false;
 }
@@ -139,9 +145,31 @@ static int dbg_int(const std::string& opts, const char* key, int dflt) {
   std::string v;
   return dbg_get(opts, key, &v) ? atoi(v.c_str()) : dflt;
 }
-static bool dbg_is(const std::string& opts, const char* key, const char* value) {
-  std::string v;
-  return dbg_get(opts, key, &v) && v == value;
+// A stale or mistyped switch would otherwise be ignored and the run would measure the production path without a word.
+static int dbg_check(const std::string& opts) {
+  static const char* const keys[] = {"force_kernel", "lane", "adaptive", "alt_hi", "epw", "delta", "restore_thr"};
+  for (const std::string& t : dbg_tokens(opts)) {
+    const size_t eq = t.find('=');
+    const std::string key = t.substr(0, eq), val = eq == std::string::npos ? "" : t.substr(eq + 1);
+    bool ok = eq != std::string::npos && std::any_of(std::begin(keys), std::end(keys), [&](const char* k) { return key == k; });
+    if (key == "force_kernel") ok = ok && (val == "lane" || val == "tile" || val == "rows" || val == "dense");
+    if (key == "lane") ok = ok && (val == "fused" || val == "ws" || val == "split");
+    if (!ok) return fail(SNK_EINVAL, "unknown debug option '%s'", t.c_str());
+  }
+  return SNK_OK;
+}
+
+// Un-paint by zero-fill + border redraw (lane_restore / cta_restore) once a lane would walk more than restore_thr segments.
+// `threads` share an image buffer (32: a warp of the fused / ws kernel; 64: k_lane_paint2).  The restore costs each of
+// them one 16-byte store per 16 * threads bytes of image plus its share of one env's border units; a walked segment costs
+// about 16 instructions.  Measured on B200 (2x19x19, 131072 envs, fruit-seeking policy, sum of lengths 22): thresholds
+// 3 / 5 / 8 / 12 -> 145.9 / 145.1 / 146.8 / 152.9 us, always-walk 161.1 us; random actions (sum of lengths 4.4)
+// unchanged.  The restore_thr switch overrides it (0 = always walk).
+static int restore_threshold(const Params& p, int threads) {
+  const int U = (p.C & 1) ? 1 : 2, lanes_per_env = threads / p.TE;
+  const int border_units = (2 * (p.V * p.C + p.C) + (p.V - 3) * 2 * p.C) / U;
+  const int stores = (int)((size_t)p.TE * p.E / (16 * threads)) + border_units / lanes_per_env;
+  return stores / 16 < 3 ? 3 : stores / 16;
 }
 
 static int cfg_check(const snk_config* c) {
@@ -301,6 +329,7 @@ extern "C" int snk_destroy(snk_handle* h) {
 extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_handle** out) {
   int rc = cfg_check(cfg);
   if (rc) return rc;
+  if ((rc = dbg_check(debug_opts ? debug_opts : ""))) return rc;
   if (!out) return fail(SNK_EINVAL, "out is NULL");
   int n_dev = 0;
   CUDA_TRY(cudaGetDeviceCount(&n_dev));
@@ -364,7 +393,7 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
     const int unit = 16 / gcd(V * p.C, 16);
     // chunk size and CTA shape measured on B200 at 16 snakes on 64x64: 4 warps (1 producer + 3 consumers) give 7 CTAs
     // per SM, and 8 KB chunks beat 12 KB (32 768 envs: classic 1280 us, cut 1502 vs 1551 us)
-    const size_t lim = (size_t)dbg_int(dbg, "rows_kb", 8) * 1024;
+    const size_t lim = 8 * 1024;
     for (int r = unit; r <= V && ((size_t)r * V * p.C <= lim || !R); r += unit) { if ((size_t)r * V * p.C > 48 * 1024) break; R = r; }
   }
   plan.kind = TE ? KIND_LANE : smem_tile <= 110 * 1024 ? KIND_TILE : R ? KIND_ROWS : KIND_DENSE;
@@ -376,13 +405,6 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   if (force == "tile" && smem_tile <= 200 * 1024) plan.kind = KIND_TILE;
   if (force == "lane" && !TE) { snk_destroy(h); return fail(SNK_EINVAL, "lane kernel does not support this configuration"); }
   p.family = plan.kind == KIND_LANE;
-  p.store_mode = dbg_is(dbg, "store", "stg") ? 1 : 0;
-  p.restore_mode = dbg_is(dbg, "restore", "tma") ? 1 : 0;
-  {  // L2 policies (l2 = bit0 obs evict-first, bit1 records evict-last)
-    const int bits = dbg_int(dbg, "l2", 3);
-    p.obs_evict_first = bits & 1; p.rec_evict_last = (bits >> 1) & 1;
-  }
-  int logic_warps = 3;
   // lane path variants (lane=fused|ws|split): every warp steps 32 envs then streams their images (default: fastest
   // measured), warp-specialised single kernel, or two kernels
   {
@@ -401,39 +423,26 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
     const bool small_image = p.E < 2048 && (N + 31) / 32 >= 2LL * h->n_sm;
     plan.ws = plan.kind == KIND_LANE && (have_lv ? lv == "ws" : (small_image && S == 1));
     plan.split = plan.kind == KIND_LANE && (have_lv ? lv == "split" : (small_image && S > 1));
-    plan.pdl = dbg_int(dbg, "pdl", 1) != 0;
-    plan.paint2 = plan.split && dbg_int(dbg, "paint2", 1) != 0;
-    p.PW = 2;
-    logic_warps = dbg_int(dbg, "logic_warps", 3);
-    if (logic_warps < 1 || logic_warps > 3) logic_warps = 3;
   }
   p.CW = (p.cap - 1 + 15) / 16;
   // lane path geometry: te envs per warp image, epw envs stepped per warp batch (a multiple of te)
   auto lane_geometry = [&](int te, int epw) {
     p.TE = te; p.EPW = epw;
     p.tile_stride = (int)(((size_t)te * p.E + 127) & ~(size_t)127);
-    // un-paint by zero-fill + border redraw (lane_restore) once a lane would walk more than restore_thr segments:
-    // the restore costs one 16-byte store per 512 bytes of image plus the border units of one env spread over its
-    // LPE lanes; a walked segment costs about 16 instructions.  Measured on B200 (2x19x19, 131072 envs, fruit-seeking
-    // policy, sum of lengths 22): thresholds 3 / 5 / 8 / 12 -> 145.9 / 145.1 / 146.8 / 152.9 us, always-walk 161.1 us;
-    // random actions (sum of lengths 4.4) unchanged.  restore_thr overrides (0 = always walk).
-    const int U = (p.C & 1) ? 1 : 2, LPE = 32 / te;
-    const int border_units = (2 * (V * p.C + p.C) + (V - 3) * 2 * p.C) / U;
-    const int stores = (int)((size_t)te * p.E / 512) + border_units / LPE;
-    p.restore_thr = dbg_int(dbg, "restore_thr", stores / 16 < 3 ? 3 : stores / 16);
-    plan.smem = (size_t)(plan.paint2 ? 1 : 2) * p.tile_stride + (size_t)dbg_int(dbg, "extra_smem", 0);  // extra_smem: fewer resident image buffers per SM (experiment)
+    p.restore_thr = dbg_int(dbg, "restore_thr", restore_threshold(p, 32));
+    plan.smem = (size_t)(plan.split ? 1 : 2) * p.tile_stride;
     p.n_groups = (N + epw - 1) / epw;
   };
   if (plan.kind == KIND_LANE) {
     p.RW = (REC_SNAKE0 + 2 * S + 2 + 3) & ~3;
     p.W = 32;
-    plan.block = plan.ws ? 32 * (p.PW + logic_warps) : 64;
+    plan.block = plan.ws ? 32 * (WS_PAINT_WARPS + WS_LOGIC_WARPS) : 64;
     lane_geometry(TE, 32);
   } else if (plan.kind == KIND_TILE) {
     p.W = W; plan.block = 32 * W; plan.smem = smem_tile;
     p.n_groups = (N + W - 1) / W;
   } else if (plan.kind == KIND_ROWS) {
-    p.W = 1; p.R = R; plan.block = dbg_int(dbg, "rows_block", 128);  // 1 producer warp + 3 consumer warps
+    p.W = 1; p.R = R; plan.block = 128;  // 1 producer warp + 3 consumer warps
     p.tile_stride = (int)(((size_t)R * V * p.C + 127) & ~(size_t)127);
     plan.smem = 2 * (((size_t)p.VV + 127) & ~(size_t)127) + 2 * (size_t)p.tile_stride + (size_t)(p.RW + p.bm_words) * 4;
     p.n_groups = N;
@@ -463,8 +472,8 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   }
   {
     long long work = plan.kind == KIND_LANE ? (p.n_groups + 1) / 2 : p.n_groups;  // lane: 2 warps per CTA
-    if (plan.split) work = plan.paint2 ? (N + p.TE - 1) / p.TE : ((N + p.TE - 1) / p.TE + 1) / 2;  // paint kernels: one image per CTA / per warp
-    if (plan.ws) { const int LW = plan.block / 32 - p.PW; work = (p.n_groups + LW - 1) / LW; }
+    if (plan.split) work = (N + p.TE - 1) / p.TE;  // k_lane_paint2: one image per CTA
+    if (plan.ws) work = (p.n_groups + WS_LOGIC_WARPS - 1) / WS_LOGIC_WARPS;
     plan.grid = (int)(work < plan.max_grid ? work : plan.max_grid);
     if (plan.grid < 1) plan.grid = 1;
   }
@@ -483,16 +492,13 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
     if (eligible) {
       h->plan_alt = plan;
       LaunchPlan& alt = h->plan_alt;
-      alt.split = true; alt.paint2 = true; alt.block = 64;
+      alt.split = true; alt.block = 64;
       alt.smem = (size_t)p.tile_stride;
       if (snk_plan(cfg->rules, alt, h->n_sm, S, K) == cudaSuccess) {
         const long long work = (N + p.TE - 1) / p.TE;
         alt.grid = (int)(work < alt.max_grid ? work : alt.max_grid);
         if (alt.grid < 1) alt.grid = 1;
-        const int U = (p.C & 1) ? 1 : 2, LPE = 64 / p.TE;
-        const int border_units = (2 * (V * p.C + p.C) + (V - 3) * 2 * p.C) / U;
-        const int stores = (int)((size_t)p.TE * p.E / 1024) + border_units / LPE;
-        h->restore_thr_alt = dbg_int(dbg, "restore_thr", stores / 16 < 3 ? 3 : stores / 16);
+        h->restore_thr_alt = dbg_int(dbg, "restore_thr", restore_threshold(p, 64));
         // thresholds in body cells per env, hysteresis between them; measured at 2646 bytes of image per env and scaled
         // with the image (the larger the image, the longer the stream hides the fused kernel's logic)
         const int hi = dbg_int(dbg, "alt_hi", 0);
@@ -1439,7 +1445,7 @@ extern "C" int snk_launch_count(const snk_handle* h, uint64_t* out) {
 extern "C" int snk_launch_form(const snk_handle* h, int32_t* out /*[4]*/) {
   if (!h || !out) return fail(SNK_EINVAL, "NULL argument");
   const LaunchPlan& pl = (h->have_alt && h->use_alt) ? h->plan_alt : h->plan;
-  out[0] = pl.kind != KIND_LANE ? -1 : pl.ws ? 1 : pl.split ? (pl.paint2 ? 3 : 2) : 0;
+  out[0] = pl.kind != KIND_LANE ? -1 : pl.ws ? 1 : pl.split ? 3 : 0;
   out[1] = pl.kind == KIND_LANE ? h->p.EPW : 0; out[2] = pl.kind == KIND_LANE ? h->p.TE : 0; out[3] = h->have_alt ? 1 : 0;
   return SNK_OK;
 }
@@ -1448,6 +1454,6 @@ extern "C" int snk_launch_info(const snk_handle* h, int32_t* out /*[6]: kind, gr
   if (!h || !out) return fail(SNK_EINVAL, "NULL argument");
   const LaunchPlan& pl = (h->have_alt && h->use_alt) ? h->plan_alt : h->plan;
   out[0] = pl.kind; out[1] = pl.grid; out[2] = pl.block; out[3] = (int32_t)pl.smem;
-  out[4] = pl.occupancy; out[5] = pl.kind == KIND_LANE ? (pl.split ? (pl.paint2 ? h->p.TE : 2 * h->p.TE) : pl.ws ? 32 * (pl.block / 32 - h->p.PW) : 2 * h->p.EPW) : h->p.W;
+  out[4] = pl.occupancy; out[5] = pl.kind == KIND_LANE ? (pl.split ? h->p.TE : pl.ws ? 32 * WS_LOGIC_WARPS : 2 * h->p.EPW) : h->p.W;
   return SNK_OK;
 }

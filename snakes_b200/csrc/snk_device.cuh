@@ -46,12 +46,8 @@ struct Params {
   int family, CW;               // 0 = ring bodies (tile / dense kernels), 1 = chain-coded bodies (lane kernel); chain words per snake
   int TE, tile_stride;          // lane kernel: envs per warp image, bytes between warp images
   int EPW;                      // fused lane kernel: envs stepped per warp batch (32; 16/8/4 when the shard is too small to give every resident warp a batch)
-  int store_mode;               // lane kernel image store: 0 = TMA bulk copy, 1 = LDS.128 + STG.128 by the warp
-  int obs_evict_first, rec_evict_last;  // L2 policies: observation stream evict-first, env records evict-last
   int R;                        // rows kernel: image rows per chunk buffer
-  int PW;                       // warp-specialised lane kernel: paint warps per CTA (the others run game logic)
   u32 magicV, magicD;           // n / V == (n * magicV) >> 16 for n < V*V, n / D likewise for n < D*D (65536 / d + 1; exact while n * d < 65536)
-  int restore_mode;             // k_lane_paint2: how a long-body image buffer is restored: 0 = zero-fill + border redraw by the threads, 1 = TMA bulk load of the border template (experiment)
   int restore_thr;              // lane kernel: un-paint an image by zero-fill + border redraw when a lane would walk more segments than this (0 = always walk)
   int delta;                    // fused lane kernel, classic step into the own buffer: an image whose envs all have frame_ok stores only the 32-byte sectors the step can change
   int frame_own;                // this launch writes a complete image of every env into the handle's own observation buffer (lane_store writes it to frame_ok)

@@ -231,41 +231,24 @@ __global__ void __launch_bounds__(BLOCK) k_step_tile(const Params p) {
 }
 
 
-// Stream one painted image (TE envs, 16-byte aligned in HBM) out of shared memory: one TMA bulk
-// copy issued by lane 0 (which then waits until the engine has READ the image, so it may be
-// modified), or LDS.128 + STG.128 by all lanes; the last, partial image uses plain byte stores.
-#ifndef SNK_LANE_BULK
-#define SNK_LANE_BULK 16384  // bytes per bulk copy of the lane kernel's image store
-#endif
-__device__ __forceinline__ void store_image(const Params& p, const u8* tile, int tile_bytes, long long e0, int lane) {
+// Stream one painted image (TE envs, 16-byte aligned in HBM) out of shared memory, shared by the `nthr` threads that own
+// the buffer.  A whole image goes out as TMA bulk copies issued by thread 0, which then waits until the engine has READ
+// the image, so it may be modified; the last, partial image is copied byte by byte by all of them.
+constexpr int LANE_BULK = 16384;  // bytes per bulk copy
+__device__ __forceinline__ void store_image(const Params& p, const u8* tile, int tile_bytes, long long e0, int tid, int nthr) {
   const long long left = p.N - e0;
   u8* gdst = p.obs + e0 * (long long)p.E;
-  if (left >= p.TE && p.store_mode == 0) {
-    if (lane == 0) {
-      if (!p.obs_evict_first) {
-        for (int off = 0; off < tile_bytes; off += SNK_LANE_BULK)
-          bulk_store_s2g(gdst + off, tile + off, (u32)min(SNK_LANE_BULK, tile_bytes - off));
-      } else {
-        const u64 pol = l2_evict_first_policy();
-        for (int off = 0; off < tile_bytes; off += SNK_LANE_BULK)
-          bulk_store_s2g_hint(gdst + off, tile + off, (u32)min(SNK_LANE_BULK, tile_bytes - off), pol);
-      }
+  if (left >= p.TE) {
+    if (tid == 0) {
+      const u64 pol = l2_evict_first_policy();
+      for (int off = 0; off < tile_bytes; off += LANE_BULK)
+        bulk_store_s2g_hint(gdst + off, tile + off, (u32)min(LANE_BULK, tile_bytes - off), pol);
       bulk_commit();
       bulk_wait_read();
     }
-  } else if (left >= p.TE) {
-    const uint4* src = reinterpret_cast<const uint4*>(tile);
-    uint4* dst = reinterpret_cast<uint4*>(gdst);
-    const int n16 = tile_bytes / 16;
-    int i = lane;
-    for (; i + 96 < n16; i += 128) {  // 4 independent 16-byte loads in flight per lane
-      const uint4 a = src[i], b = src[i + 32], c = src[i + 64], d = src[i + 96];
-      __stcs(dst + i, a); __stcs(dst + i + 32, b); __stcs(dst + i + 64, c); __stcs(dst + i + 96, d);
-    }
-    for (; i < n16; i += 32) __stcs(dst + i, src[i]);
   } else {
     const int bytes = (int)left * p.E;
-    for (int i = lane; i < bytes; i += 32) gdst[i] = tile[i];
+    for (int i = tid; i < bytes; i += nthr) gdst[i] = tile[i];
   }
 }
 
@@ -336,50 +319,12 @@ __global__ void __launch_bounds__(128, (S <= 2 ? 7 : 1)) k_lane_logic(const Para
   publish_stats(p, s_stats, tid);
 }
 
-// k_lane_paint: the observation writer.  Each warp owns one shared-memory image of TE envs holding
-// the border and loops over images: the records of the NEXT image are prefetched, the current one is
-// painted (LPE lanes per env), handed to the TMA engine, and un-painted once the engine has read it.
-// The image buffers are the scarce resource (10 per SM at 2x19x19); this kernel keeps them busy.
-template <int S, int RULES, int K>
-__global__ void __launch_bounds__(64) k_lane_paint(const Params p) {
-  extern __shared__ __align__(128) u8 smem[];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, wpc = blockDim.x >> 5;
-  const int TE = p.TE, LPE = 32 / TE, E = p.E;
-  const int tile_bytes = TE * E;
-  u8* tile = smem + warp * p.tile_stride;
-  init_border_image(p, tile, lane);
-  __syncwarp();
-  const int slot = lane / LPE, sub = lane - slot * LPE;
-  u8* img = tile + slot * E;
-  const long long n_items = (p.N + TE - 1) / TE;
-  const long long stride = (long long)gridDim.x * wpc;
-  long long item = (long long)blockIdx.x * wpc + warp;
-  PaintEnv<S> cur = paint_env_from_memory<S>(p, item < n_items ? item * TE + slot : p.N);
-  while (item < n_items) {
-    const long long next = item + stride;
-    const PaintEnv<S> nxt = paint_env_from_memory<S>(p, next < n_items ? next * TE + slot : p.N);
-    const long long e0 = item * TE;
-    const bool restore = lane_wants_restore<S>(p, cur.len, LPE);
-    lane_paint<S, RULES, K>(p, cur, e0 + slot, sub, LPE, img, true);
-    fence_async_smem();
-    __syncwarp();
-    store_image(p, tile, tile_bytes, e0, lane);
-    __syncwarp();
-    lane_unpaint<S, RULES, K>(p, cur, e0 + slot, sub, LPE, tile, tile_bytes, img, lane, restore);
-    __syncwarp();
-    cur = nxt;
-    item = next;
-  }
-  if (lane == 0) bulk_wait_all();
-}
-
-
-// k_lane_paint2: the observation writer with TWO warps per image buffer.  The image buffers are what an SM runs out
-// of (10 at 2x19x19), so with one warp each the SM holds 10 warps and every one of them is a serial chain paint ->
-// bulk store -> wait -> un-paint; here the 64 threads of a CTA share one buffer (LPE = 64/TE lanes per env), which
-// halves the trips of every per-env loop (an image takes as long as its longest snake), halves the zero-fill of the
-// restore, and doubles the warps that cover each other's latencies.  CTA-wide barriers take the place of __syncwarp.
-// Launched programmatically behind k_lane_logic: the border image is fetched before griddepcontrol.wait.
+// k_lane_paint2: the observation writer, TWO warps per image buffer.  The image buffers are what an SM runs out of
+// (10 at 2x19x19); with one warp each, every warp would be a serial chain paint -> bulk store -> wait -> un-paint.
+// The 64 threads of a CTA share one buffer (LPE = 64/TE lanes per env), which halves the trips of every per-env loop
+// (an image takes as long as its longest snake) and the zero-fill of the restore, and doubles the warps that cover each
+// other's latencies.  CTA-wide barriers order the phases.  Launched programmatically behind k_lane_logic: the border
+// image is fetched before griddepcontrol.wait.
 template <int K>
 __device__ __forceinline__ void cta_restore(u8* tile, int n16, u8* img, int V, int sub, int LPE, int tid, int NT) {
   constexpr int C = 3 * K, U = (C & 1) ? 1 : 2, PU = 2 * C / U;
@@ -405,7 +350,8 @@ __device__ __forceinline__ void cta_restore(u8* tile, int n16, u8* img, int V, i
 
 // A lane's share of one image, worked out before any shared memory is touched: per snake the contiguous run
 // [i, i1) of segments this lane paints, the cell of segment i and the chain word holding the code that leads on from it.
-// Everything here reads global memory and registers only, so it runs while the TMA engine is still restoring the buffer.
+// Everything here reads global memory and registers only, so for a CTA's first image it runs while the TMA engine is still
+// fetching the border image into the buffer.
 template <int S>
 struct PaintRuns {
   int i[S], i1[S], pos[S];
@@ -483,11 +429,8 @@ __device__ __forceinline__ void cta_paint(const Params& p, const PaintEnv<S>& pe
   }
 }
 
-// Un-paint.  Short bodies: the same walk writes zeros.  Long bodies (`restore`): the threads zero-fill the buffer and redraw
-// the border (cta_restore), or -- restore=tma, an experiment that lost -- the TMA engine fetches the border-only image from
-// its L2-resident template back into the buffer while the CTA works on the global loads of its next image: no instructions
-// for a quarter of this kernel's instruction count, but the copy's latency is longer than the stores it replaces
-// (fruit-seeking stream 90.2 vs 88.7 us per step).  A CTA's last image is not un-painted at all.
+// Un-paint.  Short bodies: the same walk writes zeros.  Long bodies (`restore`): the threads zero-fill the buffer and
+// redraw the border (cta_restore).  A CTA's last image is not un-painted at all.
 template <int S, int RULES, int K>
 __global__ void __launch_bounds__(64) k_lane_paint2(const Params p) {
   extern __shared__ __align__(128) u8 smem[];
@@ -509,10 +452,8 @@ __global__ void __launch_bounds__(64) k_lane_paint2(const Params p) {
   long long item = blockIdx.x;
   asm volatile("griddepcontrol.wait;" ::: "memory");  // the records of this step come from k_lane_logic
   PaintEnv<S> cur = paint_env_from_memory<S>(p, item < n_items ? item * TE + slot : p.N);
-  u32 phase = 0;        // parity of the mbarrier phase the buffer's next fill completes
-  bool filling = true;  // a bulk load into the buffer is in flight (the border image, later the restores)
+  bool have_image = false;  // the border image has arrived in the buffer
   const int sh = 31 - __clz(LPE);
-  const bool tma_restore = p.restore_mode == 1;
   while (item < n_items) {
     const long long next = item + stride;
     const PaintEnv<S> nxt = paint_env_from_memory<S>(p, next < n_items ? next * TE + slot : p.N);
@@ -522,58 +463,21 @@ __global__ void __launch_bounds__(64) k_lane_paint2(const Params p) {
     for (int s = 0; s < S; ++s) trips += (cur.len[s] + LPE - 1) >> sh;
     const PaintRuns<S> runs = cta_paint_prepare<S>(p, cur, e0 + slot, sub, LPE);
     const bool restore = __syncthreads_or(p.restore_thr > 0 && trips > p.restore_thr);
-    if (filling) { mbar_wait(&s_bar, phase); phase ^= 1u; filling = false; }
+    if (!have_image) { mbar_wait(&s_bar, 0); have_image = true; }
     cta_paint<S, RULES, K>(p, cur, runs, e0 + slot, sub, LPE, img, true);
     fence_async_smem();
     __syncthreads();
-    if (p.N - e0 >= TE && p.store_mode == 0) {
-      if (tid == 0) {
-        u8* gdst = p.obs + e0 * (long long)E;
-        const u64 pol = l2_evict_first_policy();
-        for (int off = 0; off < tile_bytes; off += SNK_LANE_BULK) {
-          if (p.obs_evict_first) bulk_store_s2g_hint(gdst + off, tile + off, (u32)min(SNK_LANE_BULK, tile_bytes - off), pol);
-          else bulk_store_s2g(gdst + off, tile + off, (u32)min(SNK_LANE_BULK, tile_bytes - off));
-        }
-        bulk_commit();
-        bulk_wait_read();
-        if (restore && tma_restore && next < n_items) {  // the engine has read the image: let it put the border image back
-          mbar_expect_tx(&s_bar, (u32)tile_bytes);
-          for (int c = 0; c < TE / p.G; ++c) bulk_load_g2s(tile + c * p.G * E, p.tmpl, (u32)(p.G * E), &s_bar);
-        }
-      }
-    } else {  // partial last image, or the STG experiment switch
-      u8* gdst = p.obs + e0 * (long long)E;
-      const long long left = p.N - e0;
-      const int bytes = (int)(left < TE ? left : TE) * E;
-      if (left >= TE) {
-        const uint4* src = reinterpret_cast<const uint4*>(tile);
-        uint4* dst = reinterpret_cast<uint4*>(gdst);
-        for (int i = tid; i < bytes / 16; i += NT) __stcs(dst + i, src[i]);
-      } else {
-        for (int i = tid; i < bytes; i += NT) gdst[i] = tile[i];
-      }
-      if (restore && tma_restore && next < n_items) {
-        __syncthreads();
-        if (tid == 0) {
-          mbar_expect_tx(&s_bar, (u32)tile_bytes);
-          for (int c = 0; c < TE / p.G; ++c) bulk_load_g2s(tile + c * p.G * E, p.tmpl, (u32)(p.G * E), &s_bar);
-        }
-      }
-    }
+    store_image(p, tile, tile_bytes, e0, tid, NT);
     if (next < n_items) {  // the last image of a CTA leaves its buffer as it is
-      if (restore && tma_restore) {
-        filling = true;  // waited for before the next paint; nobody touches the buffer until then
-      } else {
-        __syncthreads();
-        if (restore) cta_restore<K>(tile, tile_bytes >> 4, img, p.V, sub, LPE, tid, NT);
-        else cta_paint<S, RULES, K>(p, cur, runs, e0 + slot, sub, LPE, img, false);
-        __syncthreads();
-      }
+      __syncthreads();
+      if (restore) cta_restore<K>(tile, tile_bytes >> 4, img, p.V, sub, LPE, tid, NT);
+      else cta_paint<S, RULES, K>(p, cur, runs, e0 + slot, sub, LPE, img, false);
+      __syncthreads();
     }
     cur = nxt;
     item = next;
   }
-  if (filling) mbar_wait(&s_bar, phase);  // never leave with a bulk copy into our shared memory in flight
+  if (!have_image) mbar_wait(&s_bar, 0);  // never leave with a bulk copy into our shared memory in flight
   if (tid == 0) bulk_wait_all();
   // the dependent launch is released only once this CTA's images have left: with a policy kernel between two steps an
   // earlier release (before the drain, or before the last un-paint that this kernel no longer does) cost 5 us per step
@@ -590,17 +494,17 @@ __global__ void __launch_bounds__(64) k_lane_paint2(const Params p) {
 // need, read its records back from L2, paint -> stream out -> un-paint.  Logic never waits, so the
 // record / action latency of later batches hides under the HBM write stream of earlier ones.
 template <int S, int RULES, int K>
-__global__ void __launch_bounds__(160, 5) k_step_lane_ws(const Params p) {
+__global__ void __launch_bounds__(32 * (WS_PAINT_WARPS + WS_LOGIC_WARPS), 5) k_step_lane_ws(const Params p) {
+  constexpr int PW = WS_PAINT_WARPS, LW = WS_LOGIC_WARPS;
   extern __shared__ __align__(128) u8 smem[];
   __shared__ double s_stats[SNK_NSTATS];
-  __shared__ int s_ready[8];
-  __shared__ u32 s_bm[5][SPAWN_WORDS];  // per warp: scratch of group_spawn (logic warps)
+  __shared__ int s_ready[LW];
+  __shared__ u32 s_bm[PW + LW][SPAWN_WORDS];  // per warp: scratch of group_spawn (logic warps)
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int PW = p.PW, LW = (blockDim.x >> 5) - PW;
   const int TE = p.TE, LPE = 32 / TE, E = p.E, IPB = 32 / TE;  // images per 32-env batch
   if (tid < SNK_NSTATS) s_stats[tid] = 0.0;
   peer_push(p, tid);  // the running sums as of the previous step, to every peer (posted stores)
-  if (tid < 8) s_ready[tid] = 0;
+  if (tid < LW) s_ready[tid] = 0;
   __syncthreads();
   const long long n_batches = (p.N + 31) / 32;
   LaneStats st = {0, 0, 0, 0, 0, 0, 0, 0};
@@ -628,7 +532,7 @@ __global__ void __launch_bounds__(160, 5) k_step_lane_ws(const Params p) {
         lane_paint<S, RULES, K>(p, pe, e0 + slot, sub, LPE, img, true);
         fence_async_smem();
         __syncwarp();
-        store_image(p, tile, tile_bytes, e0, lane);
+        store_image(p, tile, tile_bytes, e0, lane, 32);
         __syncwarp();
         lane_unpaint<S, RULES, K>(p, pe, e0 + slot, sub, LPE, tile, tile_bytes, img, lane, restore);
         __syncwarp();
@@ -675,8 +579,10 @@ __global__ void __launch_bounds__(160, 5) k_step_lane_ws(const Params p) {
 // k_step_lane: see snk_lane.cuh.  A warp is an independent worker: 32 envs of logic (one per lane),
 // then 32/TE rounds of paint -> TMA bulk store -> un-paint on its private image.  No __syncthreads.
 // With Params::delta an image whose envs all qualify (delta_eligible) goes out as its changed sectors instead (delta_store).
+// Three and four snakes: left to itself ptxas caps the kernel at 168 registers and spills (up to 136 bytes); asking for
+// 4 CTAs per SM (up to 256 registers) keeps it spill-free.  One and two snakes keep the compiler's own choice.
 template <int S, int RULES, int K>
-__global__ void __launch_bounds__(64) k_step_lane(const Params p) {
+__global__ void __launch_bounds__(64, (S >= 3 ? 4 : 0)) k_step_lane(const Params p) {
   extern __shared__ __align__(128) u8 smem[];
   __shared__ double s_stats[SNK_NSTATS];
   __shared__ __align__(8) u64 s_bar[2];
@@ -769,7 +675,7 @@ __global__ void __launch_bounds__(64) k_step_lane(const Params p) {
         const DeltaOld<S> po = delta_old_from_lane<S>(old, q * TE + slot);
         delta_store<S, K>(p, pe, po, slot, sub, LPE, tile, (int)min((long long)TE, p.N - e0) * E, e0);
       } else {
-        store_image(p, tile, tile_bytes, e0, lane);
+        store_image(p, tile, tile_bytes, e0, lane, 32);
       }
       __syncwarp();
 #ifdef SNK_PHASE_TIMING
@@ -1667,34 +1573,24 @@ cudaError_t launch_rules(const Params& p, const LaunchPlan& plan, cudaStream_t s
   if (p.S == s && p.K == k) {                                                                                \
     if (plan.ws) {                                                                                           \
       k_step_lane_ws<s, RULES, k><<<plan.grid, plan.block, plan.smem, stream>>>(p);                          \
-    } else if (!plan.split) {                                                                                \
-      cudaLaunchConfig_t cfg = {};                                                                           \
-      cfg.gridDim = dim3(plan.grid); cfg.blockDim = dim3(plan.block); cfg.dynamicSmemBytes = plan.smem;      \
-      cfg.stream = stream;                                                                                   \
-      cudaLaunchAttribute attr[1];                                                                           \
-      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;                                       \
-      attr[0].val.programmaticStreamSerializationAllowed = plan.pdl ? 1 : 0;                                 \
-      cfg.attrs = attr; cfg.numAttrs = 1;                                                                    \
-      return cudaLaunchKernelEx(&cfg, k_step_lane<s, RULES, k>, p);                                          \
-    } else if (!plan.paint2) {                                                                               \
-      if (p.mode != MODE_OBSERVE) k_lane_logic<s, RULES><<<(unsigned)((p.N + 127) / 128), 128, 0, stream>>>(p); \
-      k_lane_paint<s, RULES, k><<<plan.grid, plan.block, plan.smem, stream>>>(p);                            \
-    } else {                                                                                                 \
-      cudaLaunchConfig_t cfg = {};                                                                           \
-      cfg.stream = stream;                                                                                   \
-      cudaLaunchAttribute attr[1];                                                                           \
-      attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;                                       \
-      attr[0].val.programmaticStreamSerializationAllowed = plan.pdl ? 1 : 0;                                 \
-      cfg.attrs = attr; cfg.numAttrs = 1;                                                                    \
-      if (p.mode != MODE_OBSERVE) {                                                                          \
-        cfg.gridDim = dim3((unsigned)((p.N + 127) / 128)); cfg.blockDim = dim3(128); cfg.dynamicSmemBytes = 0; \
-        cudaError_t e1 = cudaLaunchKernelEx(&cfg, k_lane_logic<s, RULES>, p);                                \
-        if (e1 != cudaSuccess) return e1;                                                                    \
-      }                                                                                                      \
-      cfg.gridDim = dim3(plan.grid); cfg.blockDim = dim3(plan.block); cfg.dynamicSmemBytes = plan.smem;      \
-      return cudaLaunchKernelEx(&cfg, k_lane_paint2<s, RULES, k>, p);                                        \
+      return cudaGetLastError();                                                                             \
     }                                                                                                        \
-    return cudaGetLastError();                                                                               \
+    /* programmatic launches: a kernel's prologue overlaps the tail of the launch before it */               \
+    cudaLaunchConfig_t cfg = {};                                                                             \
+    cfg.gridDim = dim3(plan.grid); cfg.blockDim = dim3(plan.block); cfg.dynamicSmemBytes = plan.smem;        \
+    cfg.stream = stream;                                                                                     \
+    cudaLaunchAttribute attr[1];                                                                             \
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;                                         \
+    attr[0].val.programmaticStreamSerializationAllowed = 1;                                                  \
+    cfg.attrs = attr; cfg.numAttrs = 1;                                                                      \
+    if (!plan.split) return cudaLaunchKernelEx(&cfg, k_step_lane<s, RULES, k>, p);                           \
+    if (p.mode != MODE_OBSERVE) {                                                                            \
+      cudaLaunchConfig_t lc = cfg;                                                                           \
+      lc.gridDim = dim3((unsigned)((p.N + 127) / 128)); lc.blockDim = dim3(128); lc.dynamicSmemBytes = 0;    \
+      cudaError_t e1 = cudaLaunchKernelEx(&lc, k_lane_logic<s, RULES>, p);                                   \
+      if (e1 != cudaSuccess) return e1;                                                                      \
+    }                                                                                                        \
+    return cudaLaunchKernelEx(&cfg, k_lane_paint2<s, RULES, k>, p);                                          \
   }
     LANE_COMBOS(X)
 #undef X
@@ -1738,13 +1634,9 @@ static cudaError_t plan_lane(LaunchPlan& plan, int& occ) {
     if ((err = cudaFuncSetAttribute(k_step_lane_ws<S, RULES, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_lane_ws<S, RULES, K>, plan.block, plan.smem);
   }
-  if (plan.split && plan.paint2) {
+  if (plan.split) {
     if ((err = cudaFuncSetAttribute(k_lane_paint2<S, RULES, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_lane_paint2<S, RULES, K>, plan.block, plan.smem);
-  }
-  if (plan.split) {
-    if ((err = cudaFuncSetAttribute(k_lane_paint<S, RULES, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_lane_paint<S, RULES, K>, plan.block, plan.smem);
   }
   if ((err = cudaFuncSetAttribute(k_step_lane<S, RULES, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
   return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_lane<S, RULES, K>, plan.block, plan.smem);

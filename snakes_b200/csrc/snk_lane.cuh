@@ -576,17 +576,12 @@ __device__ __forceinline__ LaneRaw<S> lane_fetch(const Params& p, long long e, b
   constexpr int RW = LaneRec<S>::RW;
   LaneRaw<S> raw;
   const uint4* g = reinterpret_cast<const uint4*>(p.rec + e * RW);
-  if (p.rec_evict_last) {  // keep the records L2-resident across steps (they are re-read by the next launch)
-    u64 pol;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
+  u64 pol;  // keep the records L2-resident across steps (they are re-read by the next launch)
+  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
 #pragma unroll
-    for (int i = 0; i < RW / 4; ++i)
-      asm volatile("ld.global.L2::cache_hint.v4.u32 {%0, %1, %2, %3}, [%4], %5;"
-                   : "=r"(raw.v[i].x), "=r"(raw.v[i].y), "=r"(raw.v[i].z), "=r"(raw.v[i].w) : "l"(g + i), "l"(pol));
-  } else {
-#pragma unroll
-    for (int i = 0; i < RW / 4; ++i) raw.v[i] = g[i];
-  }
+  for (int i = 0; i < RW / 4; ++i)
+    asm volatile("ld.global.L2::cache_hint.v4.u32 {%0, %1, %2, %3}, [%4], %5;"
+                 : "=r"(raw.v[i].x), "=r"(raw.v[i].y), "=r"(raw.v[i].z), "=r"(raw.v[i].w) : "l"(g + i), "l"(pol));
   raw.frame = p.frame_ok[e] != 0;
   raw.act = 0;
   if (with_actions) {
@@ -643,17 +638,12 @@ __device__ __forceinline__ void lane_store(const Params& p, long long e, const L
   r[REC_SNAKE0 + 2 * S + 1] = (u32)env.fruit[2] | ((u32)env.fruit[3] << 16);
   uint4* g = reinterpret_cast<uint4*>(p.rec + e * RW);
   p.frame_ok[e] = (u8)p.frame_own;
-  if (p.rec_evict_last) {
-    u64 pol;
-    asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
+  u64 pol;
+  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
 #pragma unroll
-    for (int i = 0; i < RW / 4; ++i)
-      asm volatile("st.global.L2::cache_hint.v4.u32 [%0], {%1, %2, %3, %4}, %5;" ::"l"(g + i), "r"(r[4 * i]), "r"(r[4 * i + 1]),
-                   "r"(r[4 * i + 2]), "r"(r[4 * i + 3]), "l"(pol) : "memory");
-  } else {
-#pragma unroll
-    for (int i = 0; i < RW / 4; ++i) g[i] = make_uint4(r[4 * i], r[4 * i + 1], r[4 * i + 2], r[4 * i + 3]);
-  }
+  for (int i = 0; i < RW / 4; ++i)
+    asm volatile("st.global.L2::cache_hint.v4.u32 [%0], {%1, %2, %3, %4}, %5;" ::"l"(g + i), "r"(r[4 * i]), "r"(r[4 * i + 1]),
+                 "r"(r[4 * i + 2]), "r"(r[4 * i + 3]), "l"(pol) : "memory");
 }
 
 // all C = 3K bytes of one pixel: snake s seen by every view k (self colours iff s == k)
@@ -863,25 +853,21 @@ __device__ __forceinline__ DeltaOld<S> delta_old_from_lane(const DeltaOld<S>& o,
 }
 
 // One sector: two 16-byte shared loads (an image starts 16-byte aligned in HBM, so a sector is 16-byte aligned in
-// shared memory), one 32-byte global store (STG.E.ENL2.256).  The data is in registers before the store issues, so the
-// image may be un-painted right after.
-__device__ __forceinline__ void store_sector(u8* g, const u8* s, bool hint, u64 pol) {
+// shared memory), one 32-byte global store (STG.E.ENL2.256) with the observation stream's L2 evict-first policy `pol`.
+// The data is in registers before the store issues, so the image may be un-painted right after.
+__device__ __forceinline__ void store_sector(u8* g, const u8* s, u64 pol) {
   const uint4 a = *reinterpret_cast<const uint4*>(s), b = *reinterpret_cast<const uint4*>(s + 16);
-  if (hint)
-    asm volatile("st.global.L2::cache_hint.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8}, %9;" ::"l"(g), "r"(a.x), "r"(a.y), "r"(a.z),
-                 "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w), "l"(pol) : "memory");
-  else
-    asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"l"(g), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w), "r"(b.x),
-                 "r"(b.y), "r"(b.z), "r"(b.w) : "memory");
+  asm volatile("st.global.L2::cache_hint.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8}, %9;" ::"l"(g), "r"(a.x), "r"(a.y), "r"(a.z),
+               "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w), "l"(pol) : "memory");
 }
 
 // the one or two sectors of the C-byte pixel at byte `off` of the image; `a` = the image's HBM address mod 32.  A sector
 // outside [0, bytes) is skipped: only a border cell could produce one, and those are never painted.
 template <int C>
-__device__ __forceinline__ void delta_pixel(u8* g, const u8* tile, int bytes, int a, int off, bool hint, u64 pol) {
+__device__ __forceinline__ void delta_pixel(u8* g, const u8* tile, int bytes, int a, int off, u64 pol) {
   const int r0 = ((off + a) & ~31) - a, r1 = ((off + C - 1 + a) & ~31) - a;
-  if ((u32)r0 <= (u32)(bytes - 32)) store_sector(g + r0, tile + r0, hint, pol);
-  if (r1 != r0 && (u32)r1 <= (u32)(bytes - 32)) store_sector(g + r1, tile + r1, hint, pol);
+  if ((u32)r0 <= (u32)(bytes - 32)) store_sector(g + r0, tile + r0, pol);
+  if (r1 != r0 && (u32)r1 <= (u32)(bytes - 32)) store_sector(g + r1, tile + r1, pol);
 }
 
 // Store the sectors of one env of the image.  Its paint items -- the new and the old classic fruits, then per snake the
@@ -897,9 +883,8 @@ __device__ __forceinline__ void delta_store(const Params& p, const PaintEnv<S>& 
   const long long t0 = e0 * (long long)p.E;
   u8* g = p.obs + t0;
   const int a = (int)(t0 & 31), base = slot * p.E;
-  const bool hint = p.obs_evict_first;
-  u64 pol = 0;
-  if (hint) asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
+  u64 pol;
+  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
   // A snake that moved (and was neither killed nor reset) has old segment i = new segment i + 1: of its old body only the
   // segments from new length - 1 on (the popped tail) are not in the new one.  `skip[s]` old segments are left out.
   int n = 2 * F, skip[S];
@@ -934,6 +919,6 @@ __device__ __forceinline__ void delta_store(const Params& p, const PaintEnv<S>& 
       }
       pid = head - codes_disp(w, V, i);
     }
-    if (pid >= 0) delta_pixel<C>(g, tile, bytes, a, base + pid * C, hint, pol);
+    if (pid >= 0) delta_pixel<C>(g, tile, bytes, a, base + pid * C, pol);
   }
 }

@@ -8,13 +8,13 @@
 struct Params;
 struct PeerArgs;
 enum { KIND_LANE = 0, KIND_TILE = 1, KIND_DENSE = 2, KIND_ROWS = 3 };
+// k_step_lane_ws: paint warps (each owning a shared-memory image) and logic warps per CTA
+enum { WS_PAINT_WARPS = 2, WS_LOGIC_WARPS = 3 };
 
 struct LaunchPlan {
   int kind;         // KIND_LANE (lane per env, chain bodies), KIND_TILE (warp per env), KIND_ROWS / KIND_DENSE (CTA per env)
   bool ws;          // lane path as ONE warp-specialised kernel (k_step_lane_ws): paint warps + logic warps per CTA
-  bool pdl;         // fused lane kernel launched with programmatic stream serialization (prologue overlaps the previous launch's tail)
-  bool split;       // lane path as two kernels: k_lane_logic (thread per env) + k_lane_paint (observation writer)
-  bool paint2;      // split form: the observation writer is k_lane_paint2 (two warps per image buffer, programmatic launches)
+  bool split;       // lane path as two kernels: k_lane_logic (thread per env) + k_lane_paint2 (observation writer)
   int grid, block;
   size_t smem;
   int occupancy;    // resident CTAs per SM

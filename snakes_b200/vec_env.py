@@ -793,8 +793,8 @@ class SnakeVecEnv(object):
         d["kernel"] = ("k_step_lane", "k_step_tile", "k_step_dense", "k_step_rows")[d["kind"]]
         f = (C.c_int32 * 4)()
         _lib.check(self._L.snk_launch_form(self._h, f))
-        if d["kind"] == 0:  # the lane path has four forms; the handle may move between the first and the last by itself
-            d["kernel"] = ("k_step_lane", "k_step_lane_ws", "k_lane_logic + k_lane_paint", "k_lane_logic + k_lane_paint2")[f[0]]
+        if d["kind"] == 0:  # the lane path has three forms; the handle may move between the fused and the two-kernel one by itself
+            d["kernel"] = {0: "k_step_lane", 1: "k_step_lane_ws", 3: "k_lane_logic + k_lane_paint2"}[f[0]]
             d["envs_per_warp_batch"], d["envs_per_image"], d["adaptive"] = int(f[1]), int(f[2]), bool(f[3])
         return d
 

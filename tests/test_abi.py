@@ -82,6 +82,19 @@ def test_bad_arguments_are_reported_not_crashed(L):
     assert lib.snk_comm_init(None, None, 1, 0) == -1 and lib.snk_comm_unique_id(None) == -1
     assert lib.snk_host_alloc(None, 16, None, None) == -1 and lib.snk_dump_state_range(None, 0, 1, None, 0) == -1
     assert set(L.DEVERR) == {1, 2, 4, 8, 16}
+    # the debug string: an unknown key or an unlisted value is rejected by name before any CUDA call
+    ok_cfg = L.make_config(4, 10, 2)
+    for opts in (b"store=stg", b"paint2=0", b"lane=bogus", b"lane=split,restor_thr=1"):
+        out = C.c_void_p()
+        assert lib.snk_create_ex(C.byref(ok_cfg), opts, C.byref(out)) == -1 and not out.value
+        assert opts.split(b",")[-1] in lib.snk_last_error()
+    # an empty string and known keys get past that check (without a GPU, creation then fails with SNK_ECUDA)
+    for opts in (b"", b"lane=split,restore_thr=2,epw=8"):
+        out = C.c_void_p()
+        rc = lib.snk_create_ex(C.byref(ok_cfg), opts, C.byref(out))
+        assert rc in (0, -2), (opts, rc, lib.snk_last_error())
+        if rc == 0:
+            lib.snk_destroy(out)
 
 
 def test_product_does_not_import_oracle():

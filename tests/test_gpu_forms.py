@@ -1,7 +1,7 @@
-"""The forms of the lane path added in round 2, each against the C oracle through the C ABI:
-the two-kernel form with k_lane_paint2 (two warps per image buffer) and the grouped death test of
-k_lane_logic, the regime switch between the fused and the two-kernel form in mid-run, the small-shard
-batches of 16 / 8 / 4 envs per warp, and the two occupancy sources of the scripted policy kernel.
+"""The forms of the lane path, each against the C oracle through the C ABI: the two-kernel form
+(k_lane_logic with its grouped death test, then k_lane_paint2 with two warps per image buffer), the
+regime switch between the fused and the two-kernel form in mid-run, the small-shard batches of
+16 / 8 / 4 envs per warp, and the two occupancy sources of the scripted policy kernel.
 Reference semantics: gym_snake/envs/snake_multiple_test.py:97-232 (via oracle/snake_oracle.c)."""
 import numpy as np
 import pytest
@@ -55,18 +55,6 @@ def test_two_kernel_form_other_rules(sb, rules):
         _compare_step(env, co, a, "%s split step %d" % (rules, t), check_state=(t % 30 == 29))
     env.check_errors()
     env.close()
-
-
-def test_old_paint_kernel_still_matches(sb):
-    """paint2=0 keeps k_lane_paint (one warp per image buffer) selectable for A/B runs."""
-    _scripted_run(sb, 600, 120, "lane=split,paint2=0", dict(size=19, n_snakes=2, rules="classic", seed=2))
-
-
-def test_tma_restore_switch_still_matches(sb):
-    """restore=tma: the painter's long-body buffers are restored by a TMA bulk load of the border template instead of the
-    threads' zero-fill (a measured alternative that lost; kept selectable); ragged last image included."""
-    _scripted_run(sb, 601, 160, "lane=split,restore=tma", dict(size=19, n_snakes=2, rules="classic", seed=2))
-    _scripted_run(sb, 333, 120, "lane=split,restore=tma,restore_thr=1", dict(size=10, n_snakes=3, rules="classic", seed=6))
 
 
 def test_regime_switch_mid_run(sb):

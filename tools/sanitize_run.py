@@ -22,8 +22,6 @@ def run(N, steps, debug=None, scripted=False, **kw):
 run(333, 40, size=19, n_snakes=2).close()
 run(333, 40, "lane=ws", size=19, n_snakes=2).close()
 run(333, 120, "lane=split", scripted=True, size=19, n_snakes=2).close()             # long bodies: cta_restore
-run(333, 120, "lane=split,restore=tma", scripted=True, size=19, n_snakes=2).close() # long bodies: TMA restore
-run(333, 60, "lane=split,paint2=0", scripted=True, size=19, n_snakes=2).close()
 run(70, 40, "epw=4", size=10, n_snakes=2).close()                                   # small-shard batches
 run(200, 60, size=10, n_snakes=3, rules="cut").close()
 run(200, 60, "lane=split", size=10, n_snakes=3, rules="cut").close()
