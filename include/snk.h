@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SNK_VERSION 300 /* 0.3.0 */
+#define SNK_VERSION 310 /* 0.3.1 */
 
 /* error codes */
 #define SNK_OK 0
@@ -55,6 +55,24 @@ extern "C" {
 /* observation modes */
 #define SNK_OBS_NATIVE 0   /* uint8 [N][V][V][3K], the reference's get_multi_snake_ob() stacked by np.stack */
 #define SNK_OBS_ATARI84 1  /* uint8 [N][84][84][3K]: utils.py:27-31 WarpFrame; exact when 84 % V == 0 */
+#define SNK_OBS_GRID 2     /* uint8 [N][V][V]: one cell code (SNK_CELL_*) per padded cell, row-major like the native image;
+                            * snk_buffers reports obs_h = obs_w = V, obs_c = 1, obs_bytes = N*V*V.  Lossless for all K views:
+                            * snk_expand_views turns it into the native image or any run of its views. */
+
+/* Cell codes of SNK_OBS_GRID.  They grow in the reference's paint order (get_ob_for_snake :35-58: fruits, then the
+ * snakes by index, body then head, then the border), so "a later item overwrites an earlier one" holds code by code,
+ * and S <= 32 keeps every code in a byte.  Code 2 is unused.  A fruit outside the board (adversarial rules: a dead body's
+ * cells become fruit, and a head may die one step outside) lies under the border, as in the reference.
+ * View k (0 <= k < K) of a cell, as the native observation draws it:
+ *   SNK_CELL_EMPTY  black (0, 0, 0)            SNK_CELL_FRUIT  red (255, 0, 0)       SNK_CELL_WALL  white (255, 255, 255)
+ *   code >= 3       snake s = (code - 3) >> 1, head if (code - 3) & 1, else body; the self colours (green: body (0, 204, 0),
+ *                   head (191, 242, 191)) when s == k, the other colours (blue: body (0, 51, 204), head (128, 154, 230))
+ *                   otherwise.  Views k >= S have no self snake. */
+#define SNK_CELL_EMPTY 0
+#define SNK_CELL_FRUIT 1
+#define SNK_CELL_BODY(s) (3 + 2 * (s))
+#define SNK_CELL_HEAD(s) (4 + 2 * (s))
+#define SNK_CELL_WALL 255
 
 /* RNG modes */
 #define SNK_RNG_PHILOX 0   /* Philox4x32-10, key (seed, global env id), counter = per-env draw index */
@@ -72,7 +90,8 @@ typedef struct snk_config {
   int32_t rules;       /* SNK_RULES_* */
   int32_t max_steps;   /* episode cap, reference 2000 (snake_multiple_test.py:195); 0 = 2000 */
   int32_t auto_reset;  /* 1 = SubprocVecEnv worker contract (baselines/common/vec_env/subproc_vec_env.py:13-16) */
-  int32_t obs_mode;    /* SNK_OBS_* */
+  int32_t obs_mode;    /* SNK_OBS_*; SNK_OBS_GRID takes none of the debug switches lane, delta, epw, adaptive, alt_hi,
+                        * force_kernel=tile|dense (snk_create_ex fails with SNK_EINVAL and names the switch) */
   int32_t device;      /* CUDA device ordinal */
   int32_t rng_mode;    /* SNK_RNG_* */
   int64_t num_envs;    /* N, envs held by THIS handle */
@@ -95,8 +114,8 @@ typedef struct snk_buffers {
   float* d_episode_return; /* [N]    valid where d_done: Monitor 'r' */
   int32_t* d_episode_len;  /* [N]    valid where d_done: Monitor 'l' */
   double* d_stats;         /* [SNK_NSTATS] running sums since snk_reset_stats */
-  size_t obs_bytes;        /* N*H*W*3K */
-  int32_t obs_h, obs_w, obs_c;
+  size_t obs_bytes;        /* N*H*W*3K (SNK_OBS_GRID: N*V*V) */
+  int32_t obs_h, obs_w, obs_c;  /* bytes per pixel: 3K, or 1 for SNK_OBS_GRID */
   uint8_t* d_info_block;   /* d_done, d_num_alive, d_episode_return, d_episode_len live in this one block (in this */
   size_t info_block_bytes; /* order, each 16-byte aligned): one copy snapshots a step's infos */
 } snk_buffers;
@@ -167,6 +186,7 @@ int snk_step_host(snk_handle* h, const int8_t* h_actions, uint8_t* h_obs, float*
  * (1 <= n_views_out <= 4, or 0 / K for all views).  The reference learner keeps view 0 alone in its rollout
  * (ppo_multi_agent_new.py:181, `obs[..., 0:3]`), so with n_views_out = 1 the D2H copy carries 1/K of the bytes; the
  * views are gathered on the device by a small kernel first. */
+/* SNK_OBS_GRID: h_obs receives the [N][V][V] grid; n_views_out other than 0 is SNK_EINVAL (expand on the device first). */
 int snk_step_host_views(snk_handle* h, const int8_t* h_actions, uint8_t* h_obs, int32_t n_views_out, float* h_reward,
                         uint8_t* h_done, uint8_t* h_num_alive, void* stream);
 /* VecEnv.step_async proper: enqueues the H2D copy, the step and the D2H copies and returns; the caller synchronises
@@ -210,6 +230,7 @@ int snk_set_obs_target(snk_handle* h, uint8_t* d_obs, size_t bytes);
  * transient observation buffer.  NULL switches it off.  (A gather kernel behind the step kernel: the interleaved
  * [N][H][W][3K] layout of the reference is what the step kernel streams out; see DESIGN.md section 4.9 for why a planar
  * store was not adopted.) */
+/* SNK_OBS_GRID: SNK_EINVAL (the grid is already compact; snk_expand_views with n_views = 1 gives view 0). */
 int snk_set_main_view_target(snk_handle* h, uint8_t* d_main, size_t bytes);
 
 /* T steps back to back into a caller-owned rollout buffer, no host round trip: step t reads
@@ -248,6 +269,16 @@ int snk_graph_destroy(snk_graph* g);
 int snk_gae(const float* d_rewards, const float* d_values, const uint8_t* d_dones, const float* d_last_values,
             const uint8_t* d_last_dones, double gamma, double lam, int32_t T, int64_t N, float* d_advs,
             float* d_returns, int32_t device, void* stream);
+
+/* SNK_OBS_GRID -> RGB views.  d_grid: uint8 [n][V][V] cell codes (V = size + 2, 3 <= V <= 256), e.g. a handle's grid
+ * observations, a [T][N][V][V] rollout (n = T*N) or a gathered minibatch.  d_out: uint8 [n][V][V][3 n_views] receives
+ * views first_view .. first_view + n_views - 1 of every cell (the colour rule at SNK_CELL_*), byte-identical to those
+ * channels of the native observation of the same state; with first_view = 0 and n_views = K it IS the native
+ * observation.  0 <= first_view, 1 <= n_views, first_view + n_views <= 32.  Not tied to a handle; stream-ordered on
+ * `stream` on `device`, no allocation, no synchronisation, so it can be recorded into a CUDA graph.  16-byte aligned
+ * buffers take the vector path; any alignment is accepted. */
+int snk_expand_views(const uint8_t* d_grid, int64_t n, int32_t size, int32_t first_view, int32_t n_views,
+                     uint8_t* d_out, int32_t device, void* stream);
 
 /* Replay mode: per-env tapes of the reference's np_random.randint draws
  * (snake_multiple_test.py:200, :215).  CSR: env i owns vals/bounds[offsets[i] .. offsets[i+1]).
@@ -350,7 +381,8 @@ int snk_launch_count(const snk_handle* h, uint64_t* out);
  * dynamic shared memory bytes, resident CTAs per SM, envs per CTA. */
 int snk_launch_info(const snk_handle* h, int32_t* out /*[6]*/);
 /* Which form of the lane path the NEXT step will launch (it follows the body-length regime, DESIGN.md 4.8):
- * out[0] = 0 fused kernel, 1 warp-specialised kernel, 3 two kernels (k_lane_logic + k_lane_paint2), -1 not a lane-family
+ * out[0] = 0 fused kernel, 1 warp-specialised kernel, 3 two kernels (k_lane_logic + k_lane_paint2, or + k_lane_grid in
+ * SNK_OBS_GRID, which always uses this form), -1 not a lane-family
  * configuration (2 is no longer reported); out[1] = envs stepped per warp batch of the fused kernel;
  * out[2] = envs per shared-memory image; out[3] = 1 when the handle switches forms by itself. */
 int snk_launch_form(const snk_handle* h, int32_t* out /*[4]*/);

@@ -4,13 +4,13 @@ Host-side mirror of the reference's Gym / VecEnv interface over libsnk.so (inclu
 Importing this package loads the CUDA library and fails if it has not been built.
 """
 from . import _lib
-from ._lib import SnkError  # noqa: F401
+from ._lib import CELL_EMPTY, CELL_FRUIT, CELL_WALL, SnkError, cell_body, cell_head  # noqa: F401
 
 _lib.lib()  # no CPU fallback: a missing extension is an import error
 
-from .vec_env import EnvStates, Infos, MonitorCSV, SnakeVecEnv, StepGraph, split_state  # noqa: E402,F401
+from .vec_env import EnvStates, Infos, MonitorCSV, SnakeVecEnv, StepGraph, expand_views, split_state  # noqa: E402,F401
 from .sharding import all_reduce_stats, make_sharded_env, shard_range  # noqa: E402,F401
 from .rollout import gae  # noqa: E402,F401
 from .registration import ENV_IDS, SnakeGymEnv, make, make_basic_env, register  # noqa: E402,F401
 
-__version__ = "0.3.0"
+__version__ = "0.3.1"

@@ -10,7 +10,18 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("SNK_LIB") or os.path.join(_HERE, "libsnk.so")  # SNK_LIB: A/B builds during kernel work
 
 RULES = {"classic": 0, "adversarial": 1, "cut": 2}
-OBS_NATIVE, OBS_ATARI84 = 0, 1
+OBS_NATIVE, OBS_ATARI84, OBS_GRID = 0, 1, 2
+OBS_MODES = {"native": OBS_NATIVE, "atari84": OBS_ATARI84, "grid": OBS_GRID}
+# cell codes of obs_mode 'grid' (SNK_CELL_* of include/snk.h); snake s: body 3 + 2s, head 4 + 2s
+CELL_EMPTY, CELL_FRUIT, CELL_WALL = 0, 1, 255
+
+
+def cell_body(s):
+    return 3 + 2 * s
+
+
+def cell_head(s):
+    return 4 + 2 * s
 RNG_PHILOX, RNG_TAPE = 0, 1
 NSTATS = 8
 STAT_NAMES = ("env_steps", "episodes", "return_sum", "length_sum", "fruits", "deaths", "body_cells", "draws")
@@ -89,6 +100,7 @@ _SIGNATURES = {
     "snk_gen_scripted_actions": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_uint64, C.c_int32, C.c_void_p]),
     "snk_gae": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_double, C.c_int32, C.c_int64,
                           C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    "snk_expand_views": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
     "snk_algorithmic_bytes_per_step": (C.c_int, [C.POINTER(SnkConfig), C.c_double, C.POINTER(C.c_double)]),
     "snk_launch_count": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     "snk_launch_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),

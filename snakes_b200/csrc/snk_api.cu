@@ -159,6 +159,21 @@ static int dbg_check(const std::string& opts) {
   return SNK_OK;
 }
 
+// SNK_OBS_GRID has one writer per family (k_lane_grid behind k_lane_logic; k_step_rows<RULES, true>), so the switches
+// that choose between RGB writers or tune them would silently measure something else there.  force_kernel=lane|rows and
+// restore_thr keep their meaning.
+static int dbg_check_grid(const std::string& opts) {
+  static const char* const keys[] = {"lane", "delta", "epw", "adaptive", "alt_hi"};
+  for (const std::string& t : dbg_tokens(opts)) {
+    const size_t eq = t.find('=');
+    const std::string key = t.substr(0, eq), val = eq == std::string::npos ? "" : t.substr(eq + 1);
+    const bool bad = std::any_of(std::begin(keys), std::end(keys), [&](const char* k) { return key == k; }) ||
+                     (key == "force_kernel" && (val == "tile" || val == "dense"));
+    if (bad) return fail(SNK_EINVAL, "debug option '%s' does not apply to obs_mode grid", t.c_str());
+  }
+  return SNK_OK;
+}
+
 // Un-paint by zero-fill + border redraw (lane_restore / cta_restore) once a lane would walk more than restore_thr segments.
 // `threads` share an image buffer (32: a warp of the fused / ws kernel; 64: k_lane_paint2).  The restore costs each of
 // them one 16-byte store per 16 * threads bytes of image plus its share of one env's border units; a walked segment costs
@@ -181,7 +196,8 @@ static int cfg_check(const snk_config* c) {
   if (c->rules < 0 || c->rules > 2) return fail(SNK_EINVAL, "unknown rules %d", c->rules);
   if (c->num_envs < 1) return fail(SNK_EINVAL, "num_envs must be >= 1");
   if (c->max_steps < 0 || c->max_steps > 65535) return fail(SNK_EINVAL, "max_steps must be 0..65535");
-  if (c->obs_mode != SNK_OBS_NATIVE && c->obs_mode != SNK_OBS_ATARI84) return fail(SNK_EINVAL, "unknown obs_mode %d", c->obs_mode);
+  if (c->obs_mode != SNK_OBS_NATIVE && c->obs_mode != SNK_OBS_ATARI84 && c->obs_mode != SNK_OBS_GRID)
+    return fail(SNK_EINVAL, "unknown obs_mode %d", c->obs_mode);
   if (c->obs_mode == SNK_OBS_ATARI84 && 84 % (c->size + 2) != 0)
     return fail(SNK_EINVAL, "obs_mode atari84 needs 84 %% (size + 2) == 0 (exact pixel replication); size=%d", c->size);
   if (c->obs_mode == SNK_OBS_ATARI84 && (c->n_views ? c->n_views : c->n_snakes) > 8)
@@ -330,6 +346,8 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   int rc = cfg_check(cfg);
   if (rc) return rc;
   if ((rc = dbg_check(debug_opts ? debug_opts : ""))) return rc;
+  const bool grid = cfg->obs_mode == SNK_OBS_GRID;
+  if (grid && (rc = dbg_check_grid(debug_opts ? debug_opts : ""))) return rc;
   if (!out) return fail(SNK_EINVAL, "out is NULL");
   int n_dev = 0;
   CUDA_TRY(cudaGetDeviceCount(&n_dev));
@@ -361,7 +379,7 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   memset(&p, 0, sizeof(p));
   const int D = cfg->size, V = D + 2, S = cfg->n_snakes, F = cfg->n_fruits, K = h->cfg.n_views;
   const long long N = cfg->num_envs;
-  p.D = D; p.V = V; p.VV = V * V; p.S = S; p.F = F; p.K = K; p.C = 3 * K;
+  p.D = D; p.V = V; p.VV = V * V; p.S = S; p.F = F; p.K = K; p.C = grid ? 1 : 3 * K;  // grid: one code byte per cell
   p.cap = h->lay.cap;
   p.RW = (REC_SNAKE0 + 2 * S + (F + 1) / 2 + 3) & ~3;
   p.E = p.VV * p.C;
@@ -379,7 +397,7 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   std::string force;
   dbg_get(dbg, "force_kernel", &force);
   int TE = 0;
-  if (snk_lane_supported(S, K) && F <= 4 && D <= 32) {
+  if ((grid || snk_lane_supported(S, K)) && S <= 4 && F <= 4 && D <= 32) {  // grid: k_lane_grid exists for every K
     const int cand[3] = {32, 16, 8};
     for (int i = 0; i < 3 && !TE; ++i)
       if (cand[i] % p.G == 0 && (size_t)cand[i] * p.E <= 28 * 1024) TE = cand[i];
@@ -389,7 +407,7 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   const size_t smem_tile = (size_t)(W + p.G) * p.E + (size_t)W * (REC_SNAKE0 + 2 * S + (F + 1) / 2 + 3 + p.bm_words) * 4;
   // rows kernel: chunks of R image rows must be 16-byte multiples (TMA) and fit a ~24 KB buffer
   int R = 0;
-  if (p.E % 16 == 0) {
+  if (p.E % 16 == 0 && !grid) {
     const int unit = 16 / gcd(V * p.C, 16);
     // chunk size and CTA shape measured on B200 at 16 snakes on 64x64: 4 warps (1 producer + 3 consumers) give 7 CTAs
     // per SM, and 8 KB chunks beat 12 KB (32 768 envs: classic 1280 us, cut 1502 vs 1551 us)
@@ -397,9 +415,12 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
     for (int r = unit; r <= V && ((size_t)r * V * p.C <= lim || !R); r += unit) { if ((size_t)r * V * p.C > 48 * 1024) break; R = r; }
   }
   plan.kind = TE ? KIND_LANE : smem_tile <= 110 * 1024 ? KIND_TILE : R ? KIND_ROWS : KIND_DENSE;
+  // grid: every ring-family geometry goes to the rows kernel's grid form (the producer's code grid IS the observation)
+  plan.obs_grid = grid;
+  if (grid && plan.kind != KIND_LANE) plan.kind = KIND_ROWS;
   if (force == "dense") plan.kind = KIND_DENSE;
   if (force == "rows") {
-    if (!R) { snk_destroy(h); return fail(SNK_EINVAL, "rows kernel does not support this configuration"); }
+    if (!R && !grid) { snk_destroy(h); return fail(SNK_EINVAL, "rows kernel does not support this configuration"); }
     plan.kind = KIND_ROWS;
   }
   if (force == "tile" && smem_tile <= 200 * 1024) plan.kind = KIND_TILE;
@@ -421,8 +442,8 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
     // fastest small-image form (65 536 envs, 10x10: 3 snakes cut 53.0 vs 61.3 us, 3 snakes classic 44.0 vs 48.8,
     // 2 snakes 34.6 vs 38.8; 1 M envs cut 648 vs 751 us); a single snake stays warp-specialised (23.6 vs 29.2 us).
     const bool small_image = p.E < 2048 && (N + 31) / 32 >= 2LL * h->n_sm;
-    plan.ws = plan.kind == KIND_LANE && (have_lv ? lv == "ws" : (small_image && S == 1));
-    plan.split = plan.kind == KIND_LANE && (have_lv ? lv == "split" : (small_image && S > 1));
+    plan.ws = plan.kind == KIND_LANE && !grid && (have_lv ? lv == "ws" : (small_image && S == 1));
+    plan.split = plan.kind == KIND_LANE && (grid || (have_lv ? lv == "split" : (small_image && S > 1)));
   }
   p.CW = (p.cap - 1 + 15) / 16;
   // lane path geometry: te envs per warp image, epw envs stepped per warp batch (a multiple of te)
@@ -438,12 +459,13 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
     p.W = 32;
     plan.block = plan.ws ? 32 * (WS_PAINT_WARPS + WS_LOGIC_WARPS) : 64;
     lane_geometry(TE, 32);
+    if (grid) p.restore_thr = dbg_int(dbg, "restore_thr", restore_threshold(p, 64));  // k_lane_grid: 64 threads per buffer
   } else if (plan.kind == KIND_TILE) {
     p.W = W; plan.block = 32 * W; plan.smem = smem_tile;
     p.n_groups = (N + W - 1) / W;
   } else if (plan.kind == KIND_ROWS) {
     p.W = 1; p.R = R; plan.block = 128;  // 1 producer warp + 3 consumer warps
-    p.tile_stride = (int)(((size_t)R * V * p.C + 127) & ~(size_t)127);
+    p.tile_stride = (int)(((size_t)R * V * p.C + 127) & ~(size_t)127);  // grid: R = 0, no chunk buffers
     plan.smem = 2 * (((size_t)p.VV + 127) & ~(size_t)127) + 2 * (size_t)p.tile_stride + (size_t)(p.RW + p.bm_words) * 4;
     p.n_groups = N;
   } else {
@@ -538,7 +560,7 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
     // step); the headline shard gains 64.5 -> 52.7 us.  delta=0 / delta=1 turn it off / on regardless.
     TRY(dev_alloc(h, &p.frame_ok, (size_t)N, true));
     const int dm = dbg_int(dbg, "delta", -1);
-    p.delta = cfg->rules == SNK_RULES_CLASSIC && (V + 1) * p.C >= 32 && ((uintptr_t)h->d_obs_own & 31) == 0 &&
+    p.delta = !grid && cfg->rules == SNK_RULES_CLASSIC && (V + 1) * p.C >= 32 && ((uintptr_t)h->d_obs_own & 31) == 0 &&
               (dm < 0 ? p.EPW == 32 : dm != 0);
   }
   h->d_obs84_own = nullptr;
@@ -667,7 +689,8 @@ static int launch(snk_handle* h, int mode, const int8_t* d_actions, const uint8_
     }
   }
   p.mode = mode; p.actions = d_actions; p.mask = d_mask;
-  p.frame_own = p.obs == h->d_obs_own;  // the step kernels write every env's image into p.obs
+  // the step kernels write every env's image into p.obs (frame_ok is about RGB images: a grid handle never has one)
+  p.frame_own = p.obs == h->d_obs_own && h->cfg.obs_mode != SNK_OBS_GRID;
   p.delta = p.delta && p.frame_own && mode == MODE_STEP;
   p.tape_vals = h->d_tape_vals; p.tape_bounds = h->d_tape_bounds; p.tape_off = h->d_tape_off;
   if (p.rng_mode == SNK_RNG_TAPE && !p.tape_vals) return fail(SNK_EINVAL, "rng_mode is TAPE but no tape was set");
@@ -778,7 +801,7 @@ static int graph_create_impl(snk_handle* h, const int8_t* d_actions, int32_t n_b
       // (occupancy from the previous captured step's observations; step 0 walks the bodies: the graph cannot know where
       // the observations of the state it will be launched on are)
       if (snk_launch_scripted_actions(h->p, h->d_actions_own, scripted->step0 + (uint64_t)t, scripted->seed, scripted->eps_permille,
-                                      t ? g->last_native_obs : nullptr, s) != cudaSuccess)
+                                      t && h->cfg.obs_mode != SNK_OBS_GRID ? g->last_native_obs : nullptr, s) != cudaSuccess)
         rc = fail(SNK_ECUDA, "capture: scripted policy kernel");
       h->launches++;
     }
@@ -872,6 +895,8 @@ static int step_host_impl(snk_handle* h, const int8_t* h_actions, uint8_t* h_obs
   if (!h || !h_actions) return fail(SNK_EINVAL, "NULL argument");
   cudaStream_t s = (cudaStream_t)stream;
   const Params& p = h->p;
+  if (h->cfg.obs_mode == SNK_OBS_GRID && n_views_out != 0)
+    return fail(SNK_EINVAL, "obs_mode grid copies the grid: n_views_out must be 0 (snk_expand_views gives views)");
   if (n_views_out <= 0 || n_views_out > p.K) n_views_out = p.K;
   if (n_views_out < p.K && n_views_out > 4) return fail(SNK_EINVAL, "a view subset holds at most 4 views");
   CUDA_TRY(cudaSetDevice(h->cfg.device));
@@ -1070,6 +1095,7 @@ extern "C" int snk_set_obs_target(snk_handle* h, uint8_t* d_obs, size_t bytes) {
 extern "C" int snk_set_main_view_target(snk_handle* h, uint8_t* d_main, size_t bytes) {
   if (!h) return fail(SNK_EINVAL, "handle is NULL");
   if (!d_main) { h->d_main_target = nullptr; return SNK_OK; }
+  if (h->cfg.obs_mode == SNK_OBS_GRID) return fail(SNK_EINVAL, "obs_mode grid has no main-view target: expand view 0 with snk_expand_views");
   const size_t need = (size_t)h->p.N * (h->obs_out_env_bytes / (size_t)h->p.C) * 3;
   if (bytes < need) return fail(SNK_EINVAL, "main-view target too small: %zu < %zu", bytes, need);
   h->d_main_target = d_main;
@@ -1410,7 +1436,9 @@ extern "C" int snk_gen_scripted_actions(snk_handle* h, int8_t* d_actions, uint64
   if (h->p.family != 1 || h->cfg.rules != SNK_RULES_CLASSIC)
     return fail(SNK_EINVAL, "the scripted policy needs a lane-family configuration with classic rules");
   CUDA_TRY(cudaSetDevice(h->cfg.device));
-  CUDA_TRY(snk_launch_scripted_actions(h->p, d_actions, step, seed, eps_permille, h->obs_current, (cudaStream_t)stream));
+  // the policy reads occupancy from the green bytes of a native image; a grid handle's kernel walks the bodies instead
+  const uint8_t* occ = h->cfg.obs_mode == SNK_OBS_GRID ? nullptr : h->obs_current;
+  CUDA_TRY(snk_launch_scripted_actions(h->p, d_actions, step, seed, eps_permille, occ, (cudaStream_t)stream));
   h->launches++;
   return SNK_OK;
 }
@@ -1426,13 +1454,26 @@ extern "C" int snk_gae(const float* d_rewards, const float* d_values, const uint
   return SNK_OK;
 }
 
+extern "C" int snk_expand_views(const uint8_t* d_grid, int64_t n, int32_t size, int32_t first_view, int32_t n_views,
+                                uint8_t* d_out, int32_t device, void* stream) {
+  if (!d_grid || !d_out) return fail(SNK_EINVAL, "NULL argument");
+  if (n < 1) return fail(SNK_EINVAL, "n must be >= 1, got %lld", (long long)n);
+  if (size < 2 || size > 254) return fail(SNK_EINVAL, "size must be 2..254, got %d", size);
+  if (n_views < 1 || first_view < 0 || first_view + n_views > 32)
+    return fail(SNK_EINVAL, "views [%d, %d) outside [0, 32) or empty", first_view, first_view + n_views);
+  CUDA_TRY(cudaSetDevice(device));
+  const long long VV = (long long)(size + 2) * (size + 2);
+  CUDA_TRY(snk_launch_expand_views(d_grid, n * VV, first_view, n_views, d_out, (cudaStream_t)stream));
+  return SNK_OK;
+}
+
 extern "C" int snk_algorithmic_bytes_per_step(const snk_config* c, double mean_sum_len, double* out) {
   int rc = cfg_check(c);
   if (rc) return rc;
   if (!out) return fail(SNK_EINVAL, "out is NULL");
   const double V = c->size + 2.0, S = c->n_snakes, F = c->n_fruits, K = c->n_views ? c->n_views : c->n_snakes;
-  const double side = c->obs_mode == SNK_OBS_ATARI84 ? 84.0 : V;
-  *out = K * side * side * 3.0 + 19.0 * S + 2.0 * mean_sum_len + 2.0 * F + 30.0;  // SURVEY.md section 8d
+  const double side = c->obs_mode == SNK_OBS_ATARI84 ? 84.0 : V, obs = c->obs_mode == SNK_OBS_GRID ? V * V : K * side * side * 3.0;
+  *out = obs + 19.0 * S + 2.0 * mean_sum_len + 2.0 * F + 30.0;  // SURVEY.md section 8d
   return SNK_OK;
 }
 

@@ -325,9 +325,9 @@ __global__ void __launch_bounds__(128, (S <= 2 ? 7 : 1)) k_lane_logic(const Para
 // (an image takes as long as its longest snake) and the zero-fill of the restore, and doubles the warps that cover each
 // other's latencies.  CTA-wide barriers order the phases.  Launched programmatically behind k_lane_logic: the border
 // image is fetched before griddepcontrol.wait.
-template <int K>
+template <int C>
 __device__ __forceinline__ void cta_restore(u8* tile, int n16, u8* img, int V, int sub, int LPE, int tid, int NT) {
-  constexpr int C = 3 * K, U = (C & 1) ? 1 : 2, PU = 2 * C / U;
+  constexpr int U = (C & 1) ? 1 : 2, PU = 2 * C / U;
   uint4* t4 = reinterpret_cast<uint4*>(tile);
   const uint4 z = make_uint4(0u, 0u, 0u, 0u);
   for (int i = tid; i < n16; i += NT) t4[i] = z;
@@ -380,19 +380,23 @@ __device__ __forceinline__ PaintRuns<S> cta_paint_prepare(const Params& p, const
   return r;
 }
 
-// fruits, then the snakes in index order (get_ob_for_snake :35-58); `paint` false = the same walk writes zeros
-template <int S, int RULES, int K>
+// fruits, then the snakes in index order (get_ob_for_snake :35-58); `paint` false = the same walk writes zeros.
+// GRID: the image is the cell-code grid of SNK_OBS_GRID (one byte per cell, K does not enter), the same walk writes codes.
+template <int S, int RULES, int K, bool GRID = false>
 __device__ __forceinline__ void cta_paint(const Params& p, const PaintEnv<S>& pe, const PaintRuns<S>& runs, long long e_owner, int sub, int LPE,
                                           u8* img, bool paint) {
-  constexpr int C = 3 * K;
+  constexpr int C = GRID ? 1 : 3 * K;
   const int V = p.V, F = p.F;
-  const u8 red = paint ? 255 : 0;
+  const u8 red = paint ? (GRID ? SNK_CELL_FRUIT : 255) : 0;
   if (RULES == SNK_RULES_CLASSIC) {
 #pragma unroll
     for (int f = 0; f < 4; ++f) {
       if (pe.valid && f < F && (f & (LPE - 1)) == sub) {
+        if (GRID) img[pe.fruit[f]] = red;
+        else {
 #pragma unroll
-        for (int k = 0; k < K; ++k) img[pe.fruit[f] * C + 3 * k] = red;
+          for (int k = 0; k < K; ++k) img[pe.fruit[f] * C + 3 * k] = red;
+        }
       }
     }
   } else if (pe.valid) {
@@ -403,8 +407,11 @@ __device__ __forceinline__ void cta_paint(const Params& p, const PaintEnv<S>& pe
         // cells outside the board lie under the border (the reference paints them, then the wall over them, :52-56)
         const u32 px = ((u32)pid * p.magicV) >> 16, py = (u32)pid - px * (u32)V;
         if (px - 1u < (u32)(V - 2) && py - 1u < (u32)(V - 2)) {
+          if (GRID) img[pid] = red;
+          else {
 #pragma unroll
-          for (int k = 0; k < K; ++k) img[pid * C + 3 * k] = red;
+            for (int k = 0; k < K; ++k) img[pid * C + 3 * k] = red;
+          }
         }
       }
     }
@@ -418,7 +425,8 @@ __device__ __forceinline__ void cta_paint(const Params& p, const PaintEnv<S>& pe
       const int i1 = runs.i1[s];
       u32 w = runs.w[s];
       for (;;) {
-        put_pixel<S, K>(img + pos * C, s, i == 0, paint);
+        if (GRID) img[pos] = paint ? (u8)(i == 0 ? SNK_CELL_HEAD(s) : SNK_CELL_BODY(s)) : 0;
+        else put_pixel<S, K>(img + pos * C, s, i == 0, paint);
         if (i + 1 >= i1) break;
         pos -= chain_delta((w >> (2 * (i & 15))) & 3, V);
         ++i;
@@ -431,10 +439,9 @@ __device__ __forceinline__ void cta_paint(const Params& p, const PaintEnv<S>& pe
 
 // Un-paint.  Short bodies: the same walk writes zeros.  Long bodies (`restore`): the threads zero-fill the buffer and
 // redraw the border (cta_restore).  A CTA's last image is not un-painted at all.
-template <int S, int RULES, int K>
-__global__ void __launch_bounds__(64) k_lane_paint2(const Params p) {
-  extern __shared__ __align__(128) u8 smem[];
-  __shared__ __align__(8) u64 s_bar;
+// GRID: the same writer for SNK_OBS_GRID (k_lane_grid), images of TE cell-code grids of V*V bytes.
+template <int S, int RULES, int K, bool GRID>
+__device__ __forceinline__ void lane_paint2_body(const Params& p, u8* smem, u64& s_bar) {
   const int tid = threadIdx.x, NT = 64;
   const int TE = p.TE, LPE = NT / TE, E = p.E;
   const int tile_bytes = TE * E;
@@ -464,14 +471,14 @@ __global__ void __launch_bounds__(64) k_lane_paint2(const Params p) {
     const PaintRuns<S> runs = cta_paint_prepare<S>(p, cur, e0 + slot, sub, LPE);
     const bool restore = __syncthreads_or(p.restore_thr > 0 && trips > p.restore_thr);
     if (!have_image) { mbar_wait(&s_bar, 0); have_image = true; }
-    cta_paint<S, RULES, K>(p, cur, runs, e0 + slot, sub, LPE, img, true);
+    cta_paint<S, RULES, K, GRID>(p, cur, runs, e0 + slot, sub, LPE, img, true);
     fence_async_smem();
     __syncthreads();
     store_image(p, tile, tile_bytes, e0, tid, NT);
     if (next < n_items) {  // the last image of a CTA leaves its buffer as it is
       __syncthreads();
-      if (restore) cta_restore<K>(tile, tile_bytes >> 4, img, p.V, sub, LPE, tid, NT);
-      else cta_paint<S, RULES, K>(p, cur, runs, e0 + slot, sub, LPE, img, false);
+      if (restore) cta_restore<GRID ? 1 : 3 * K>(tile, tile_bytes >> 4, img, p.V, sub, LPE, tid, NT);
+      else cta_paint<S, RULES, K, GRID>(p, cur, runs, e0 + slot, sub, LPE, img, false);
       __syncthreads();
     }
     cur = nxt;
@@ -484,6 +491,22 @@ __global__ void __launch_bounds__(64) k_lane_paint2(const Params p) {
   // (fruit-seeking stream 114.5 vs 109.1 us), and nothing without one (88.7 vs 89.2 us)
   __syncthreads();
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+}
+
+template <int S, int RULES, int K>
+__global__ void __launch_bounds__(64) k_lane_paint2(const Params p) {
+  extern __shared__ __align__(128) u8 smem[];
+  __shared__ __align__(8) u64 s_bar;
+  lane_paint2_body<S, RULES, K, false>(p, smem, s_bar);
+}
+
+// k_lane_grid: the observation writer of SNK_OBS_GRID behind k_lane_logic.  A grid image is 1/(3K) of the RGB one, so a
+// CTA's buffer holds TE = 32 envs' grids (16 when they exceed 28 KB); K does not enter, the kernel exists per (S, rules).
+template <int S, int RULES>
+__global__ void __launch_bounds__(64) k_lane_grid(const Params p) {
+  extern __shared__ __align__(128) u8 smem[];
+  __shared__ __align__(8) u64 s_bar;
+  lane_paint2_body<S, RULES, 1, true>(p, smem, s_bar);
 }
 
 
@@ -820,7 +843,9 @@ __device__ __forceinline__ void rows_expand(const u8* __restrict__ code, u8* __r
   for (int i = ct; i < cells; i += cn) rows_emit<CT>(tile, i, code[i], C, K);
 }
 
-template <int RULES>
+// GRID (SNK_OBS_GRID): the consumers store the finished code grid itself, V*V bytes at obs + e*V*V (not 16-byte aligned
+// in general: plain coalesced stores), and there are no chunk buffers.
+template <int RULES, bool GRID>
 __global__ void __launch_bounds__(160, 5) k_step_rows(const Params p) {
   extern __shared__ __align__(128) u8 smem[];
   __shared__ double s_stats[SNK_NSTATS];
@@ -836,7 +861,7 @@ __global__ void __launch_bounds__(160, 5) k_step_rows(const Params p) {
   __syncthreads();
   WarpStats st = {0, 0, 0, 0, 0, 0, 0, 0};
   u32 errs = 0;
-  const int n_chunks = (V + R - 1) / R;
+  const int n_chunks = GRID ? 0 : (V + R - 1) / R;
   int issued = 0;  // chunks handed to the TMA engine so far (bulk groups of the consumers' thread 0)
 #ifdef SNK_PHASE_TIMING  // experiment build (tools/phase_rows.py)
   long long tA = 0, tB = 0, tC = 0, tD = 0; const long long tStart = clock64();
@@ -930,7 +955,11 @@ __global__ void __launch_bounds__(160, 5) k_step_rows(const Params p) {
     }
     if (it == 0) __syncthreads();  // grid 0 ready
     if (e >= p.N) break;
-    if (warp > 0) {
+    if (GRID && warp > 0) {
+      const u8* code = codes + (it & 1) * code_stride;
+      u8* out = p.obs + e * (long long)VV;
+      for (int i = tid - 32; i < VV; i += blockDim.x - 32) out[i] = code[i];
+    } else if (warp > 0) {
       const int ct = tid - 32, cn = blockDim.x - 32;
       const u8* code = codes + (it & 1) * code_stride;
       u8* out = p.obs + e * (long long)p.E;
@@ -968,7 +997,7 @@ __global__ void __launch_bounds__(160, 5) k_step_rows(const Params p) {
     }
     __syncthreads();  // grid (it + 1) & 1 built, grid it & 1 consumed
   }
-  if (tid == 32) bulk_wait_all();
+  if (!GRID && tid == 32) bulk_wait_all();
 #ifdef SNK_PHASE_TIMING  // total, producer logic, producer grid build, consumers, of which TMA read-wait
   if (tid == 0) { atomicAdd(&p.stats[3], (double)(clock64() - tStart)); atomicAdd(&p.stats[4], (double)tA); atomicAdd(&p.stats[5], (double)tB); }
   if (tid == 32) { atomicAdd(&p.stats[6], (double)tC); atomicAdd(&p.stats[7], (double)tD); }
@@ -1524,6 +1553,72 @@ __global__ void k_extract_views(const u8* __restrict__ src, u8* __restrict__ dst
   }
 }
 
+// ------------------------------------------------------------------ SNK_OBS_GRID -> RGB views (snk_expand_views)
+// A pure write stream: one code byte in, 3 n_views bytes out per cell.  The colours of one cell: `other` for every view
+// but the one of its own snake, `own` for that view, whose index relative to first_view is `rel` (-1 / out of range:
+// none).  Packed R | G << 8 | B << 16 like snake_rgb.
+__device__ __forceinline__ void cell_colours(u32 c, int first_view, u32& other, u32& own, int& rel) {
+  other = c == SNK_CELL_FRUIT ? 255u : c == SNK_CELL_WALL ? 0xffffffu : 0u;
+  own = other;
+  rel = -1;
+  if (c >= 3 && c != SNK_CELL_WALL) {
+    other = snake_rgb(false, (c - 3) & 1);
+    own = snake_rgb(true, (c - 3) & 1);
+    rel = (int)((c - 3) >> 1) - first_view;
+  }
+}
+
+// k_expand_views<NV>: NV views, compile time.  A thread takes P cells, the fewest whose P * 3 NV output bytes are whole
+// 16-byte words (NV = 1: 16 cells, 2: 8, 3: 16, 16: 1), so the byte positions of the period fold to constants.  The warp
+// stages its 32 periods in shared memory and stores them as consecutive 16-byte words: one 512-byte run per store
+// instruction instead of 32 pieces 3 NV * P bytes apart.  B200, 131 072 envs of 21x21: 2 views 95.7 -> 90.3 us, 3 views
+// 184.5 -> 102.4, 16 views 717 -> 543; one view 57.2 -> 64.3 (DESIGN.md section 4.15).
+template <int NV>
+__global__ void __launch_bounds__(256) k_expand_views(const u8* __restrict__ grid, uint4* __restrict__ out, long long n_periods, int first_view) {
+  constexpr int C = 3 * NV, P = 16 / (C % 16 == 0 ? 16 : C % 8 == 0 ? 8 : C % 4 == 0 ? 4 : C % 2 == 0 ? 2 : 1), W = P * C / 4, Q = W / 4;
+  __shared__ uint4 s_out[8][32 * Q];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const long long g = blockIdx.x * (long long)blockDim.x + threadIdx.x, g0 = g - lane;
+  if (g0 >= n_periods) return;  // warp-uniform
+  if (g < n_periods) {
+    u32 other[P], own[P];
+    int rel[P];
+#pragma unroll
+    for (int q = 0; q < P; ++q) cell_colours(__ldg(grid + g * P + q), first_view, other[q], own[q], rel[q]);
+    u32 w[W];
+#pragma unroll
+    for (int i = 0; i < W; ++i) {
+      u32 v = 0;
+#pragma unroll
+      for (int b = 0; b < 4; ++b) {
+        const int j = 4 * i + b, q = j / C, view = (j % C) / 3, ch = j % 3;
+        v |= (((rel[q] == view ? own[q] : other[q]) >> (8 * ch)) & 0xffu) << (8 * b);
+      }
+      w[i] = v;
+    }
+#pragma unroll
+    for (int i = 0; i < Q; ++i) s_out[warp][lane * Q + i] = make_uint4(w[4 * i], w[4 * i + 1], w[4 * i + 2], w[4 * i + 3]);
+  }
+  __syncwarp();
+  const int n16 = (int)min(32LL, n_periods - g0) * Q;
+  for (int i = lane; i < n16; i += 32) __stcs(out + g0 * Q + i, s_out[warp][i]);
+}
+
+// any view count, ragged tails, unaligned destinations: one thread per cell, byte stores
+__global__ void k_expand_views_any(const u8* __restrict__ grid, u8* __restrict__ out, long long first_cell, long long n_cells,
+                                   int first_view, int n_views) {
+  const long long i = first_cell + blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  if (i >= n_cells) return;
+  u32 other, own;
+  int rel;
+  cell_colours(__ldg(grid + i), first_view, other, own, rel);
+  u8* px = out + i * 3 * n_views;
+  for (int k = 0; k < n_views; ++k) {
+    const u32 v = k == rel ? own : other;
+    px[3 * k] = (u8)v; px[3 * k + 1] = (u8)(v >> 8); px[3 * k + 2] = (u8)(v >> 16);
+  }
+}
+
 // snk_get_stats_global in the peer-memory form: push the rank's CURRENT sums to the peers (the final step's, which no
 // later step would push) and add up the own sums and what the peers have pushed so far
 __global__ void k_sum_inbox(const PeerArgs a, const double* __restrict__ stats, double* __restrict__ glob) {
@@ -1566,8 +1661,32 @@ bool snk_lane_supported(int S, int K) {
 }
 #endif
 
+// SNK_OBS_GRID, lane family: k_lane_logic + k_lane_grid, instantiated per snake count (the views do not enter)
+#define GRID_SNAKES(X) X(1) X(2) X(3) X(4)
+
 template <int RULES>
 cudaError_t launch_rules(const Params& p, const LaunchPlan& plan, cudaStream_t stream) {
+  if (plan.kind == KIND_LANE && plan.obs_grid) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(plan.grid); cfg.blockDim = dim3(plan.block); cfg.dynamicSmemBytes = plan.smem; cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr; cfg.numAttrs = 1;
+    cudaLaunchConfig_t lc = cfg;
+    lc.gridDim = dim3((unsigned)((p.N + 127) / 128)); lc.blockDim = dim3(128); lc.dynamicSmemBytes = 0;
+#define X(s)                                                                            \
+  if (p.S == s) {                                                                       \
+    if (p.mode != MODE_OBSERVE) {                                                       \
+      cudaError_t e1 = cudaLaunchKernelEx(&lc, k_lane_logic<s, RULES>, p);              \
+      if (e1 != cudaSuccess) return e1;                                                 \
+    }                                                                                   \
+    return cudaLaunchKernelEx(&cfg, k_lane_grid<s, RULES>, p);                          \
+  }
+    GRID_SNAKES(X)
+#undef X
+    return cudaErrorInvalidConfiguration;
+  }
   if (plan.kind == KIND_LANE) {
 #define X(s, k)                                                                                              \
   if (p.S == s && p.K == k) {                                                                                \
@@ -1597,7 +1716,8 @@ cudaError_t launch_rules(const Params& p, const LaunchPlan& plan, cudaStream_t s
     return cudaErrorInvalidConfiguration;
   }
   if (plan.kind == KIND_ROWS) {
-    k_step_rows<RULES><<<plan.grid, plan.block, plan.smem, stream>>>(p);
+    if (plan.obs_grid) k_step_rows<RULES, true><<<plan.grid, plan.block, plan.smem, stream>>>(p);
+    else k_step_rows<RULES, false><<<plan.grid, plan.block, plan.smem, stream>>>(p);
     return cudaGetLastError();
   }
   if (plan.kind == KIND_TILE) {
@@ -1646,14 +1766,26 @@ template <int RULES>
 cudaError_t plan_rules(LaunchPlan& plan, int n_sm, int S, int K) {
   cudaError_t err = cudaErrorInvalidConfiguration;
   int occ = 0;
-  if (plan.kind == KIND_LANE) {
+  if (plan.kind == KIND_LANE && plan.obs_grid) {
+#define X(s)                                                                                                                  \
+  if (S == s) {                                                                                                               \
+    if ((err = cudaFuncSetAttribute(k_lane_grid<s, RULES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err; \
+    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_lane_grid<s, RULES>, plan.block, plan.smem);                  \
+  }
+    GRID_SNAKES(X)
+#undef X
+    if (err) return err;
+  } else if (plan.kind == KIND_LANE) {
 #define X(s, k) if (S == s && K == k) err = plan_lane<s, RULES, k>(plan, occ);
     LANE_COMBOS(X)
 #undef X
     if (err) return err;
+  } else if (plan.kind == KIND_ROWS && plan.obs_grid) {
+    if ((err = cudaFuncSetAttribute(k_step_rows<RULES, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
+    if ((err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_rows<RULES, true>, plan.block, plan.smem))) return err;
   } else if (plan.kind == KIND_ROWS) {
-    if ((err = cudaFuncSetAttribute(k_step_rows<RULES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
-    if ((err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_rows<RULES>, plan.block, plan.smem))) return err;
+    if ((err = cudaFuncSetAttribute(k_step_rows<RULES, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
+    if ((err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_rows<RULES, false>, plan.block, plan.smem))) return err;
   } else if (plan.kind == KIND_TILE && plan.block <= 256) {
     if ((err = cudaFuncSetAttribute(k_step_tile<RULES, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
     if ((err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_tile<RULES, 256>, plan.block, plan.smem))) return err;
@@ -1738,6 +1870,33 @@ cudaError_t snk_launch_extract_views(const uint8_t* src, uint8_t* dst, long long
   }
   const long long n = (n_pixels - done + 3) / 4;
   k_extract_views<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(src, dst, done, n_pixels, C, n_out);
+  return cudaGetLastError();
+}
+
+template <int NV>
+static long long launch_expand(const u8* grid, long long n_cells, int first_view, u8* out, cudaStream_t stream) {
+  constexpr int C = 3 * NV, P = 16 / (C % 16 == 0 ? 16 : C % 8 == 0 ? 8 : C % 4 == 0 ? 4 : C % 2 == 0 ? 2 : 1);
+  const long long n_periods = n_cells / P;
+  if (n_periods > 0)
+    k_expand_views<NV><<<(unsigned)((n_periods + 255) / 256), 256, 0, stream>>>(grid, reinterpret_cast<uint4*>(out), n_periods, first_view);
+  return n_periods * P;
+}
+
+cudaError_t snk_launch_expand_views(const uint8_t* grid, long long n_cells, int first_view, int n_views, uint8_t* out, cudaStream_t stream) {
+  long long done = 0;
+  if ((reinterpret_cast<uintptr_t>(out) & 15) == 0) {
+    switch (n_views) {
+      case 1: done = launch_expand<1>(grid, n_cells, first_view, out, stream); break;
+      case 2: done = launch_expand<2>(grid, n_cells, first_view, out, stream); break;
+      case 3: done = launch_expand<3>(grid, n_cells, first_view, out, stream); break;
+      case 16: done = launch_expand<16>(grid, n_cells, first_view, out, stream); break;
+      default: break;
+    }
+  }
+  if (done < n_cells) {
+    const long long n = n_cells - done;
+    k_expand_views_any<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(grid, out, done, n_cells, first_view, n_views);
+  }
   return cudaGetLastError();
 }
 

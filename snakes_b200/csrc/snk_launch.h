@@ -15,6 +15,7 @@ struct LaunchPlan {
   int kind;         // KIND_LANE (lane per env, chain bodies), KIND_TILE (warp per env), KIND_ROWS / KIND_DENSE (CTA per env)
   bool ws;          // lane path as ONE warp-specialised kernel (k_step_lane_ws): paint warps + logic warps per CTA
   bool split;       // lane path as two kernels: k_lane_logic (thread per env) + k_lane_paint2 (observation writer)
+  bool obs_grid;    // SNK_OBS_GRID: k_lane_logic + k_lane_grid (lane, always split) or k_step_rows<RULES, true> (rows)
   int grid, block;
   size_t smem;
   int occupancy;    // resident CTAs per SM
@@ -32,6 +33,7 @@ cudaError_t snk_launch_restore(const Params& p, const int64_t* idx, long long co
                                cudaStream_t stream);
 cudaError_t snk_launch_copy(const Params& p, const int64_t* src, const int64_t* dst, long long count, cudaStream_t stream);
 cudaError_t snk_launch_sum_inbox(const PeerArgs& a, const double* stats, double* glob, cudaStream_t stream);
+cudaError_t snk_launch_expand_views(const uint8_t* grid, long long n_cells, int first_view, int n_views, uint8_t* out, cudaStream_t stream);
 cudaError_t snk_launch_extract_views(const uint8_t* src, uint8_t* dst, long long n_pixels, int C, int n_out, cudaStream_t stream);
 cudaError_t snk_launch_scripted_actions(const Params& p, int8_t* actions, uint64_t step, uint64_t seed, int eps_permille,
                                         const uint8_t* occ_obs, cudaStream_t stream);

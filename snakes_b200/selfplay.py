@@ -221,6 +221,8 @@ class Runner(object):
         self.env, self.model, self.opponents = env, model, list(opponent_models)
         self.nsteps, self.gamma, self.lam = nsteps, gamma, lam
         N, dev = env.num_envs, env.device
+        if getattr(env, "obs_mode", "native") == "grid":
+            raise ValueError("Runner keeps RGB views in its rollout: create the env with obs_mode 'native', not 'grid'")
         h, w, c = env.observation_space.shape
         if c < 3 * (1 + len(self.opponents)):
             raise ValueError("the env must emit one view per controlled snake (n_views >= n_snakes)")

@@ -169,9 +169,11 @@ class SnakeVecEnv(object):
     (K; the reference's SnakeEnv emits 3, snake_multiple_test.py:93-95), `seed`, `device`,
     `env_id_base` (global id of env 0: shard offset under multi-GPU), `auto_reset`, `obs_mode`
     ('native' [V,V,3K] or 'atari84' [84,84,3K]: the reference's WarpFrame, utils.py:15-31; exact
-    pixel replication, so it needs 84 % (size + 2) == 0, e.g. size 10 or 19).
+    pixel replication, so it needs 84 % (size + 2) == 0, e.g. size 10 or 19; or 'grid' [V,V]: one
+    cell code per cell (CELL_* constants), lossless for all K views at 1/(3K) of the bytes --
+    `expand_views(obs, K)` is the native observation).
     Host I/O: `host_io=True` (numpy in / numpy out), `host_views` (how many views of each pixel
-    come back, default all K; 1 = the main snake's view only, ppo_multi_agent_new.py:181),
+    come back, default all K; 1 = the main snake's view only, ppo_multi_agent_new.py:181; not with 'grid'),
     `host_copy` (default True: fresh arrays every step like np.stack; False: views of the pinned,
     NUMA-local staging buffers).  `debug`: experiment switches, a "key=value,..." string
     (include/snk.h, snk_create_ex); None reads the SNK_DEBUG environment variable.
@@ -190,11 +192,13 @@ class SnakeVecEnv(object):
             device = device.index or 0
         elif isinstance(device, str):
             device = torch.device(device).index or 0
-        if obs_mode not in ("native", "atari84"):
-            raise ValueError("obs_mode must be 'native' or 'atari84'")
+        if obs_mode not in _lib.OBS_MODES:
+            raise ValueError("obs_mode must be 'native', 'atari84' or 'grid'")
+        if obs_mode == "grid" and host_views is not None:
+            raise ValueError("obs_mode 'grid' returns the whole grid: host_views must be None (expand views on the device)")
         self.obs_mode = obs_mode
         self.cfg = _lib.make_config(num_envs, size, n_snakes, n_fruits, n_views, rules, max_steps, auto_reset,
-                                    obs_mode=_lib.OBS_ATARI84 if obs_mode == "atari84" else _lib.OBS_NATIVE,
+                                    obs_mode=_lib.OBS_MODES[obs_mode],
                                     device=device, env_id_base=env_id_base, seed=seed)
         self.device = torch.device("cuda", self.cfg.device)
         torch.cuda.init()
@@ -215,8 +219,8 @@ class SnakeVecEnv(object):
         self.screen_res = screen_res
         self.host_io = host_io
         self.host_copy = bool(host_copy)
-        self.host_views = self.K if not host_views else int(host_views)
-        if not 1 <= self.host_views <= self.K:
+        self.host_views = None if obs_mode == "grid" else self.K if not host_views else int(host_views)
+        if obs_mode != "grid" and not 1 <= self.host_views <= self.K:
             raise ValueError("host_views must be 1..n_views")
         self._last_infos = None
         self._graphs = {}
@@ -230,7 +234,7 @@ class SnakeVecEnv(object):
         self.host_numa_node = None
         if host_io:
             # pinned staging buffers from the C layer, placed on the GPU's NUMA node (snk_host_alloc)
-            oshape = tuple(self.obs.shape[:3]) + (3 * self.host_views,)
+            oshape = tuple(self.obs.shape) if obs_mode == "grid" else tuple(self.obs.shape[:3]) + (3 * self.host_views,)
             self._h_actions = self._host_array((self.N, self.S), np.int8)
             self._h_obs = self._host_array(oshape, np.uint8)
             self._h_reward = self._host_array((self.N,), np.float32)
@@ -250,7 +254,8 @@ class SnakeVecEnv(object):
         b = _lib.SnkBuffers()
         _lib.check(self._L.snk_get_buffers(self._h, C.byref(b)))
         N, S, dev = self.N, self.S, self.device
-        self.obs = _alias(b.d_obs, (N, b.obs_h, b.obs_w, b.obs_c), "|u1", dev)
+        shape = (N, b.obs_h, b.obs_w) if self.obs_mode == "grid" else (N, b.obs_h, b.obs_w, b.obs_c)
+        self.obs = _alias(b.d_obs, shape, "|u1", dev)
         self.rewards = _alias(b.d_reward, (N,), "<f4", dev)
         self.rewards_all = _alias(b.d_reward_all, (N, S), "<f4", dev)
         self._done_u8 = _alias(b.d_done, (N,), "|u1", dev)
@@ -289,8 +294,8 @@ class SnakeVecEnv(object):
         self.obs, self.rewards, self._done_u8 = self._own
 
     def _host_obs(self):
-        """[N,H,W,3K] (or the first host_views views) of the current device observations as numpy."""
-        if self.host_views == self.K:
+        """[N,H,W,3K] (or the first host_views views; [N,V,V] in grid mode) of the current device observations as numpy."""
+        if self.host_views is None or self.host_views == self.K:
             return self.obs.cpu().numpy()
         return self.obs[..., :3 * self.host_views].contiguous().cpu().numpy()
 
@@ -316,7 +321,7 @@ class SnakeVecEnv(object):
         if self.host_io:
             self._h_actions[...] = np.asarray(actions).reshape(self.N, self.S)
             p = lambda a: C.c_void_p(a.ctypes.data)
-            _lib.check(self._L.snk_step_host_async(self._h, p(self._h_actions), p(self._h_obs), self.host_views, p(self._h_reward),
+            _lib.check(self._L.snk_step_host_async(self._h, p(self._h_actions), p(self._h_obs), self.host_views or 0, p(self._h_reward),
                                                    p(self._h_done), p(self._h_alive), self._stream()))
         else:
             if isinstance(actions, torch.Tensor) and actions.is_cuda and actions.dtype == torch.int8 and actions.is_contiguous():
@@ -416,9 +421,20 @@ class SnakeVecEnv(object):
         """World view of one env as the reference's get_ob_world draws it (snake_multiple_test.py:60-91):
         one [V, V, 3] uint8 image, fruit red, snake i in the i-th colour pair, white border.  It is
         rebuilt on the host from the env's K views (snake k is the green one of view k), so it needs
-        K >= S and the native observation mode; there is no pyglet window on a GPU box."""
+        K >= S and the native observation mode -- or, in grid mode, straight from the cell codes, for any K;
+        there is no pyglet window on a GPU box."""
         if mode != "rgb_array":
             raise NotImplementedError("only mode='rgb_array'")
+        if self.obs_mode == "grid":
+            g = self.obs[env_index].cpu().numpy()
+            world = np.zeros((self.V, self.V, 3), dtype=np.uint8)
+            world[g == _lib.CELL_FRUIT] = (255, 0, 0)
+            for s in range(min(self.S, 4)):   # the reference has 4 colour pairs
+                body_c, head_c = self._WORLD_COLOURS[s]
+                world[g == _lib.cell_body(s)] = body_c
+                world[g == _lib.cell_head(s)] = head_c
+            world[g == _lib.CELL_WALL] = (255, 255, 255)
+            return world
         if self.obs_mode != "native" or self.K < min(self.S, 4):
             return self.obs[env_index, :, :, 0:3].cpu().numpy()
         ob = self.obs[env_index].cpu().numpy().reshape(self.V, self.V, self.K, 3)
@@ -457,7 +473,10 @@ class SnakeVecEnv(object):
 
     def set_main_view_target(self, tensor):
         """Every following step / reset also writes the MAIN snake's view of all envs, packed [N,H,W,3], into `tensor`
-        (slot t of the learner's [nsteps,N,H,W,3] rollout buffer, ppo_multi_agent_new.py:181); None switches it off."""
+        (slot t of the learner's [nsteps,N,H,W,3] rollout buffer, ppo_multi_agent_new.py:181); None switches it off.
+        Not in grid mode: expand_views(obs, 1) gives view 0."""
+        if self.obs_mode == "grid":
+            raise ValueError("obs_mode 'grid' has no main-view target: use expand_views(env.obs, 1)")
         if tensor is None:
             _lib.check(self._L.snk_set_main_view_target(self._h, None, 0))
         else:
@@ -467,7 +486,7 @@ class SnakeVecEnv(object):
 
     def make_graph(self, actions, T=None, obs_out=None, rewards_out=None, dones_out=None, sync_back=False):
         """T steps as one CUDA graph launch (snk_graph_create).  actions: int8 CUDA tensor [B, N, S]; step t plays
-        batch t % B (T defaults to B).  obs_out [T,N,H,W,3K] / rewards_out [T,N] f32 / dones_out [T,N] u8 redirect the
+        batch t % B (T defaults to B).  obs_out [T,N,H,W,3K] ([T,N,V,V] in grid mode) / rewards_out [T,N] f32 / dones_out [T,N] u8 redirect the
         per-step outputs into rollout slots; without them every step writes the env's own buffers."""
         a = actions
         assert a.is_cuda and a.dtype == torch.int8 and a.is_contiguous() and tuple(a.shape[1:]) == (self.N, self.S)
@@ -793,8 +812,12 @@ class SnakeVecEnv(object):
         d["kernel"] = ("k_step_lane", "k_step_tile", "k_step_dense", "k_step_rows")[d["kind"]]
         f = (C.c_int32 * 4)()
         _lib.check(self._L.snk_launch_form(self._h, f))
+        if self.obs_mode == "grid" and d["kind"] == 3:
+            d["kernel"] = "k_step_rows (grid)"
         if d["kind"] == 0:  # the lane path has three forms; the handle may move between the fused and the two-kernel one by itself
             d["kernel"] = {0: "k_step_lane", 1: "k_step_lane_ws", 3: "k_lane_logic + k_lane_paint2"}[f[0]]
+            if self.obs_mode == "grid":
+                d["kernel"] = "k_lane_logic + k_lane_grid"
             d["envs_per_warp_batch"], d["envs_per_image"], d["adaptive"] = int(f[1]), int(f[2]), bool(f[3])
         return d
 
@@ -802,6 +825,34 @@ class SnakeVecEnv(object):
         out = C.c_double(0)
         _lib.check(self._L.snk_algorithmic_bytes_per_step(C.byref(self.cfg), float(mean_sum_len), C.byref(out)))
         return out.value
+
+
+def expand_views(grid, n_views, first_view=0, out=None):
+    """Cell-code grids (obs_mode 'grid') -> RGB views on the device (snk_expand_views).  `grid`: a CUDA uint8 tensor whose
+    last two dims are (V, V) -- an env's `obs`, a [T, N, V, V] rollout, a gathered minibatch.  Returns
+    [..., V, V, 3 * n_views]: views first_view .. first_view + n_views - 1 of every cell, byte-identical to those channels
+    of the native observation, so expand_views(env.obs, env.K) equals a native env's `obs` of the same state.  `out`
+    (uint8, that shape, contiguous, on the grid's device) is written instead of allocating.  Stream-ordered on the
+    current stream; no synchronisation."""
+    if not isinstance(grid, torch.Tensor) or not grid.is_cuda or grid.dtype != torch.uint8:
+        raise TypeError("grid must be a CUDA uint8 tensor")
+    if grid.dim() < 2 or grid.shape[-1] != grid.shape[-2]:
+        raise ValueError("the last two dims of a grid are (V, V), got %r" % (tuple(grid.shape),))
+    V, n_views, first_view = int(grid.shape[-1]), int(n_views), int(first_view)
+    shape = tuple(grid.shape) + (3 * n_views,)
+    if out is None:
+        out = torch.empty(shape, dtype=torch.uint8, device=grid.device)
+    elif (not isinstance(out, torch.Tensor) or tuple(out.shape) != shape or out.dtype != torch.uint8 or not out.is_contiguous()
+          or out.device != grid.device):
+        raise ValueError("out must be a contiguous uint8 tensor of shape %r on %s" % (shape, grid.device))
+    n = grid.numel() // (V * V)
+    if n == 0:
+        return out
+    g = grid.contiguous()
+    dev = grid.device.index or 0
+    stream = C.c_void_p(torch.cuda.current_stream(grid.device).cuda_stream)
+    _lib.check(_lib.lib().snk_expand_views(C.c_void_p(g.data_ptr()), n, V - 2, first_view, n_views, C.c_void_p(out.data_ptr()), dev, stream))
+    return out
 
 
 class EnvStates(object):
