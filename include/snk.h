@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SNK_VERSION 310 /* 0.3.1 */
+#define SNK_VERSION 320 /* 0.3.2 */
 
 /* error codes */
 #define SNK_OK 0
@@ -279,6 +279,47 @@ int snk_gae(const float* d_rewards, const float* d_values, const uint8_t* d_done
  * buffers take the vector path; any alignment is accepted. */
 int snk_expand_views(const uint8_t* d_grid, int64_t n, int32_t size, int32_t first_view, int32_t n_views,
                      uint8_t* d_out, int32_t device, void* stream);
+
+/* SNK_OBS_GRID -> the first layer of a policy network: a 3x3 SAME convolution 3 -> C (C = 32, the `custom` network of
+ * the reference's policies.py), + bias, ReLU, over view `view` of the grid scaled by 1/255, without the RGB image.
+ * Class order (the colour of view k at SNK_CELL_*, as c = 0..6):
+ *   0 empty (0, 0, 0)   1 fruit (255, 0, 0)   2 wall (255, 255, 255)   3 self body (0, 204, 0)   4 self head (191, 242, 191)
+ *   5 other body (0, 51, 204)   6 other head (128, 154, 230)
+ * A snake cell is "self" when its snake index equals `view`, so views >= S have no self cells; code 2 is class 0.  The
+ * zero padding of SAME is class 0.  Taps t = 3 dy + dx, dy, dx = 0..2 row-major over the kernel window, cell (y + dy - 1,
+ * x + dx - 1), as Conv2d's cross-correlation indexes weight[o][rgb][dy][dx].
+ * snk_grid_conv_in: d_table float [9][7][C], d_table[t][c][o] = sum_rgb weight[o][rgb][t] colour[c][rgb] / 255 (rows
+ * c = 0 are zero, since empty is black, and are not read: empty taps are skipped); d_bias float [C].  d_out float [n][V][V][C] (NHWC: a channels_last [n, C, V, V] tensor) receives
+ *   out[i][p][o] = max(0, bias[o] + sum_t table[t][class(grid[i][p + t])][o])   (taps summed in increasing t).
+ * snk_grid_conv_in_wgrad: d_out is that output (its zeros are the ReLU mask) and d_gout float [n][V][V][C] the gradient
+ * of the loss with respect to it.  d_hist float [9][7][C] receives
+ *   hist[t][c][o] = sum over cells p of every grid with class(grid[p + t]) == c of (out[p][o] > 0 ? gout[p][o] : 0),
+ * from which dweight[o][rgb][t] = sum_c colour[c][rgb] / 255 hist[t][c][o] and dbias[o] = sum_c hist[4][c][o].  Class 0
+ * is computed as the total minus classes 1..6.  Deterministic: the same inputs give the same bits on every call (per-CTA
+ * partials in shared memory, written to d_work, added up in a fixed order; no atomics).  d_work: at least
+ * SNK_GRID_CONV_WORK_BYTES(n * V * V) bytes, 4-byte aligned; never more than SNK_GRID_CONV_WORK_BYTES_MAX.
+ * Rejected (SNK_EINVAL): channels other than SNK_GRID_CONV_CHANNELS; size outside 1..254 (3 <= V <= 256); view outside
+ * 0..31; n < 0; a NULL buffer or, for snk_grid_conv_in, d_table / d_bias / d_out not 16-byte aligned; for the wgrad
+ * d_out / d_gout / d_hist / d_work not 4-byte aligned or work_bytes below the formula.  n = 0 does nothing (d_hist is
+ * not written).  Not tied to a handle; stream-ordered on `stream` on `device`, no allocation, no synchronisation, so
+ * both can be recorded into a CUDA graph. */
+#define SNK_GRID_CONV_CHANNELS 32
+#define SNK_GRID_CONV_CLASSES 7
+#define SNK_GRID_CONV_WGRAD_CELLS_PER_CTA 2048
+#define SNK_GRID_CONV_WGRAD_MAX_CTAS 592
+#define SNK_GRID_CONV_PART_FLOATS ((9 * (SNK_GRID_CONV_CLASSES - 1) + 1) * SNK_GRID_CONV_CHANNELS) /* per CTA */
+#define SNK_GRID_CONV_WORK_BYTES(n_cells)                                                                              \
+  ((size_t)((((n_cells) + SNK_GRID_CONV_WGRAD_CELLS_PER_CTA - 1) / SNK_GRID_CONV_WGRAD_CELLS_PER_CTA) <                \
+                    SNK_GRID_CONV_WGRAD_MAX_CTAS                                                                       \
+                ? (((n_cells) + SNK_GRID_CONV_WGRAD_CELLS_PER_CTA - 1) / SNK_GRID_CONV_WGRAD_CELLS_PER_CTA)            \
+                : SNK_GRID_CONV_WGRAD_MAX_CTAS) *                                                                      \
+   SNK_GRID_CONV_PART_FLOATS * 4)
+#define SNK_GRID_CONV_WORK_BYTES_MAX ((size_t)SNK_GRID_CONV_WGRAD_MAX_CTAS * SNK_GRID_CONV_PART_FLOATS * 4)
+int snk_grid_conv_in(const uint8_t* d_grid, int64_t n, int32_t size, int32_t view, const float* d_table,
+                     const float* d_bias, int32_t channels, float* d_out, int32_t device, void* stream);
+int snk_grid_conv_in_wgrad(const uint8_t* d_grid, int64_t n, int32_t size, int32_t view, const float* d_out,
+                           const float* d_gout, int32_t channels, float* d_hist, void* d_work, size_t work_bytes,
+                           int32_t device, void* stream);
 
 /* Replay mode: per-env tapes of the reference's np_random.randint draws
  * (snake_multiple_test.py:200, :215).  CSR: env i owns vals/bounds[offsets[i] .. offsets[i+1]).

@@ -22,6 +22,20 @@ def cell_body(s):
 
 def cell_head(s):
     return 4 + 2 * s
+
+# snk_grid_conv_in (SNK_GRID_CONV_* of include/snk.h): classes of a cell in view k, their RGB colours, the workspace
+GRID_CONV_CHANNELS = 32
+GRID_CONV_COLOURS = ((0, 0, 0), (255, 0, 0), (255, 255, 255), (0, 204, 0), (191, 242, 191), (0, 51, 204), (128, 154, 230))
+GRID_CONV_WGRAD_CELLS_PER_CTA, GRID_CONV_WGRAD_MAX_CTAS = 2048, 592
+GRID_CONV_PART_FLOATS = (9 * (len(GRID_CONV_COLOURS) - 1) + 1) * GRID_CONV_CHANNELS
+
+
+def grid_conv_work_bytes(n_cells):
+    """SNK_GRID_CONV_WORK_BYTES: the workspace snk_grid_conv_in_wgrad needs for n_cells = n * V * V."""
+    ctas = min(-(-int(n_cells) // GRID_CONV_WGRAD_CELLS_PER_CTA), GRID_CONV_WGRAD_MAX_CTAS)
+    return ctas * GRID_CONV_PART_FLOATS * 4
+
+
 RNG_PHILOX, RNG_TAPE = 0, 1
 NSTATS = 8
 STAT_NAMES = ("env_steps", "episodes", "return_sum", "length_sum", "fruits", "deaths", "body_cells", "draws")
@@ -101,7 +115,11 @@ _SIGNATURES = {
     "snk_gae": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_double, C.c_int32, C.c_int64,
                           C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "snk_expand_views": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p]),
-    "snk_algorithmic_bytes_per_step": (C.c_int, [C.POINTER(SnkConfig), C.c_double, C.POINTER(C.c_double)]),
+    "snk_grid_conv_in": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
+                                   C.c_int32, C.c_void_p]),
+    "snk_grid_conv_in_wgrad": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
+                                         C.c_void_p, C.c_void_p, C.c_size_t, C.c_int32, C.c_void_p]),
+    "snk_algorithmic_bytes_per_step":(C.c_int, [C.POINTER(SnkConfig), C.c_double, C.POINTER(C.c_double)]),
     "snk_launch_count": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     "snk_launch_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),
     "snk_launch_form": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),

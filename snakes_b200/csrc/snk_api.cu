@@ -1467,6 +1467,49 @@ extern "C" int snk_expand_views(const uint8_t* d_grid, int64_t n, int32_t size, 
   return SNK_OK;
 }
 
+static int grid_conv_check(int64_t n, int32_t size, int32_t view, int32_t channels) {
+  if (channels != SNK_GRID_CONV_CHANNELS)
+    return fail(SNK_EINVAL, "channels must be %d, got %d", SNK_GRID_CONV_CHANNELS, channels);
+  if (size < 1 || size > 254) return fail(SNK_EINVAL, "size must be 1..254, got %d", size);
+  if (view < 0 || view > 31) return fail(SNK_EINVAL, "view must be 0..31, got %d", view);
+  if (n < 0) return fail(SNK_EINVAL, "n must be >= 0, got %lld", (long long)n);
+  return SNK_OK;
+}
+
+static bool misaligned(const void* p, uintptr_t a) { return ((uintptr_t)p & (a - 1)) != 0; }
+
+extern "C" int snk_grid_conv_in(const uint8_t* d_grid, int64_t n, int32_t size, int32_t view, const float* d_table,
+                                const float* d_bias, int32_t channels, float* d_out, int32_t device, void* stream) {
+  int rc = grid_conv_check(n, size, view, channels);
+  if (rc) return rc;
+  if (n == 0) return SNK_OK;
+  if (!d_grid || !d_table || !d_bias || !d_out) return fail(SNK_EINVAL, "NULL argument");
+  if (misaligned(d_table, 16) || misaligned(d_bias, 16) || misaligned(d_out, 16))
+    return fail(SNK_EINVAL, "d_table, d_bias and d_out must be 16-byte aligned");
+  CUDA_TRY(cudaSetDevice(device));
+  const long long V = size + 2;
+  CUDA_TRY(snk_launch_grid_conv_in(d_grid, n * V * V, (int)V, view, d_table, d_bias, d_out, (cudaStream_t)stream));
+  return SNK_OK;
+}
+
+extern "C" int snk_grid_conv_in_wgrad(const uint8_t* d_grid, int64_t n, int32_t size, int32_t view, const float* d_out,
+                                      const float* d_gout, int32_t channels, float* d_hist, void* d_work, size_t work_bytes,
+                                      int32_t device, void* stream) {
+  int rc = grid_conv_check(n, size, view, channels);
+  if (rc) return rc;
+  if (n == 0) return SNK_OK;
+  if (!d_grid || !d_out || !d_gout || !d_hist || !d_work) return fail(SNK_EINVAL, "NULL argument");
+  if (misaligned(d_out, 4) || misaligned(d_gout, 4) || misaligned(d_hist, 4) || misaligned(d_work, 4))
+    return fail(SNK_EINVAL, "d_out, d_gout, d_hist and d_work must be 4-byte aligned");
+  const long long V = size + 2, n_cells = n * V * V;
+  if (work_bytes < SNK_GRID_CONV_WORK_BYTES(n_cells))
+    return fail(SNK_EINVAL, "workspace too small: %zu < %zu bytes", work_bytes, (size_t)SNK_GRID_CONV_WORK_BYTES(n_cells));
+  CUDA_TRY(cudaSetDevice(device));
+  CUDA_TRY(snk_launch_grid_conv_in_wgrad(d_grid, n_cells, (int)V, view, d_out, d_gout, d_hist, (float*)d_work,
+                                         (cudaStream_t)stream));
+  return SNK_OK;
+}
+
 extern "C" int snk_algorithmic_bytes_per_step(const snk_config* c, double mean_sum_len, double* out) {
   int rc = cfg_check(c);
   if (rc) return rc;

@@ -34,6 +34,12 @@ cudaError_t snk_launch_restore(const Params& p, const int64_t* idx, long long co
 cudaError_t snk_launch_copy(const Params& p, const int64_t* src, const int64_t* dst, long long count, cudaStream_t stream);
 cudaError_t snk_launch_sum_inbox(const PeerArgs& a, const double* stats, double* glob, cudaStream_t stream);
 cudaError_t snk_launch_expand_views(const uint8_t* grid, long long n_cells, int first_view, int n_views, uint8_t* out, cudaStream_t stream);
+// snk_grid_conv.cu: the grid's first convolution layer (n_cells = n * V * V) and the CTA count of its weight gradient
+cudaError_t snk_launch_grid_conv_in(const uint8_t* grid, long long n_cells, int V, int view, const float* table,
+                                    const float* bias, float* out, cudaStream_t stream);
+cudaError_t snk_launch_grid_conv_in_wgrad(const uint8_t* grid, long long n_cells, int V, int view, const float* out,
+                                          const float* gout, float* hist, float* work, cudaStream_t stream);
+int snk_grid_conv_wgrad_ctas(long long n_cells);
 cudaError_t snk_launch_extract_views(const uint8_t* src, uint8_t* dst, long long n_pixels, int C, int n_out, cudaStream_t stream);
 cudaError_t snk_launch_scripted_actions(const Params& p, int8_t* actions, uint64_t step, uint64_t seed, int eps_permille,
                                         const uint8_t* occ_obs, cudaStream_t stream);

@@ -28,6 +28,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import rollout as _rollout
+from .grid_conv import grid_conv_in
 
 OPPONENT_SAVE_INTERVAL = 50   # config.py:13
 MAX_SAVED_OPPONENTS = 1000    # config.py:14
@@ -42,12 +43,18 @@ def _ortho_(w, scale):
 class CnnPolicy(nn.Module):
     """policies.py:40-67.  `arch='custom'` is custom_cnn (four 3x3 SAME convs 32-32-64-64, fc 512;
     Config.USE_ATARI_SIZE False), `arch='nature'` is nature_cnn (8/4, 4/2, 3/1 VALID convs, fc 512; 84x84
-    input).  Input: uint8 [B, H, W, C] exactly as the env writes it (NHWC); scaled by 1/255 here."""
+    input).  Input: uint8 [B, H, W, C] exactly as the env writes it (NHWC); scaled by 1/255 here.
 
-    def __init__(self, ob_shape, n_actions, arch="custom"):
+    `grid=True` (custom only): the input is a cell-code grid uint8 [B, V, V] (obs_mode 'grid') and the first conv, its
+    bias and ReLU are grid_conv_in on view `view` of it: the RGB view is never built.  The parameters are the same, so
+    the network, its checkpoints and to_tf_list / from_tf_list are those of the RGB policy of ob_shape (V, V, 3)."""
+
+    def __init__(self, ob_shape, n_actions, arch="custom", grid=False):
         super().__init__()
         h, w, c = ob_shape
-        self.ob_shape, self.n_actions, self.arch = tuple(ob_shape), int(n_actions), arch
+        self.ob_shape, self.n_actions, self.arch, self.grid = tuple(ob_shape), int(n_actions), arch, bool(grid)
+        if grid and (arch != "custom" or c != 3):
+            raise ValueError("grid=True needs arch 'custom' and ob_shape (V, V, 3): grid and atari84 are separate env modes")
         if arch == "nature":
             spec = [(32, 8, 4, 0), (64, 4, 2, 0), (64, 3, 1, 0)]
         elif arch == "custom":
@@ -71,10 +78,17 @@ class CnnPolicy(nn.Module):
         _ortho_(self.pi.weight, 0.01); nn.init.zeros_(self.pi.bias)
         _ortho_(self.v.weight, 1.0); nn.init.zeros_(self.v.bias)
 
-    def forward(self, ob):
-        x = ob.permute(0, 3, 1, 2).float() * (1.0 / 255.0)
-        x = x.contiguous(memory_format=torch.channels_last)
-        for conv in self.convs:
+    def forward(self, ob, view=0):
+        """(logits, value).  `view`: which snake's view of a grid input is read (a grid policy only; an RGB input is
+        already one view)."""
+        if self.grid:
+            x = grid_conv_in(ob, view, self.convs[0].weight, self.convs[0].bias)
+            convs = self.convs[1:]
+        else:
+            x = ob.permute(0, 3, 1, 2).float() * (1.0 / 255.0)
+            x = x.contiguous(memory_format=torch.channels_last)
+            convs = self.convs
+        for conv in convs:
             x = F.relu(conv(x))
         # conv_to_fc flattens NHWC (baselines.a2c.utils.conv_to_fc): keep that order so fc1 is interchangeable
         x = x.permute(0, 2, 3, 1).reshape(x.shape[0], -1)
@@ -82,16 +96,16 @@ class CnnPolicy(nn.Module):
         return self.pi(hid), self.v(hid)[:, 0]
 
     @torch.no_grad()
-    def step(self, ob):
+    def step(self, ob, view=0):
         """a0 = pd.sample(), vf, neglogp0 (policies.py:53-59); CategoricalPd samples with the Gumbel trick."""
-        logits, v = self.forward(ob)
+        logits, v = self.forward(ob, view)
         u = torch.rand_like(logits).clamp_(1e-20, 1.0)
         a = torch.argmax(logits - torch.log(-torch.log(u)), dim=-1)
         return a, v, F.cross_entropy(logits, a, reduction="none")
 
     @torch.no_grad()
-    def value(self, ob):
-        return self.forward(ob)[1]
+    def value(self, ob, view=0):
+        return self.forward(ob, view)[1]
 
     # ---- interchange with the reference's checkpoints (ppo_multi_agent_new.py:104-125, evaluate_snake.py:21-40):
     # joblib list of ndarrays in tf.trainable_variables order: c1/w, c1/b, ..., fc1/w, fc1/b, pi/w, pi/b, v/w, v/b
@@ -143,13 +157,14 @@ def ppo_loss(logits, vpred, actions, advs, returns, old_neglogp, old_v, cliprang
 
 
 class Model(object):
-    """ppo_multi_agent_new.py:48-135: one policy network with its PPO2 trainer, save / load."""
+    """ppo_multi_agent_new.py:48-135: one policy network with its PPO2 trainer, save / load.  `grid=True`: the network
+    reads cell-code grids (CnnPolicy grid=True); `step` / `value` take the view index, `train` reads view 0."""
 
     loss_names = ["policy_loss", "value_loss", "policy_entropy", "approxkl", "clipfrac"]
 
     def __init__(self, ob_shape, n_actions, ent_coef=0.01, vf_coef=0.5, max_grad_norm=0.5, arch="custom", device="cuda",
-                 trainable=True):
-        self.net = CnnPolicy(ob_shape, n_actions, arch).to(device).to(memory_format=torch.channels_last)
+                 trainable=True, grid=False):
+        self.net = CnnPolicy(ob_shape, n_actions, arch, grid).to(device).to(memory_format=torch.channels_last)
         self.ent_coef, self.vf_coef, self.max_grad_norm = ent_coef, vf_coef, max_grad_norm
         self.opt = torch.optim.Adam(self.net.parameters(), lr=2.5e-4, eps=1e-5) if trainable else None
         self.step, self.value = self.net.step, self.net.value
@@ -215,14 +230,19 @@ def sf01(t):
 
 
 class Runner(object):
-    """Runner of ppo_multi_agent_new.py:138-220 with every buffer on the device."""
+    """Runner of ppo_multi_agent_new.py:138-220 with every buffer on the device.
+
+    On an obs_mode 'grid' env (with grid models only) the rollout keeps cell-code grids: mb_obs is uint8 [nsteps, N, V, V],
+    the main model reads view 0 of a slot and opponent i view i + 1 of the same slot."""
 
     def __init__(self, env, model, opponent_models, nsteps, gamma=0.99, lam=0.95):
         self.env, self.model, self.opponents = env, model, list(opponent_models)
         self.nsteps, self.gamma, self.lam = nsteps, gamma, lam
         N, dev = env.num_envs, env.device
-        if getattr(env, "obs_mode", "native") == "grid":
-            raise ValueError("Runner keeps RGB views in its rollout: create the env with obs_mode 'native', not 'grid'")
+        self.grid = getattr(env, "obs_mode", "native") == "grid"
+        if self.grid:
+            self._init_grid(N, dev)
+            return
         h, w, c = env.observation_space.shape
         if c < 3 * (1 + len(self.opponents)):
             raise ValueError("the env must emit one view per controlled snake (n_views >= n_snakes)")
@@ -237,6 +257,57 @@ class Runner(object):
         self.full_actions = torch.zeros((N, env.S), dtype=torch.int8, device=dev)
         self.main_spare = torch.empty((N, h, w, 3), dtype=torch.uint8, device=dev)  # main view after the rollout's last step
         self.main_next = None
+
+    def _init_grid(self, N, dev):
+        env, nsteps = self.env, self.nsteps
+        if not all(getattr(getattr(m, "net", None), "grid", False) for m in [self.model] + [o for o in self.opponents if o is not None]):
+            raise ValueError("a grid env needs grid models (Model(..., grid=True)): the rollout keeps cell-code grids, not RGB views")
+        if 1 + len(self.opponents) > env.S:
+            raise ValueError("%d models for %d snakes: one model per controlled snake" % (1 + len(self.opponents), env.S))
+        V = env.V
+        # slots 16-byte aligned: the env writes a step's grid straight into one (set_obs_target)
+        slot = -(-N * V * V // 16) * 16
+        self.mb_obs = torch.empty((nsteps, slot), dtype=torch.uint8, device=dev)[:, :N * V * V].view(nsteps, N, V, V)
+        self.obs = env.reset()
+        self.dones = torch.zeros(N, dtype=torch.bool, device=dev)
+        self.mb_rewards = torch.empty((nsteps, N), dtype=torch.float32, device=dev)
+        self.mb_actions = torch.empty((nsteps, N), dtype=torch.int64, device=dev)
+        self.mb_values = torch.empty((nsteps, N), dtype=torch.float32, device=dev)
+        self.mb_neglogp = torch.empty((nsteps, N), dtype=torch.float32, device=dev)
+        self.mb_dones = torch.empty((nsteps, N), dtype=torch.bool, device=dev)
+        self.full_actions = torch.zeros((N, env.S), dtype=torch.int8, device=dev)
+
+    def _act_grid(self, grid):
+        """MultiModel.multi_step on one grid: the main model reads view 0, opponent i view i + 1."""
+        a, v, nlp = self.model.step(grid, 0)
+        self.full_actions[:, 0] = a.to(torch.int8)
+        for i, opp in enumerate(self.opponents):
+            self.full_actions[:, i + 1] = 1 if opp is None else opp.step(grid, i + 1)[0].to(torch.int8)
+        return a, v, nlp
+
+    def _run_grid(self):
+        """run() on a grid env: the env writes each step's grid into mb_obs[t + 1] through set_obs_target, and the last
+        step's into its own buffer (the target is switched off), so env.obs is the current grid, the env never holds a
+        pointer into the runner's memory, and slot 0 of the next rollout is one copy of it.  No view is expanded and no
+        step is copied."""
+        env = self.env
+        before = env.stats(False)
+        self.mb_obs[0].copy_(env.obs)
+        for t in range(self.nsteps):
+            a, v, nlp = self._act_grid(self.mb_obs[t])
+            self.mb_actions[t], self.mb_values[t], self.mb_neglogp[t] = a, v, nlp
+            self.mb_dones[t] = self.dones
+            env.set_obs_target(self.mb_obs[t + 1] if t + 1 < self.nsteps else None)
+            _, rew, dones, _ = env.step(self.full_actions)
+            self.mb_rewards[t] = rew
+            self.dones = dones.clone()
+        self.obs = env.obs
+        last_values = self.model.value(env.obs, 0)
+        advs, returns = _rollout.gae(self.mb_rewards, self.mb_values, self.mb_dones, last_values, self.dones, self.gamma, self.lam)
+        after = env.stats(False)
+        ep = {k: after[k] - before[k] for k in ("episodes", "return_sum", "length_sum")}
+        return (sf01(self.mb_obs), sf01(returns), sf01(self.mb_dones), sf01(self.mb_actions), sf01(self.mb_values),
+                sf01(self.mb_neglogp), None, ep)
 
     def _views(self):
         """use_multi_agent_obs (:161-165): view 0 is the main snake's, view i + 1 opponent i's."""
@@ -256,6 +327,8 @@ class Runner(object):
         returns straight into the slot the NEXT step's policy call reads it from (set_main_view_target: mb_obs[t + 1],
         the last one into a spare slot), so mb_obs is filled by the env and the policy reads a contiguous [N,H,W,3]
         tensor; the opponents' views stay in the env's own transient buffer."""
+        if self.grid:
+            return self._run_grid()
         env = self.env
         before = env.stats(False)
         for t in range(self.nsteps):
@@ -330,13 +403,14 @@ def learn(env, nsteps=128, total_timesteps=int(1e6), ent_coef=0.01, lr=2.5e-4, v
     clip_fn = cliprange if callable(cliprange) else (lambda _f, _v=cliprange: _v)
     rng = random.Random(seed)
     N, S, dev = env.num_envs, env.S, env.device
-    h, w, _ = env.observation_space.shape
+    h, w = env.observation_space.shape[:2]
     ob_shape = (h, w, 3)
+    grid = getattr(env, "obs_mode", "native") == "grid"   # grid models: the rollout and the minibatches hold cell codes
     n_act = env.action_space.n
     nbatch = N * nsteps
     assert nbatch % nminibatches == 0
     nbatch_train = nbatch // nminibatches
-    mk = lambda trainable: Model(ob_shape, n_act, ent_coef, vf_coef, max_grad_norm, arch, dev, trainable)
+    mk = lambda trainable: Model(ob_shape, n_act, ent_coef, vf_coef, max_grad_norm, arch, dev, trainable, grid)
     model = sync_model_across_ranks(mk(True))   # one model, N replicas: identical weights from the first update on
     opponent_models = [mk(False) for _ in range(S - 1)]
     # opponent sampling uses `rng`, seeded identically on every rank, so all ranks load the same past selves
