@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SNK_VERSION 320 /* 0.3.2 */
+#define SNK_VERSION 330 /* 0.3.3 */
 
 /* error codes */
 #define SNK_OK 0
@@ -320,6 +320,47 @@ int snk_grid_conv_in(const uint8_t* d_grid, int64_t n, int32_t size, int32_t vie
 int snk_grid_conv_in_wgrad(const uint8_t* d_grid, int64_t n, int32_t size, int32_t view, const float* d_out,
                            const float* d_gout, int32_t channels, float* d_hist, void* d_work, size_t work_bytes,
                            int32_t device, void* stream);
+
+/* SNK_OBS_GRID -> the first layer of the reference's `nature_cnn` on its WarpFrame view: an 8x8 stride-4 VALID
+ * convolution 3 -> C (C = 32) + bias, ReLU, over view `view` replicated f x f per cell to 84 x 84 and scaled by 1/255
+ * (the observation of SNK_OBS_ATARI84), without the image.  V = size + 2 must divide 84 with 3 <= V <= 42 (V = 3, 4, 6,
+ * 7, 12, 14, 21, 28, 42); f = 84 / V pixels per cell.  Classes and colours are those of snk_grid_conv_in.
+ * Output pixel (oy, ox), 0 <= oy, ox < 20, reads pixel rows 4 oy .. 4 oy + 7, i.e. cell rows floor(4 oy / f) + a.  How
+ * the 8 kernel rows fall on those cells depends only on the phase oy mod P, P = f / gcd(f, 4):
+ *   M[phi][a][d] = 1 if floor((4 phi + d) / f) - floor(4 phi / f) == a else 0     (0 <= a < C, 0 <= d < 8)
+ * with C the most cells a window spans per axis; block a of phase phi is reached when M[phi][a] is not all zero.
+ * snk_grid_conv84_geometry: out[0..3] = f, P, C and the workspace bytes snk_grid_conv84_in_wgrad needs for n grids.  Pure
+ * host arithmetic.  SNK_EINVAL for an unsupported size, n < 0 or a NULL out.
+ * snk_grid_conv84_in: d_table float [P][P][C][C][7][C_out],
+ *   table[py][px][a][b][c][o] = sum_{dy,dx} M[py][a][dy] M[px][b][dx] sum_rgb weight[o][rgb][dy][dx] colour[c][rgb] / 255
+ * (rows c = 0 are zero and not read: empty blocks are skipped); d_bias float [C_out].  d_out float [n][20][20][C_out]
+ * (NHWC: a channels_last [n, C_out, 20, 20] tensor) receives
+ *   out[i][oy][ox][o] = max(0, bias[o] + sum_{a,b} table[oy % P][ox % P][a][b][class(grid[i][cy + a][cx + b])][o]),
+ *   cy = floor(4 oy / f), cx = floor(4 ox / f), blocks summed in increasing a C + b, unreached blocks skipped.
+ * snk_grid_conv84_in_wgrad: d_out is that output (its zeros are the ReLU mask), d_gout float [n][20][20][C_out] the
+ * gradient of the loss with respect to it.  d_hist float [P][P][C][C][7][C_out] receives
+ *   hist[py][px][a][b][c][o] = sum over outputs (oy, ox) of every grid with oy % P = py, ox % P = px and
+ *                              class(grid[cy + a][cx + b]) == c of (out > 0 ? gout : 0)
+ * (zero for unreached blocks; class 0 is the phase's total minus classes 1..6), from which
+ *   dweight[o][rgb][dy][dx] = sum M[py][a][dy] M[px][b][dx] colour[c][rgb] / 255 hist[py][px][a][b][c][o]
+ *   dbias[o] = sum_{py,px,c} hist[py][px][0][0][c][o].
+ * Deterministic: the work is split by phase pair and the CTA count depends on (n, V) only; each CTA adds its warps' bins
+ * in warp order into one partial in d_work, and the partials are added in CTA order.  No atomics.  d_work: at least
+ * geometry's out[3] bytes, 4-byte aligned.
+ * Rejected (SNK_EINVAL): channels other than SNK_GRID_CONV_CHANNELS; an unsupported size; view outside 0..31; n < 0; a
+ * NULL buffer or, for snk_grid_conv84_in, d_table / d_bias / d_out not 16-byte aligned; for the wgrad d_out / d_gout /
+ * d_hist / d_work not 4-byte aligned or work_bytes below geometry's figure.  n = 0 does nothing (d_hist is not written).
+ * Not tied to a handle; stream-ordered on `stream` on `device`, no allocation, no synchronisation, so both can be
+ * recorded into a CUDA graph. */
+#define SNK_GRID_CONV84_OUT 20 /* output rows and columns */
+#define SNK_GRID_CONV84_WGRAD_OUTPUTS_PER_CTA 2048
+#define SNK_GRID_CONV84_WGRAD_MAX_CTAS 592
+int snk_grid_conv84_geometry(int32_t size, int64_t n, int64_t* out /*[4]: f, P, C, workspace bytes for n grids*/);
+int snk_grid_conv84_in(const uint8_t* d_grid, int64_t n, int32_t size, int32_t view, const float* d_table,
+                       const float* d_bias, int32_t channels, float* d_out, int32_t device, void* stream);
+int snk_grid_conv84_in_wgrad(const uint8_t* d_grid, int64_t n, int32_t size, int32_t view, const float* d_out,
+                             const float* d_gout, int32_t channels, float* d_hist, void* d_work, size_t work_bytes,
+                             int32_t device, void* stream);
 
 /* Replay mode: per-env tapes of the reference's np_random.randint draws
  * (snake_multiple_test.py:200, :215).  CSR: env i owns vals/bounds[offsets[i] .. offsets[i+1]).

@@ -36,6 +36,14 @@ def grid_conv_work_bytes(n_cells):
     return ctas * GRID_CONV_PART_FLOATS * 4
 
 
+def grid_conv84_geometry(V, n=0):
+    """snk_grid_conv84_geometry for V x V grids: (f, P, C, workspace bytes of snk_grid_conv84_in_wgrad for n grids).
+    Raises SnkError for a V that does not divide 84 or lies outside 3..42."""
+    out = (C.c_int64 * 4)()
+    check(lib().snk_grid_conv84_geometry(int(V) - 2, int(n), out))
+    return tuple(int(x) for x in out)
+
+
 RNG_PHILOX, RNG_TAPE = 0, 1
 NSTATS = 8
 STAT_NAMES = ("env_steps", "episodes", "return_sum", "length_sum", "fruits", "deaths", "body_cells", "draws")
@@ -119,6 +127,11 @@ _SIGNATURES = {
                                    C.c_int32, C.c_void_p]),
     "snk_grid_conv_in_wgrad": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
                                          C.c_void_p, C.c_void_p, C.c_size_t, C.c_int32, C.c_void_p]),
+    "snk_grid_conv84_geometry": (C.c_int, [C.c_int32, C.c_int64, C.POINTER(C.c_int64)]),
+    "snk_grid_conv84_in": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
+                                     C.c_int32, C.c_void_p]),
+    "snk_grid_conv84_in_wgrad": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
+                                           C.c_void_p, C.c_void_p, C.c_size_t, C.c_int32, C.c_void_p]),
     "snk_algorithmic_bytes_per_step":(C.c_int, [C.POINTER(SnkConfig), C.c_double, C.POINTER(C.c_double)]),
     "snk_launch_count": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     "snk_launch_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),

@@ -1510,6 +1510,57 @@ extern "C" int snk_grid_conv_in_wgrad(const uint8_t* d_grid, int64_t n, int32_t 
   return SNK_OK;
 }
 
+extern "C" int snk_grid_conv84_geometry(int32_t size, int64_t n, int64_t* out) {
+  GridConv84Geometry g;
+  if (!out) return fail(SNK_EINVAL, "out is NULL");
+  if (n < 0) return fail(SNK_EINVAL, "n must be >= 0, got %lld", (long long)n);
+  if (size < 1 || size > 40 || !snk_grid_conv84_geometry_of(size + 2, n, g))
+    return fail(SNK_EINVAL, "size %d: V = size + 2 must divide 84 with 3 <= V <= 42", size);
+  out[0] = g.f; out[1] = g.P; out[2] = g.C; out[3] = (int64_t)g.work_bytes;
+  return SNK_OK;
+}
+
+static int grid_conv84_check(int64_t n, int32_t size, int32_t view, int32_t channels, GridConv84Geometry& g) {
+  if (channels != SNK_GRID_CONV_CHANNELS)
+    return fail(SNK_EINVAL, "channels must be %d, got %d", SNK_GRID_CONV_CHANNELS, channels);
+  if (view < 0 || view > 31) return fail(SNK_EINVAL, "view must be 0..31, got %d", view);
+  if (n < 0) return fail(SNK_EINVAL, "n must be >= 0, got %lld", (long long)n);
+  if (size < 1 || size > 40 || !snk_grid_conv84_geometry_of(size + 2, n, g))
+    return fail(SNK_EINVAL, "size %d: V = size + 2 must divide 84 with 3 <= V <= 42", size);
+  return SNK_OK;
+}
+
+extern "C" int snk_grid_conv84_in(const uint8_t* d_grid, int64_t n, int32_t size, int32_t view, const float* d_table,
+                                  const float* d_bias, int32_t channels, float* d_out, int32_t device, void* stream) {
+  GridConv84Geometry g;
+  int rc = grid_conv84_check(n, size, view, channels, g);
+  if (rc) return rc;
+  if (n == 0) return SNK_OK;
+  if (!d_grid || !d_table || !d_bias || !d_out) return fail(SNK_EINVAL, "NULL argument");
+  if (misaligned(d_table, 16) || misaligned(d_bias, 16) || misaligned(d_out, 16))
+    return fail(SNK_EINVAL, "d_table, d_bias and d_out must be 16-byte aligned");
+  CUDA_TRY(cudaSetDevice(device));
+  CUDA_TRY(snk_launch_grid_conv84_in(d_grid, n, size + 2, view, d_table, d_bias, d_out, (cudaStream_t)stream));
+  return SNK_OK;
+}
+
+extern "C" int snk_grid_conv84_in_wgrad(const uint8_t* d_grid, int64_t n, int32_t size, int32_t view, const float* d_out,
+                                        const float* d_gout, int32_t channels, float* d_hist, void* d_work, size_t work_bytes,
+                                        int32_t device, void* stream) {
+  GridConv84Geometry g;
+  int rc = grid_conv84_check(n, size, view, channels, g);
+  if (rc) return rc;
+  if (n == 0) return SNK_OK;
+  if (!d_grid || !d_out || !d_gout || !d_hist || !d_work) return fail(SNK_EINVAL, "NULL argument");
+  if (misaligned(d_out, 4) || misaligned(d_gout, 4) || misaligned(d_hist, 4) || misaligned(d_work, 4))
+    return fail(SNK_EINVAL, "d_out, d_gout, d_hist and d_work must be 4-byte aligned");
+  if (work_bytes < g.work_bytes) return fail(SNK_EINVAL, "workspace too small: %zu < %zu bytes", work_bytes, g.work_bytes);
+  CUDA_TRY(cudaSetDevice(device));
+  CUDA_TRY(snk_launch_grid_conv84_in_wgrad(d_grid, n, size + 2, view, d_out, d_gout, d_hist, (float*)d_work,
+                                           (cudaStream_t)stream));
+  return SNK_OK;
+}
+
 extern "C" int snk_algorithmic_bytes_per_step(const snk_config* c, double mean_sum_len, double* out) {
   int rc = cfg_check(c);
   if (rc) return rc;

@@ -12,6 +12,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "snk_grid_class.cuh"
 #include "snk_launch.h"
 
 typedef unsigned char u8;
@@ -21,13 +22,6 @@ static constexpr int FW_THREADS = 256, FW_CELLS = 1024;  // forward: cells per c
 static constexpr int WG_WARPS = 6;                        // wgrad: warps per CTA, each with private bins (41 KB of shared per CTA)
 static constexpr int WG_ROWS = SNK_GRID_CONV_PART_FLOATS / GC_C;  // 9 taps x classes 1..6, then the total row
 static_assert(WG_ROWS == GC_TAPS * (GC_CLS - 1) + 1, "the partial layout of snk.h");
-
-// class of a cell code in view `view` (the order of SNK_GRID_CONV_CLASSES; code 2 is unused and drawn black)
-static __device__ __forceinline__ unsigned cell_class(unsigned c, int view) {
-  if (c == SNK_CELL_WALL) return 2u;
-  if (c < 3u) return c == SNK_CELL_FRUIT ? 1u : 0u;
-  return (((c - 3u) >> 1) == (unsigned)view ? 3u : 5u) + ((c - 3u) & 1u);
-}
 
 // the nine tap classes of cell (y, x); `cls` points at the cell in a row-major class image of width V that holds its
 // rows y - 1 .. y + 1 (rows outside 0 .. V - 1 are not read: off the image is empty)

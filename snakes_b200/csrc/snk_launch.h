@@ -40,6 +40,17 @@ cudaError_t snk_launch_grid_conv_in(const uint8_t* grid, long long n_cells, int 
 cudaError_t snk_launch_grid_conv_in_wgrad(const uint8_t* grid, long long n_cells, int V, int view, const float* out,
                                           const float* gout, float* hist, float* work, cudaStream_t stream);
 int snk_grid_conv_wgrad_ctas(long long n_cells);
+// snk_grid_conv84.cu: nature_cnn's first layer on the WarpFrame view of a grid (n grids of V x V).  Geometry: f, P, C of
+// include/snk.h, K weight-gradient CTAs per phase pair and the workspace; false for an unsupported V or n < 0.
+struct GridConv84Geometry {
+  int f, P, C, K;
+  size_t work_bytes;
+};
+bool snk_grid_conv84_geometry_of(int V, long long n, GridConv84Geometry& g);
+cudaError_t snk_launch_grid_conv84_in(const uint8_t* grid, long long n, int V, int view, const float* table, const float* bias,
+                                      float* out, cudaStream_t stream);
+cudaError_t snk_launch_grid_conv84_in_wgrad(const uint8_t* grid, long long n, int V, int view, const float* out, const float* gout,
+                                            float* hist, float* work, cudaStream_t stream);
 cudaError_t snk_launch_extract_views(const uint8_t* src, uint8_t* dst, long long n_pixels, int C, int n_out, cudaStream_t stream);
 cudaError_t snk_launch_scripted_actions(const Params& p, int8_t* actions, uint64_t step, uint64_t seed, int eps_permille,
                                         const uint8_t* occ_obs, cudaStream_t stream);

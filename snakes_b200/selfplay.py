@@ -28,7 +28,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import rollout as _rollout
-from .grid_conv import grid_conv_in
+from .grid_conv import conv84_supported, grid_conv84_in, grid_conv_in
 
 OPPONENT_SAVE_INTERVAL = 50   # config.py:13
 MAX_SAVED_OPPONENTS = 1000    # config.py:14
@@ -45,16 +45,22 @@ class CnnPolicy(nn.Module):
     Config.USE_ATARI_SIZE False), `arch='nature'` is nature_cnn (8/4, 4/2, 3/1 VALID convs, fc 512; 84x84
     input).  Input: uint8 [B, H, W, C] exactly as the env writes it (NHWC); scaled by 1/255 here.
 
-    `grid=True` (custom only): the input is a cell-code grid uint8 [B, V, V] (obs_mode 'grid') and the first conv, its
-    bias and ReLU are grid_conv_in on view `view` of it: the RGB view is never built.  The parameters are the same, so
-    the network, its checkpoints and to_tf_list / from_tf_list are those of the RGB policy of ob_shape (V, V, 3)."""
+    `grid=True`: the input is a cell-code grid uint8 [B, V, V] (obs_mode 'grid') and the first conv, its bias and ReLU
+    are computed from view `view` of it: the RGB view is never built.  `custom` (grid_conv_in) is the network of the RGB
+    policy of ob_shape (V, V, 3); `nature` (grid_conv84_in, V dividing 84 with 3 <= V <= 42) is nature_cnn on the 84x84
+    WarpFrame of the view, the network of the RGB policy of ob_shape (84, 84, 3) on an obs_mode 'atari84' env.  The
+    parameters are the same, so checkpoints and to_tf_list / from_tf_list move between the two."""
 
     def __init__(self, ob_shape, n_actions, arch="custom", grid=False):
         super().__init__()
         h, w, c = ob_shape
         self.ob_shape, self.n_actions, self.arch, self.grid = tuple(ob_shape), int(n_actions), arch, bool(grid)
-        if grid and (arch != "custom" or c != 3):
-            raise ValueError("grid=True needs arch 'custom' and ob_shape (V, V, 3): grid and atari84 are separate env modes")
+        if grid and c != 3:
+            raise ValueError("grid=True needs ob_shape (V, V, 3), got %r" % (tuple(ob_shape),))
+        if grid and arch == "nature":
+            if h != w or not conv84_supported(h):
+                raise ValueError("grid=True with arch 'nature' needs V dividing 84 with 3 <= V <= 42, got V = %d" % h)
+            h = w = 84   # the network sees the WarpFrame view
         if arch == "nature":
             spec = [(32, 8, 4, 0), (64, 4, 2, 0), (64, 3, 1, 0)]
         elif arch == "custom":
@@ -82,7 +88,8 @@ class CnnPolicy(nn.Module):
         """(logits, value).  `view`: which snake's view of a grid input is read (a grid policy only; an RGB input is
         already one view)."""
         if self.grid:
-            x = grid_conv_in(ob, view, self.convs[0].weight, self.convs[0].bias)
+            conv_in = grid_conv84_in if self.arch == "nature" else grid_conv_in
+            x = conv_in(ob, view, self.convs[0].weight, self.convs[0].bias)
             convs = self.convs[1:]
         else:
             x = ob.permute(0, 3, 1, 2).float() * (1.0 / 255.0)

@@ -1,6 +1,6 @@
 """The self-play learner on grids against the RGB learner: the first conv layer alone, then Runner.run and Model.train.
 
-    python tools/grid_learner_probe.py [--rounds R] [--out FILE]
+    python tools/grid_learner_probe.py [--rounds R] [--out FILE] [--arch custom|nature]
 
 1. Input stage at n in {1 024, 32 768, 131 072} grids of V in {21, 12} (live grid envs, 2 snakes, after 30 steps):
    grid_conv_in forward (snk_grid_conv_in) and backward (snk_grid_conv_in_wgrad + the fold into dW / dbias; also the two
@@ -12,6 +12,10 @@
 2. Runner.run time per rollout step (16 steps, main model and one opponent) and Model.train time per minibatch
    (N * 16 / 4 samples, at most 32 768) for 2 snakes on 19 x 19 at N in {32, 4 096, 16 384}, native env + RGB models
    against grid env + grid models, torch defaults (cuDNN TF32 on).  And the bytes of mb_obs.
+--arch nature: the same for nature_cnn on the 84 x 84 WarpFrame view: grid_conv84_in (snk_grid_conv84_in / _wgrad) against
+the RGB stage on the WarpFrame of the same grids (uint8 84 x 84 -> float, channels_last, cuDNN 8x8 stride-4 conv1 + ReLU),
+bytes n V^2 + n 400 * 128 forward and n V^2 + 2 n 400 * 128 backward; and the learner as obs_mode 'atari84' env + RGB
+nature models against grid env + grid nature models.
 Every time is CUDA events (or a host clock around work that ends in a synchronise) over repeated calls after untimed warm-up
 calls of the same shapes; native and grid alternate `rounds` times, rows give the mean and the spread over the rounds.  The
 card's name and power limit are printed with the numbers.  Needs a GPU; writes nothing but --out."""
@@ -59,29 +63,41 @@ def live_grids(sb, n, V, seed=0):
     return g
 
 
-def input_stage(sb, say, rounds):
+def input_stage(sb, say, rounds, arch="custom"):
     from snakes_b200 import _lib
     torch.manual_seed(0)
-    conv = torch.nn.Conv2d(3, 32, 3, 1, 1).cuda()
+    nature = arch == "nature"
+    conv = (torch.nn.Conv2d(3, 32, 8, 4) if nature else torch.nn.Conv2d(3, 32, 3, 1, 1)).cuda()
     w, b = conv.weight, conv.bias
-    say("\n1. input stage (first conv + bias + ReLU), view 0; us per call, mean [min-max] over %d rounds" % rounds)
+    conv_in, wgrad = (sb.grid_conv84_in, "snk_grid_conv84_in_wgrad") if nature else (sb.grid_conv_in, "snk_grid_conv_in_wgrad")
+    say("\n1. input stage (first conv + bias + ReLU), view 0; us per call, mean [min-max] over %d rounds" % rounds
+        + ("; nature_cnn on the 84x84 WarpFrame" if nature else ""))
     say("%-14s %-26s %24s %24s %10s %10s" % ("shape", "path", "forward", "backward", "fwd GB/s", "bwd GB/s"))
     for V in (21, 12):
         for n in (1024, 32768, 131072):
             g = live_grids(sb, n, V)
             x = sb.expand_views(g, 1)
+            if nature:   # the obs_mode 'atari84' view: every cell replicated 84 / V times
+                x = x.repeat_interleave(84 // V, 1).repeat_interleave(84 // V, 2).contiguous()
             cells = n * V * V
-            reps = max(3, min(50, int(2e10 // (cells * 128))))
-            gy = torch.randn((n, V, V, 32), device="cuda").permute(0, 3, 1, 2)   # channels_last, as conv2 hands it back
-            hist = torch.empty((9, 7, 32), device="cuda")
-            work = torch.empty((_lib.grid_conv_work_bytes(cells) // 4,), device="cuda")
+            side = 20 if nature else V   # output rows and columns
+            outs = n * side * side
+            reps = max(3, min(50, int(2e10 // (outs * 128))))
+            gy = torch.randn((n, side, side, 32), device="cuda").permute(0, 3, 1, 2)   # channels_last, as conv2 hands it back
+            if nature:
+                _, P, Cb, wbytes = _lib.grid_conv84_geometry(V, n)
+                hist = torch.empty((P, P, Cb, Cb, 7, 32), device="cuda")
+            else:
+                wbytes = _lib.grid_conv_work_bytes(cells)
+                hist = torch.empty((9, 7, 32), device="cuda")
+            work = torch.empty((wbytes // 4,), device="cuda")
             L, st = _lib.lib(), C.c_void_p(torch.cuda.current_stream().cuda_stream)
 
             def grid_fwd():
                 with torch.no_grad():
-                    return sb.grid_conv_in(g, 0, w, b)
+                    return conv_in(g, 0, w, b)
 
-            yg = sb.grid_conv_in(g, 0, w, b)
+            yg = conv_in(g, 0, w, b)
             go = gy.permute(0, 2, 3, 1)
             yo = yg.permute(0, 2, 3, 1)
 
@@ -89,9 +105,9 @@ def input_stage(sb, say, rounds):
                 torch.autograd.grad(yg, (w, b), gy, retain_graph=True)
 
             def grid_wgrad_kernels():
-                _lib.check(L.snk_grid_conv_in_wgrad(C.c_void_p(g.data_ptr()), n, V - 2, 0, C.c_void_p(yo.data_ptr()),
-                                                    C.c_void_p(go.data_ptr()), 32, C.c_void_p(hist.data_ptr()),
-                                                    C.c_void_p(work.data_ptr()), work.numel() * 4, 0, st))
+                _lib.check(getattr(L, wgrad)(C.c_void_p(g.data_ptr()), n, V - 2, 0, C.c_void_p(yo.data_ptr()),
+                                             C.c_void_p(go.data_ptr()), 32, C.c_void_p(hist.data_ptr()),
+                                             C.c_void_p(work.data_ptr()), work.numel() * 4, 0, st))
 
             def rgb_out():
                 xf = x.permute(0, 3, 1, 2).float() * (1.0 / 255.0)
@@ -117,7 +133,7 @@ def input_stage(sb, say, rounds):
                 res["grid kernels"][0].append(res["grid"][0][-1])
                 res["grid kernels"][1].append(events(grid_wgrad_kernels, reps))
             torch.backends.cudnn.allow_tf32 = True
-            fb, bb = cells * (1 + 128), cells * (1 + 256)
+            fb, bb = cells + outs * 128, cells + outs * 256
             for k, (f, bw) in res.items():
                 gf, gb = fb / (np.mean(f) * 1e-6) / 1e9, bb / (np.mean(bw) * 1e-6) / 1e9
                 note = ""
@@ -129,19 +145,22 @@ def input_stage(sb, say, rounds):
             torch.cuda.empty_cache()
 
 
-def learner(sb, say, rounds):
+def learner(sb, say, rounds, arch="custom"):
     from snakes_b200 import selfplay
     nsteps = 16
-    say("\n2. learner, 2 snakes on 19x19, nsteps %d, one opponent model; ms, mean [min-max] over %d rounds" % (nsteps, rounds))
+    nature = arch == "nature"
+    say("\n2. learner, 2 snakes on 19x19, nsteps %d, one opponent model; ms, mean [min-max] over %d rounds" % (nsteps, rounds)
+        + ("; nature_cnn, atari84 env + RGB models against grid env + grid models" if nature else ""))
     say("%-8s %-7s %28s %28s %16s" % ("N", "mode", "Runner.run per step", "Model.train per minibatch", "mb_obs bytes"))
     for N in (32, 4096, 16384):
         setups = {}
-        for mode in ("native", "grid"):
+        for mode in ("atari84" if nature else "native", "grid"):
             torch.manual_seed(0)
             env = sb.SnakeVecEnv(N, size=19, n_snakes=2, seed=1, obs_mode=mode)
             grid = mode == "grid"
-            model = selfplay.Model((21, 21, 3), 5, device=env.device, grid=grid)
-            opp = selfplay.Model((21, 21, 3), 5, device=env.device, trainable=False, grid=grid)
+            shape = (84, 84, 3) if mode == "atari84" else (21, 21, 3)
+            model = selfplay.Model(shape, 5, arch=arch, device=env.device, grid=grid)
+            opp = selfplay.Model(shape, 5, arch=arch, device=env.device, trainable=False, grid=grid)
             runner = selfplay.Runner(env, model, [opp], nsteps)
             setups[mode] = (env, model, runner)
         mb_size = min(N * nsteps // 4, 32768)
@@ -180,6 +199,7 @@ def main():
     ap.add_argument("--rounds", type=int, default=3)
     ap.add_argument("--out", default=None)
     ap.add_argument("--part", choices=("all", "input", "learner"), default="all")
+    ap.add_argument("--arch", choices=("custom", "nature"), default="custom")
     args = ap.parse_args()
     assert torch.cuda.is_available(), "the probe needs a CUDA device"
     import snakes_b200 as sb
@@ -192,9 +212,9 @@ def main():
     say("card: %s" % card())
     say("torch %s, cuDNN %s" % (torch.__version__, torch.backends.cudnn.version()))
     if args.part in ("all", "input"):
-        input_stage(sb, say, args.rounds)
+        input_stage(sb, say, args.rounds, args.arch)
     if args.part in ("all", "learner"):
-        learner(sb, say, args.rounds)
+        learner(sb, say, args.rounds, args.arch)
     if args.out:
         with open(args.out, "w") as f:
             f.write("\n".join(lines) + "\n")
