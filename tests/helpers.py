@@ -1,4 +1,5 @@
 """Shared helpers for the parity tests: golden loading, state digests, oracle runners."""
+import ctypes
 import glob
 import json
 import os
@@ -133,4 +134,21 @@ def random_long_snake_states(lay, cfg, rng, min_len=20, max_len=70):
                 st["fruit_grid"][e, pid(fx, fy)] += 1
             else:
                 st["fruit"][e, f] = pid(fx, fy)
+    return blob
+
+
+def tiled_long_snake_states(lay, cfg, rng, pool=256):
+    """random_long_snake_states for a batch too large to walk env by env in Python: `pool` envs are drawn and env e
+    takes state e % pool.  Twins part at their first draw, which is keyed by the global env id.  `cfg` / `lay`: the
+    oracle's (c_oracle.Config / Layout)."""
+    sub = c_oracle.Config.from_buffer_copy(cfg)
+    sub.num_envs = min(pool, cfg.num_envs)
+    sub_lay = c_oracle.Layout()
+    c_oracle.lib().so_state_layout_of(ctypes.byref(sub), ctypes.byref(sub_lay))
+    src = c_oracle.split_state(random_long_snake_states(sub_lay, sub, rng), sub_lay, sub)
+    blob = np.zeros(lay.total_bytes, dtype=np.uint8)
+    dst = c_oracle.split_state(blob, lay, cfg)
+    idx = np.arange(cfg.num_envs) % sub.num_envs
+    for k in dst:
+        dst[k][...] = src[k][idx]
     return blob
