@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SNK_VERSION 330 /* 0.3.3 */
+#define SNK_VERSION 340 /* 0.3.4 */
 
 /* error codes */
 #define SNK_OK 0
@@ -453,6 +453,41 @@ int snk_gen_actions(snk_handle* h, int8_t* d_actions, uint64_t step, uint64_t se
  * SigmaL, fewer resets).  Lane-family configurations with classic fruit lists only. */
 int snk_gen_scripted_actions(snk_handle* h, int8_t* d_actions, uint64_t step, uint64_t seed,
                              int32_t eps_permille, void* stream);
+
+/* Head-to-head evaluation (the reference's evaluate_snake.py, played over many envs at once; DESIGN.md section 4.18).
+ * Outcome of one episode of one env: let d_s be the step within the episode at which seat s got reward -1 (it died), or
+ * +infinity if it never did.  Seat s WINS if d_s > d_j for every other seat j, DRAWS if d_s >= d_j for every j and
+ * d_s == d_j for at least one j != s, and otherwise LOSES.  Under the reference's rules (an episode ends when seat 0 dies
+ * or at max_steps) both seats alive at the timeout is a draw, dying on the same step is a draw, seat 1 dying first and
+ * seat 0 later is a win for seat 0, and at S = 1 every episode is a win (only the score fields mean anything).
+ * Per seat the counters also hold the fruits (sum of positive rewards; more than 1 on a step when fruit stacks on a cell
+ * under the adversarial and cut rules), deaths, steps alive (counting the death step; the episode length for a seat
+ * that survives), the sum of squared episode returns (return = fruits - 1 if the seat died, else fruits) and the sum of
+ * episode lengths.  Every counter is an int64 sum of integers, so a result is the same bits on every run.
+ * snk_tally_layout: out[0] = bytes of the work area for the handle (int32 step counter and episodes counted [N], death
+ * step and fruits [N][S] of the running episode, each part 16-byte aligned), out[1] = SNK_TALLY_FIELDS.  Host only.
+ * snk_tally, launched after every snk_step on the step's stream (one kernel): reads the handle's d_reward_all, d_done and
+ * d_episode_len, and d_group (int32 [N]: the counter group of every env).  Every finished episode of an env adds its
+ * outcome per seat to d_counts (int64 [n_groups][S][SNK_TALLY_FIELDS]) row d_group[env].  An env that has counted
+ * episodes_per_env episodes is ignored from then on, and *d_envs_done (int64) counts such envs: poll it until it
+ * reaches N and every env has contributed exactly episodes_per_env episodes.  The caller zeroes d_work, d_counts and
+ * d_envs_done when it resets the envs (snk_reset), and the handle must auto-reset.  Stream-ordered, no allocation, no
+ * synchronisation, so it can be recorded into a CUDA graph.
+ * Rejected (SNK_EINVAL, before any CUDA call): n_groups < 1, episodes_per_env < 1, a NULL argument, d_group not 4-byte,
+ * d_work not 16-byte, d_counts or d_envs_done not 8-byte aligned.  A group id outside [0, n_groups) raises
+ * SNK_DEVERR_BAD_STATE (read it with snk_check_errors) and that env is skipped: it is never counted and never finished. */
+#define SNK_TALLY_WINS 0
+#define SNK_TALLY_DRAWS 1
+#define SNK_TALLY_LOSSES 2
+#define SNK_TALLY_FRUITS 3
+#define SNK_TALLY_DEATHS 4
+#define SNK_TALLY_STEPS_ALIVE 5
+#define SNK_TALLY_RETURN_SQ 6
+#define SNK_TALLY_LENGTH 7
+#define SNK_TALLY_FIELDS 8
+int snk_tally_layout(const snk_handle* h, size_t* out /*[2]*/);
+int snk_tally(snk_handle* h, const int32_t* d_group, int32_t n_groups, int32_t episodes_per_env, void* d_work,
+              int64_t* d_counts, int64_t* d_envs_done, void* stream);
 
 /* Algorithmic bytes of one env-step (SURVEY.md section 8d): obs K*H*W*3 + state 19S + 2*SigmaL + 2F + 30. */
 int snk_algorithmic_bytes_per_step(const snk_config* cfg, double mean_sum_len, double* out);

@@ -50,6 +50,8 @@ STAT_NAMES = ("env_steps", "episodes", "return_sum", "length_sum", "fruits", "de
 DEVERR = {1: "draw tape underrun", 2: "draw tape bound mismatch", 4: "fruit count overflow", 8: "body ring overflow",
           16: "bad state (non-adjacent segments, cell id or length out of range) or env index out of range"}
 GRAPH_SYNC_BACK = 1
+# snk_tally counters (SNK_TALLY_* of include/snk.h): [n_groups][S][fields] int64, in this order
+TALLY_FIELDS = ("wins", "draws", "losses", "fruits", "deaths", "steps_alive", "return_sq", "length")
 
 
 class SnkConfig(C.Structure):
@@ -132,6 +134,8 @@ _SIGNATURES = {
                                      C.c_int32, C.c_void_p]),
     "snk_grid_conv84_in_wgrad": (C.c_int, [C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32,
                                            C.c_void_p, C.c_void_p, C.c_size_t, C.c_int32, C.c_void_p]),
+    "snk_tally_layout": (C.c_int, [C.c_void_p, C.POINTER(C.c_size_t)]),
+    "snk_tally": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "snk_algorithmic_bytes_per_step":(C.c_int, [C.POINTER(SnkConfig), C.c_double, C.POINTER(C.c_double)]),
     "snk_launch_count": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     "snk_launch_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),

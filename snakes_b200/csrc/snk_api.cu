@@ -1478,6 +1478,45 @@ static int grid_conv_check(int64_t n, int32_t size, int32_t view, int32_t channe
 
 static bool misaligned(const void* p, uintptr_t a) { return ((uintptr_t)p & (a - 1)) != 0; }
 
+// the work area of snk_tally: t [N] | episodes [N] | death [N][S] | fruits [N][S], each part 16-byte aligned
+static size_t tally_work_bytes(long long N, int S, size_t off[4]) {
+  const size_t env = align16((size_t)N * 4), seat = align16((size_t)N * S * 4);
+  off[0] = 0; off[1] = env; off[2] = 2 * env; off[3] = 2 * env + seat;
+  return 2 * env + 2 * seat;
+}
+
+extern "C" int snk_tally_layout(const snk_handle* h, size_t* out) {
+  if (!h || !out) return fail(SNK_EINVAL, "NULL argument");
+  size_t off[4];
+  out[0] = tally_work_bytes(h->p.N, h->p.S, off);
+  out[1] = SNK_TALLY_FIELDS;
+  return SNK_OK;
+}
+
+extern "C" int snk_tally(snk_handle* h, const int32_t* d_group, int32_t n_groups, int32_t episodes_per_env, void* d_work,
+                         int64_t* d_counts, int64_t* d_envs_done, void* stream) {
+  if (n_groups < 1) return fail(SNK_EINVAL, "n_groups must be >= 1, got %d", n_groups);
+  if (episodes_per_env < 1) return fail(SNK_EINVAL, "episodes_per_env must be >= 1, got %d", episodes_per_env);
+  if (!d_group || !d_work || !d_counts || !d_envs_done) return fail(SNK_EINVAL, "NULL argument");
+  if (misaligned(d_group, 4)) return fail(SNK_EINVAL, "d_group must be 4-byte aligned");
+  if (misaligned(d_work, 16)) return fail(SNK_EINVAL, "d_work must be 16-byte aligned");
+  if (misaligned(d_counts, 8) || misaligned(d_envs_done, 8)) return fail(SNK_EINVAL, "d_counts and d_envs_done must be 8-byte aligned");
+  if (!h) return fail(SNK_EINVAL, "handle is NULL");
+  CUDA_TRY(cudaSetDevice(h->cfg.device));
+  const Params& p = h->p;
+  size_t off[4];
+  tally_work_bytes(p.N, p.S, off);
+  uint8_t* w = (uint8_t*)d_work;
+  TallyArgs a;
+  a.reward_all = p.reward_all; a.done = p.done; a.ep_len = p.fin_len; a.group = d_group;
+  a.t = (int32_t*)(w + off[0]); a.episodes = (int32_t*)(w + off[1]); a.death = (int32_t*)(w + off[2]); a.fruits = (int32_t*)(w + off[3]);
+  a.counts = d_counts; a.envs_done = d_envs_done; a.err = p.err;
+  a.N = p.N; a.S = p.S; a.n_groups = n_groups; a.episodes_per_env = episodes_per_env;
+  CUDA_TRY(snk_launch_tally(a, (cudaStream_t)stream));
+  h->launches++;
+  return SNK_OK;
+}
+
 extern "C" int snk_grid_conv_in(const uint8_t* d_grid, int64_t n, int32_t size, int32_t view, const float* d_table,
                                 const float* d_bias, int32_t channels, float* d_out, int32_t device, void* stream) {
   int rc = grid_conv_check(n, size, view, channels);

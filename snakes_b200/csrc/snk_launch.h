@@ -59,3 +59,20 @@ cudaError_t snk_launch_gae(const float* rewards, const float* values, const uint
                            cudaStream_t stream);
 cudaError_t snk_launch_gen_actions(int8_t* actions, long long N, int S, long long env_id_base, uint64_t step,
                                    uint64_t seed, int n_actions, cudaStream_t stream);
+// snk_arena.cu: per-seat match accounting after a step (snk_tally).  The work area of include/snk.h split into its parts.
+struct TallyArgs {
+  const float* reward_all;  // [N][S] the handle's per-step outputs
+  const uint8_t* done;
+  const int32_t* ep_len;
+  const int32_t* group;     // [N]
+  int32_t* t;               // [N] step within the running episode, -1 once the env has counted episodes_per_env episodes
+  int32_t* episodes;        // [N] episodes counted
+  int32_t* death;           // [N][S] step of the seat's death in the running episode, 0 = alive
+  int32_t* fruits;          // [N][S] fruits of the running episode
+  int64_t* counts;          // [n_groups][S][SNK_TALLY_FIELDS]
+  int64_t* envs_done;
+  uint32_t* err;
+  long long N;
+  int S, n_groups, episodes_per_env;
+};
+cudaError_t snk_launch_tally(const TallyArgs& a, cudaStream_t stream);
