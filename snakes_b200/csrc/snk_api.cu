@@ -67,7 +67,6 @@ struct snk_handle {
   // regime-adaptive lane path: `plan` is the fused kernel, `plan_alt` the two-kernel form (k_lane_logic + k_lane_paint2)
   LaunchPlan plan_alt;
   bool have_alt, use_alt;
-  int restore_thr_alt;
   double* h_regime;            // mapped pinned host memory [2]: env-steps, body cells (Params::regime_out)
   double reg_steps0, reg_cells0, alt_hi, alt_lo;
   const uint8_t* obs_current;  // where the native observations of the CURRENT state are (NULL: not encoded since the state changed)
@@ -185,6 +184,144 @@ static int restore_threshold(const Params& p, int threads) {
   const int border_units = (2 * (p.V * p.C + p.C) + (p.V - 3) * 2 * p.C) / U;
   const int stores = (int)((size_t)p.TE * p.E / (16 * threads)) + border_units / lanes_per_env;
   return stores / 16 < 3 ? 3 : stores / 16;
+}
+
+// Launch planning: fills h->plan, h->plan_alt and the lane geometry of h->p.  Decisions, in order: the kernel family,
+// a forced kernel, the lane path's form, small-shard batches, the regime-adaptive alternative.
+static int plan_launch(snk_handle* h) {
+  const std::string& dbg = h->debug;
+  Params& p = h->p;
+  const bool grid = h->cfg.obs_mode == SNK_OBS_GRID;
+  const int D = p.D, V = p.V, S = p.S, F = p.F, K = p.K;
+  const long long N = p.N;
+  LaunchPlan& plan = h->plan;
+  // grid = work: the CTAs it takes to cover every env
+  auto finish = [&](LaunchPlan& pl) {
+    return snk_plan(h->cfg.rules, pl, h->n_sm, S, K, (N + pl.envs_per_cta - 1) / pl.envs_per_cta);
+  };
+  // lane form `form` at te envs per warp image and epw envs per warp batch.  `threads` is what restore_threshold counts
+  // as sharing an image buffer: k_lane_grid and the adaptive alternative count k_lane_paint2's 64, the other lane
+  // plans a warp's 32.
+  auto plan_lane = [&](LaunchPlan& pl, int form, int te, int epw, int threads) {
+    p.TE = te; p.EPW = epw;
+    p.tile_stride = (int)(((size_t)te * p.E + 127) & ~(size_t)127);
+    p.n_groups = (N + epw - 1) / epw;
+    const bool two = form == FORM_LANE_SPLIT || form == FORM_LANE_GRID;  // the observation writer: one image per CTA
+    pl.form = form;
+    pl.block = form == FORM_LANE_WS ? 32 * (WS_PAINT_WARPS + WS_LOGIC_WARPS) : 64;
+    pl.smem = (size_t)(two ? 1 : 2) * p.tile_stride;
+    pl.envs_per_cta = two ? te : form == FORM_LANE_WS ? 32 * WS_LOGIC_WARPS : 2 * epw;  // fused: 2 warps per CTA
+    pl.restore_thr = dbg_int(dbg, "restore_thr", restore_threshold(p, threads));
+    return finish(pl);
+  };
+
+  // lane kernel (chain-coded bodies, lane per env) for small boards; otherwise the warp-per-env tile kernel while
+  // W observations + template + scratch leave room for >= 2 CTAs per SM; otherwise the CTA-per-env rows / dense kernel.
+  std::string force;
+  dbg_get(dbg, "force_kernel", &force);
+  int TE = 0;
+  if ((grid || snk_lane_supported(S, K)) && S <= 4 && F <= 4 && D <= 32) {  // grid: k_lane_grid exists for every K
+    const int cand[3] = {32, 16, 8};
+    for (int i = 0; i < 3 && !TE; ++i)
+      if (cand[i] % p.G == 0 && (size_t)cand[i] * p.E <= 28 * 1024) TE = cand[i];
+    if (!TE && p.G <= 8 && (size_t)8 * p.E <= 48 * 1024) TE = 8;
+  }
+  const int W = p.G > 8 ? p.G : 8;
+  const size_t smem_tile = (size_t)(W + p.G) * p.E + (size_t)W * (REC_SNAKE0 + 2 * S + (F + 1) / 2 + 3 + p.bm_words) * 4;
+  // rows kernel: chunks of R image rows must be 16-byte multiples (TMA) and fit a ~24 KB buffer
+  int R = 0;
+  if (p.E % 16 == 0 && !grid) {
+    const int unit = 16 / gcd(V * p.C, 16);
+    // chunk size and CTA shape measured on B200 at 16 snakes on 64x64: 4 warps (1 producer + 3 consumers) give 7 CTAs
+    // per SM, and 8 KB chunks beat 12 KB (32 768 envs: classic 1280 us, cut 1502 vs 1551 us)
+    const size_t lim = 8 * 1024;
+    for (int r = unit; r <= V && ((size_t)r * V * p.C <= lim || !R); r += unit) { if ((size_t)r * V * p.C > 48 * 1024) break; R = r; }
+  }
+  int form = TE ? FORM_LANE : smem_tile <= 110 * 1024 ? FORM_TILE : R ? FORM_ROWS : FORM_DENSE;
+  // grid: every ring-family geometry goes to the rows kernel's grid form (the producer's code grid IS the observation)
+  if (grid && form != FORM_LANE) form = FORM_ROWS;
+  if (force == "dense") form = FORM_DENSE;
+  if (force == "rows") {
+    if (!R && !grid) return fail(SNK_EINVAL, "rows kernel does not support this configuration");
+    form = FORM_ROWS;
+  }
+  if (force == "tile" && smem_tile <= 200 * 1024) form = FORM_TILE;
+  if (force == "lane" && !TE) return fail(SNK_EINVAL, "lane kernel does not support this configuration");
+  p.family = form == FORM_LANE;
+  if (form == FORM_LANE) {
+    // lane path forms (lane=fused|ws|split): every warp steps 32 envs then streams their images (default: fastest
+    // measured), warp-specialised single kernel, or two kernels
+    std::string lv;
+    const bool have_lv = dbg_get(dbg, "lane", &lv);
+    // measured on B200: with a small image per env (3 views of 12x12: 1296 B) the step is bound by the
+    // logic's latency and the warp-specialised form (more logic warps per image buffer) is 1.4x faster;
+    // with 2646 B per env (2 views of 21x21) the image stream dominates and the fused form wins
+    // ... unless there are too few 32-env batches to give every SM a few (4 096 envs of 2x10x10: one
+    // batch per SM at most): then a warp that steps AND paints its batch has the shortest critical path
+    // (13.8 us vs 19.0 us per step)
+    // Since the respawns became warp-cooperative function calls the register-capped warp-specialised kernel pays for
+    // them in spills, and for S >= 2 the two-kernel form (logic at full occupancy, then the observation writer) is the
+    // fastest small-image form (65 536 envs, 10x10: 3 snakes cut 53.0 vs 61.3 us, 3 snakes classic 44.0 vs 48.8,
+    // 2 snakes 34.6 vs 38.8; 1 M envs cut 648 vs 751 us); a single snake stays warp-specialised (23.6 vs 29.2 us).
+    const bool small_image = p.E < 2048 && (N + 31) / 32 >= 2LL * h->n_sm;
+    if (grid) form = FORM_LANE_GRID;
+    else if (have_lv ? lv == "ws" : (small_image && S == 1)) form = FORM_LANE_WS;
+    else if (have_lv ? lv == "split" : (small_image && S > 1)) form = FORM_LANE_SPLIT;
+    p.RW = (REC_SNAKE0 + 2 * S + 2 + 3) & ~3;
+    p.W = 32;
+    int te = TE, epw = 32;
+    if (form == FORM_LANE) {
+      // Small shards.  A warp's pass (logic of its batch, then one image after the other) is a serial chain, and a lane
+      // per env keeps 32 envs on it; when the shard has fewer 32-env batches than the GPU holds warps (4 096 envs of
+      // 2x10x10 = 128 warps on 148 SMs: 14 us per step, all of it one warp's latency) the batch shrinks to 16 / 8 / 4 envs
+      // -- the idle lanes cost issue slots nobody wants, the chain gets shorter (one image, painted by 32/epw lanes per
+      // env) -- as long as every batch still finds a resident warp.  epw=<n> overrides.
+      const int forced = dbg_int(dbg, "epw", 0);
+      for (int cand = 16; cand >= 4; cand >>= 1) {
+        if (cand % p.G != 0 || (forced && cand < forced)) break;
+        CUDA_TRY(plan_lane(plan, form, cand < TE ? cand : TE, cand, 32));
+        if (!forced && (N + cand - 1) / cand > (long long)plan.max_grid * 2) break;  // more batches than resident warps (2 per CTA)
+        te = p.TE; epw = cand;
+      }
+    }
+    CUDA_TRY(plan_lane(plan, form, te, epw, form == FORM_LANE_GRID ? 64 : 32));
+  } else {
+    if (form == FORM_TILE) {
+      p.W = W; plan.block = 32 * W; plan.smem = smem_tile;
+    } else if (form == FORM_ROWS) {
+      if (grid) form = FORM_ROWS_GRID;
+      p.W = 1; p.R = R; plan.block = 128;  // 1 producer warp + 3 consumer warps
+      p.tile_stride = (int)(((size_t)R * V * p.C + 127) & ~(size_t)127);  // grid: R = 0, no chunk buffers
+      plan.smem = 2 * (((size_t)p.VV + 127) & ~(size_t)127) + 2 * (size_t)p.tile_stride + (size_t)(p.RW + p.bm_words) * 4;
+    } else {
+      p.W = 1; plan.block = 256; plan.smem = align16((size_t)p.VV) + (size_t)(p.RW + p.bm_words) * 4;
+      if (plan.smem > 200 * 1024) return fail(SNK_EINVAL, "board too large for shared memory");
+    }
+    p.n_groups = (N + p.W - 1) / p.W;
+    plan.form = form;
+    plan.envs_per_cta = p.W;
+    CUDA_TRY(finish(plan));
+  }
+  // Regime-adaptive lane path.  With short bodies the fused kernel wins (2x19x19, 131 072 envs, random actions: 64.5 us
+  // against 73.3 us for the two-kernel form: the logic hides under the observation stream); with long bodies its warps
+  // -- ten per SM, each a serial chain through 78 KB of code, 2.4x the instruction cache -- fall behind and the two
+  // small kernels win.  Measured on one box, mean body cells per env 5.8 / 8.6 / 12.8 / 22.2 (fruit-seeking policy with
+  // 70 / 40 / 20 / 5 % random actions): fused 72.6 / 83.0 / 92.4 / 109.9 us, two kernels 75.9 / 79.8 / 85.6 / 93.4 us.  The host cannot know
+  // the regime without the statistics, so the first CTA of every step posts the running sums into mapped host memory
+  // (peer_push) and regime_update() reads them -- no synchronisation, a step or two late, which is early enough
+  // for a quantity that moves over hundreds of steps.  Results are bit-identical either way.  adaptive=0 turns it off.
+  std::string lv;
+  if (form == FORM_LANE && p.EPW == 32 && !dbg_get(dbg, "lane", &lv) && dbg_int(dbg, "adaptive", 1) != 0) {
+    // the alternative steps the same 32-env batches: p's lane geometry stays as it is
+    h->have_alt = plan_lane(h->plan_alt, FORM_LANE_SPLIT, p.TE, 32, 64) == cudaSuccess;
+    cudaGetLastError();
+    // thresholds in body cells per env, hysteresis between them; measured at 2646 bytes of image per env and scaled
+    // with the image (the larger the image, the longer the stream hides the fused kernel's logic)
+    const int hi = dbg_int(dbg, "alt_hi", 0);
+    h->alt_hi = hi > 0 ? (double)hi : 8.0 * (double)p.E / 2646.0;
+    h->alt_lo = 0.75 * h->alt_hi;
+  }
+  return SNK_OK;
 }
 
 static int cfg_check(const snk_config* c) {
@@ -381,6 +518,7 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   const long long N = cfg->num_envs;
   p.D = D; p.V = V; p.VV = V * V; p.S = S; p.F = F; p.K = K; p.C = grid ? 1 : 3 * K;  // grid: one code byte per cell
   p.cap = h->lay.cap;
+  p.CW = (p.cap - 1 + 15) / 16;
   p.RW = (REC_SNAKE0 + 2 * S + (F + 1) / 2 + 3) & ~3;
   p.E = p.VV * p.C;
   p.G = 16 / gcd(p.E, 16);
@@ -390,155 +528,20 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   p.max_steps = h->cfg.max_steps; p.auto_reset = cfg->auto_reset != 0; p.rng_mode = cfg->rng_mode;
   p.N = N; p.env_id_base = cfg->env_id_base; p.seed = cfg->seed;
 
-  // launch plan.  lane kernel (chain-coded bodies, lane per env) for small boards; otherwise the
-  // warp-per-env tile kernel while W observations + template + scratch leave room for >= 2 CTAs per
-  // SM; otherwise the CTA-per-env rows / dense kernel.
-  LaunchPlan& plan = h->plan;
-  std::string force;
-  dbg_get(dbg, "force_kernel", &force);
-  int TE = 0;
-  if ((grid || snk_lane_supported(S, K)) && S <= 4 && F <= 4 && D <= 32) {  // grid: k_lane_grid exists for every K
-    const int cand[3] = {32, 16, 8};
-    for (int i = 0; i < 3 && !TE; ++i)
-      if (cand[i] % p.G == 0 && (size_t)cand[i] * p.E <= 28 * 1024) TE = cand[i];
-    if (!TE && p.G <= 8 && (size_t)8 * p.E <= 48 * 1024) TE = 8;
-  }
-  const int W = p.G > 8 ? p.G : 8;
-  const size_t smem_tile = (size_t)(W + p.G) * p.E + (size_t)W * (REC_SNAKE0 + 2 * S + (F + 1) / 2 + 3 + p.bm_words) * 4;
-  // rows kernel: chunks of R image rows must be 16-byte multiples (TMA) and fit a ~24 KB buffer
-  int R = 0;
-  if (p.E % 16 == 0 && !grid) {
-    const int unit = 16 / gcd(V * p.C, 16);
-    // chunk size and CTA shape measured on B200 at 16 snakes on 64x64: 4 warps (1 producer + 3 consumers) give 7 CTAs
-    // per SM, and 8 KB chunks beat 12 KB (32 768 envs: classic 1280 us, cut 1502 vs 1551 us)
-    const size_t lim = 8 * 1024;
-    for (int r = unit; r <= V && ((size_t)r * V * p.C <= lim || !R); r += unit) { if ((size_t)r * V * p.C > 48 * 1024) break; R = r; }
-  }
-  plan.kind = TE ? KIND_LANE : smem_tile <= 110 * 1024 ? KIND_TILE : R ? KIND_ROWS : KIND_DENSE;
-  // grid: every ring-family geometry goes to the rows kernel's grid form (the producer's code grid IS the observation)
-  plan.obs_grid = grid;
-  if (grid && plan.kind != KIND_LANE) plan.kind = KIND_ROWS;
-  if (force == "dense") plan.kind = KIND_DENSE;
-  if (force == "rows") {
-    if (!R && !grid) { snk_destroy(h); return fail(SNK_EINVAL, "rows kernel does not support this configuration"); }
-    plan.kind = KIND_ROWS;
-  }
-  if (force == "tile" && smem_tile <= 200 * 1024) plan.kind = KIND_TILE;
-  if (force == "lane" && !TE) { snk_destroy(h); return fail(SNK_EINVAL, "lane kernel does not support this configuration"); }
-  p.family = plan.kind == KIND_LANE;
-  // lane path variants (lane=fused|ws|split): every warp steps 32 envs then streams their images (default: fastest
-  // measured), warp-specialised single kernel, or two kernels
-  {
-    std::string lv;
-    const bool have_lv = dbg_get(dbg, "lane", &lv);
-    // measured on B200: with a small image per env (3 views of 12x12: 1296 B) the step is bound by the
-    // logic's latency and the warp-specialised form (more logic warps per image buffer) is 1.4x faster;
-    // with 2646 B per env (2 views of 21x21) the image stream dominates and the fused form wins
-    // ... unless there are too few 32-env batches to give every SM a few (4 096 envs of 2x10x10: one
-    // batch per SM at most): then a warp that steps AND paints its batch has the shortest critical path
-    // (13.8 us vs 19.0 us per step)
-    // Since the respawns became warp-cooperative function calls the register-capped warp-specialised kernel pays for
-    // them in spills, and for S >= 2 the two-kernel form (logic at full occupancy, then the observation writer) is the
-    // fastest small-image form (65 536 envs, 10x10: 3 snakes cut 53.0 vs 61.3 us, 3 snakes classic 44.0 vs 48.8,
-    // 2 snakes 34.6 vs 38.8; 1 M envs cut 648 vs 751 us); a single snake stays warp-specialised (23.6 vs 29.2 us).
-    const bool small_image = p.E < 2048 && (N + 31) / 32 >= 2LL * h->n_sm;
-    plan.ws = plan.kind == KIND_LANE && !grid && (have_lv ? lv == "ws" : (small_image && S == 1));
-    plan.split = plan.kind == KIND_LANE && (grid || (have_lv ? lv == "split" : (small_image && S > 1)));
-  }
-  p.CW = (p.cap - 1 + 15) / 16;
-  // lane path geometry: te envs per warp image, epw envs stepped per warp batch (a multiple of te)
-  auto lane_geometry = [&](int te, int epw) {
-    p.TE = te; p.EPW = epw;
-    p.tile_stride = (int)(((size_t)te * p.E + 127) & ~(size_t)127);
-    p.restore_thr = dbg_int(dbg, "restore_thr", restore_threshold(p, 32));
-    plan.smem = (size_t)(plan.split ? 1 : 2) * p.tile_stride;
-    p.n_groups = (N + epw - 1) / epw;
-  };
-  if (plan.kind == KIND_LANE) {
-    p.RW = (REC_SNAKE0 + 2 * S + 2 + 3) & ~3;
-    p.W = 32;
-    plan.block = plan.ws ? 32 * (WS_PAINT_WARPS + WS_LOGIC_WARPS) : 64;
-    lane_geometry(TE, 32);
-    if (grid) p.restore_thr = dbg_int(dbg, "restore_thr", restore_threshold(p, 64));  // k_lane_grid: 64 threads per buffer
-  } else if (plan.kind == KIND_TILE) {
-    p.W = W; plan.block = 32 * W; plan.smem = smem_tile;
-    p.n_groups = (N + W - 1) / W;
-  } else if (plan.kind == KIND_ROWS) {
-    p.W = 1; p.R = R; plan.block = 128;  // 1 producer warp + 3 consumer warps
-    p.tile_stride = (int)(((size_t)R * V * p.C + 127) & ~(size_t)127);  // grid: R = 0, no chunk buffers
-    plan.smem = 2 * (((size_t)p.VV + 127) & ~(size_t)127) + 2 * (size_t)p.tile_stride + (size_t)(p.RW + p.bm_words) * 4;
-    p.n_groups = N;
-  } else {
-    p.W = 1; plan.block = 256; plan.smem = align16((size_t)p.VV) + (size_t)(p.RW + p.bm_words) * 4;
-    p.n_groups = N;
-    if (plan.smem > 200 * 1024) { snk_destroy(h); return fail(SNK_EINVAL, "board too large for shared memory"); }
-  }
-  CUDA_TRY_H(snk_plan(cfg->rules, plan, h->n_sm, S, K));
-  if (plan.kind == KIND_LANE && !plan.ws && !plan.split) {
-    // Small shards.  A warp's pass (logic of its batch, then one image after the other) is a serial chain, and a lane
-    // per env keeps 32 envs on it; when the shard has fewer 32-env batches than the GPU holds warps (4 096 envs of
-    // 2x10x10 = 128 warps on 148 SMs: 14 us per step, all of it one warp's latency) the batch shrinks to 16 / 8 / 4 envs
-    // -- the idle lanes cost issue slots nobody wants, the chain gets shorter (one image, painted by 32/epw lanes per
-    // env) -- as long as every batch still finds a resident warp.  epw=<n> overrides.
-    const int forced = dbg_int(dbg, "epw", 0);
-    int te = TE, epw = 32;
-    for (int cand = 16; cand >= 4; cand >>= 1) {
-      if (cand % p.G != 0 || (forced && cand < forced)) break;
-      lane_geometry(cand < TE ? cand : TE, cand);
-      CUDA_TRY_H(snk_plan(cfg->rules, plan, h->n_sm, S, K));
-      if (!forced && (N + cand - 1) / cand > (long long)plan.max_grid * 2) break;  // more batches than resident warps (2 per CTA)
-      te = p.TE; epw = cand;
+  TRY(plan_launch(h));
+  if (h->have_alt) {  // regime_update() reads the running sums the step kernels post here (Params::regime_out)
+    h->have_alt = false;
+    void* hp = nullptr;
+    if (cudaHostAlloc(&hp, 2 * sizeof(double), cudaHostAllocMapped) == cudaSuccess) {
+      void* dp = nullptr;
+      if (cudaHostGetDevicePointer(&dp, hp, 0) == cudaSuccess) {
+        h->h_regime = (double*)hp; h->h_regime[0] = h->h_regime[1] = 0.0;
+        h->host_allocs.push_back(std::make_pair(hp, 2 * sizeof(double)));
+        p.regime_out = (double*)dp;
+        h->have_alt = true;
+      } else cudaFreeHost(hp);
     }
-    lane_geometry(te, epw);
-    CUDA_TRY_H(snk_plan(cfg->rules, plan, h->n_sm, S, K));
-  }
-  {
-    long long work = plan.kind == KIND_LANE ? (p.n_groups + 1) / 2 : p.n_groups;  // lane: 2 warps per CTA
-    if (plan.split) work = (N + p.TE - 1) / p.TE;  // k_lane_paint2: one image per CTA
-    if (plan.ws) work = (p.n_groups + WS_LOGIC_WARPS - 1) / WS_LOGIC_WARPS;
-    plan.grid = (int)(work < plan.max_grid ? work : plan.max_grid);
-    if (plan.grid < 1) plan.grid = 1;
-  }
-  // Regime-adaptive lane path.  With short bodies the fused kernel wins (2x19x19, 131 072 envs, random actions: 64.5 us
-  // against 73.3 us for the two-kernel form: the logic hides under the observation stream); with long bodies its warps
-  // -- ten per SM, each a serial chain through 78 KB of code, 2.4x the instruction cache -- fall behind and the two
-  // small kernels win.  Measured on one box, mean body cells per env 5.8 / 8.6 / 12.8 / 22.2 (fruit-seeking policy with
-  // 70 / 40 / 20 / 5 % random actions): fused 72.6 / 83.0 / 92.4 / 109.9 us, two kernels 75.9 / 79.8 / 85.6 / 93.4 us.  The host cannot know
-  // the regime without the statistics, so the first CTA of every step posts the running sums into mapped host memory
-  // (peer_push) and regime_update() below reads them -- no synchronisation, a step or two late, which is early enough
-  // for a quantity that moves over hundreds of steps.  Results are bit-identical either way.  adaptive=0 turns it off.
-  {
-    std::string lv;
-    const bool eligible = plan.kind == KIND_LANE && !plan.ws && !plan.split && p.EPW == 32 && !dbg_get(dbg, "lane", &lv) &&
-                          dbg_int(dbg, "adaptive", 1) != 0;
-    if (eligible) {
-      h->plan_alt = plan;
-      LaunchPlan& alt = h->plan_alt;
-      alt.split = true; alt.block = 64;
-      alt.smem = (size_t)p.tile_stride;
-      if (snk_plan(cfg->rules, alt, h->n_sm, S, K) == cudaSuccess) {
-        const long long work = (N + p.TE - 1) / p.TE;
-        alt.grid = (int)(work < alt.max_grid ? work : alt.max_grid);
-        if (alt.grid < 1) alt.grid = 1;
-        h->restore_thr_alt = dbg_int(dbg, "restore_thr", restore_threshold(p, 64));
-        // thresholds in body cells per env, hysteresis between them; measured at 2646 bytes of image per env and scaled
-        // with the image (the larger the image, the longer the stream hides the fused kernel's logic)
-        const int hi = dbg_int(dbg, "alt_hi", 0);
-        h->alt_hi = hi > 0 ? (double)hi : 8.0 * (double)p.E / 2646.0;
-        h->alt_lo = 0.75 * h->alt_hi;
-        void* hp = nullptr;
-        if (cudaHostAlloc(&hp, 2 * sizeof(double), cudaHostAllocMapped) == cudaSuccess) {
-          void* dp = nullptr;
-          if (cudaHostGetDevicePointer(&dp, hp, 0) == cudaSuccess) {
-            h->h_regime = (double*)hp; h->h_regime[0] = h->h_regime[1] = 0.0;
-            h->host_allocs.push_back(std::make_pair(hp, 2 * sizeof(double)));
-            p.regime_out = (double*)dp;
-            h->have_alt = true;
-          } else cudaFreeHost(hp);
-        }
-        cudaGetLastError();
-      }
-    }
+    cudaGetLastError();
   }
 
   // device buffers
@@ -718,10 +721,10 @@ static int launch(snk_handle* h, int mode, const int8_t* d_actions, const uint8_
   if (mode == MODE_STEP) regime_update(h);
   const bool alt = h->have_alt && h->use_alt;
   const LaunchPlan& plan = alt ? h->plan_alt : h->plan;
-  if (alt) p.restore_thr = h->restore_thr_alt;
-  CUDA_TRY(snk_launch_step(p, h->cfg.rules, plan, stream));
+  p.restore_thr = plan.restore_thr;
+  CUDA_TRY(snk_launch_step(p, plan, stream));
   if (!capturing) h->obs_current = p.obs;
-  h->launches += (plan.split && mode != MODE_OBSERVE) ? 2 : 1;
+  h->launches += (plan.logic && mode != MODE_OBSERVE) ? 2 : 1;
   if (reduce) {
     // side stream: all-reduce this step's snapshot while the next step runs; its result is read one step late
     cudaEvent_t es = capturing ? h->cev_step[0] : h->ev_step[sl], er = capturing ? h->cev_red[0] : h->ev_red[sl];
@@ -1616,18 +1619,22 @@ extern "C" int snk_launch_count(const snk_handle* h, uint64_t* out) {
   return SNK_OK;
 }
 
+// include/snk.h's numbers for each form: snk_launch_info's kind (0 lane, 1 tile, 2 dense, 3 rows) and snk_launch_form's
+// code (0 fused, 1 warp-specialised, 3 two kernels, -1 not the lane family)
+static const struct { int32_t kind, code; } kFormCodes[FORM_COUNT] = {
+    {0, 0}, {0, 1}, {0, 3}, {0, 3}, {1, -1}, {2, -1}, {3, -1}, {3, -1}};
+
 extern "C" int snk_launch_form(const snk_handle* h, int32_t* out /*[4]*/) {
   if (!h || !out) return fail(SNK_EINVAL, "NULL argument");
   const LaunchPlan& pl = (h->have_alt && h->use_alt) ? h->plan_alt : h->plan;
-  out[0] = pl.kind != KIND_LANE ? -1 : pl.ws ? 1 : pl.split ? 3 : 0;
-  out[1] = pl.kind == KIND_LANE ? h->p.EPW : 0; out[2] = pl.kind == KIND_LANE ? h->p.TE : 0; out[3] = h->have_alt ? 1 : 0;
+  out[0] = kFormCodes[pl.form].code;
+  out[1] = h->p.family ? h->p.EPW : 0; out[2] = h->p.family ? h->p.TE : 0; out[3] = h->have_alt ? 1 : 0;
   return SNK_OK;
 }
 
 extern "C" int snk_launch_info(const snk_handle* h, int32_t* out /*[6]: kind, grid, block, smem, occupancy, envs per CTA*/) {
   if (!h || !out) return fail(SNK_EINVAL, "NULL argument");
   const LaunchPlan& pl = (h->have_alt && h->use_alt) ? h->plan_alt : h->plan;
-  out[0] = pl.kind; out[1] = pl.grid; out[2] = pl.block; out[3] = (int32_t)pl.smem;
-  out[4] = pl.occupancy; out[5] = pl.kind == KIND_LANE ? (pl.split ? h->p.TE : pl.ws ? 32 * WS_LOGIC_WARPS : 2 * h->p.EPW) : h->p.W;
+  out[0] = kFormCodes[pl.form].kind; out[1] = pl.grid; out[2] = pl.block; out[3] = (int32_t)pl.smem; out[4] = pl.occupancy; out[5] = pl.envs_per_cta;
   return SNK_OK;
 }

@@ -1664,158 +1664,95 @@ bool snk_lane_supported(int S, int K) {
 // SNK_OBS_GRID, lane family: k_lane_logic + k_lane_grid, instantiated per snake count (the views do not enter)
 #define GRID_SNAKES(X) X(1) X(2) X(3) X(4)
 
+// plan.logic and plan.kernel of plan.form for S snakes and K views under RULES
 template <int RULES>
-cudaError_t launch_rules(const Params& p, const LaunchPlan& plan, cudaStream_t stream) {
-  if (plan.kind == KIND_LANE && plan.obs_grid) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(plan.grid); cfg.blockDim = dim3(plan.block); cfg.dynamicSmemBytes = plan.smem; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    cudaLaunchConfig_t lc = cfg;
-    lc.gridDim = dim3((unsigned)((p.N + 127) / 128)); lc.blockDim = dim3(128); lc.dynamicSmemBytes = 0;
-#define X(s)                                                                            \
-  if (p.S == s) {                                                                       \
-    if (p.mode != MODE_OBSERVE) {                                                       \
-      cudaError_t e1 = cudaLaunchKernelEx(&lc, k_lane_logic<s, RULES>, p);              \
-      if (e1 != cudaSuccess) return e1;                                                 \
-    }                                                                                   \
-    return cudaLaunchKernelEx(&cfg, k_lane_grid<s, RULES>, p);                          \
+cudaError_t resolve(LaunchPlan& plan, int S, int K) {
+  const void* logic = nullptr;
+  const void* kernel = nullptr;
+  switch (plan.form) {
+    case FORM_LANE:
+    case FORM_LANE_WS:
+    case FORM_LANE_SPLIT:
+#define X(s, k)                                                                  \
+  if (S == s && K == k) {                                                        \
+    if (plan.form == FORM_LANE) {                                                \
+      kernel = (const void*)k_step_lane<s, RULES, k>;                            \
+    } else if (plan.form == FORM_LANE_WS) {                                      \
+      kernel = (const void*)k_step_lane_ws<s, RULES, k>;                         \
+    } else {                                                                     \
+      logic = (const void*)k_lane_logic<s, RULES>;                               \
+      kernel = (const void*)k_lane_paint2<s, RULES, k>;                          \
+    }                                                                            \
   }
-    GRID_SNAKES(X)
+      LANE_COMBOS(X)
 #undef X
-    return cudaErrorInvalidConfiguration;
+      break;
+    case FORM_LANE_GRID:
+#define X(s)                                     \
+  if (S == s) {                                  \
+    logic = (const void*)k_lane_logic<s, RULES>; \
+    kernel = (const void*)k_lane_grid<s, RULES>; \
   }
-  if (plan.kind == KIND_LANE) {
-#define X(s, k)                                                                                              \
-  if (p.S == s && p.K == k) {                                                                                \
-    if (plan.ws) {                                                                                           \
-      k_step_lane_ws<s, RULES, k><<<plan.grid, plan.block, plan.smem, stream>>>(p);                          \
-      return cudaGetLastError();                                                                             \
-    }                                                                                                        \
-    /* programmatic launches: a kernel's prologue overlaps the tail of the launch before it */               \
-    cudaLaunchConfig_t cfg = {};                                                                             \
-    cfg.gridDim = dim3(plan.grid); cfg.blockDim = dim3(plan.block); cfg.dynamicSmemBytes = plan.smem;        \
-    cfg.stream = stream;                                                                                     \
-    cudaLaunchAttribute attr[1];                                                                             \
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;                                         \
-    attr[0].val.programmaticStreamSerializationAllowed = 1;                                                  \
-    cfg.attrs = attr; cfg.numAttrs = 1;                                                                      \
-    if (!plan.split) return cudaLaunchKernelEx(&cfg, k_step_lane<s, RULES, k>, p);                           \
-    if (p.mode != MODE_OBSERVE) {                                                                            \
-      cudaLaunchConfig_t lc = cfg;                                                                           \
-      lc.gridDim = dim3((unsigned)((p.N + 127) / 128)); lc.blockDim = dim3(128); lc.dynamicSmemBytes = 0;    \
-      cudaError_t e1 = cudaLaunchKernelEx(&lc, k_lane_logic<s, RULES>, p);                                   \
-      if (e1 != cudaSuccess) return e1;                                                                      \
-    }                                                                                                        \
-    return cudaLaunchKernelEx(&cfg, k_lane_paint2<s, RULES, k>, p);                                          \
-  }
-    LANE_COMBOS(X)
+      GRID_SNAKES(X)
 #undef X
-    return cudaErrorInvalidConfiguration;
+      break;
+    case FORM_TILE: kernel = plan.block <= 256 ? (const void*)k_step_tile<RULES, 256> : (const void*)k_step_tile<RULES, 512>; break;
+    case FORM_DENSE: kernel = (const void*)k_step_dense<RULES>; break;
+    case FORM_ROWS: kernel = (const void*)k_step_rows<RULES, false>; break;
+    case FORM_ROWS_GRID: kernel = (const void*)k_step_rows<RULES, true>; break;
   }
-  if (plan.kind == KIND_ROWS) {
-    if (plan.obs_grid) k_step_rows<RULES, true><<<plan.grid, plan.block, plan.smem, stream>>>(p);
-    else k_step_rows<RULES, false><<<plan.grid, plan.block, plan.smem, stream>>>(p);
-    return cudaGetLastError();
-  }
-  if (plan.kind == KIND_TILE) {
-    if (plan.block <= 256) k_step_tile<RULES, 256><<<plan.grid, plan.block, plan.smem, stream>>>(p);
-    else k_step_tile<RULES, 512><<<plan.grid, plan.block, plan.smem, stream>>>(p);
-  } else {
-    k_step_dense<RULES><<<plan.grid, plan.block, plan.smem, stream>>>(p);
-  }
-  return cudaGetLastError();
+  plan.logic = logic;
+  plan.kernel = kernel;
+  return kernel ? cudaSuccess : cudaErrorInvalidConfiguration;
 }
 
 #if SNK_TU >= 0 && SNK_TU <= 2
-template cudaError_t launch_rules<SNK_TU>(const Params&, const LaunchPlan&, cudaStream_t);
+template cudaError_t resolve<SNK_TU>(LaunchPlan&, int, int);
 #elif SNK_TU == 3
-extern template cudaError_t launch_rules<SNK_RULES_CLASSIC>(const Params&, const LaunchPlan&, cudaStream_t);
-extern template cudaError_t launch_rules<SNK_RULES_ADVERSARIAL>(const Params&, const LaunchPlan&, cudaStream_t);
-extern template cudaError_t launch_rules<SNK_RULES_CUT>(const Params&, const LaunchPlan&, cudaStream_t);
+extern template cudaError_t resolve<SNK_RULES_CLASSIC>(LaunchPlan&, int, int);
+extern template cudaError_t resolve<SNK_RULES_ADVERSARIAL>(LaunchPlan&, int, int);
+extern template cudaError_t resolve<SNK_RULES_CUT>(LaunchPlan&, int, int);
 #endif
 #if SNK_TU == -1 || SNK_TU == 3
-cudaError_t snk_launch_step(const Params& p, int rules, const LaunchPlan& plan, cudaStream_t stream) {
-  switch (rules) {
-    case SNK_RULES_CLASSIC: return launch_rules<SNK_RULES_CLASSIC>(p, plan, stream);
-    case SNK_RULES_ADVERSARIAL: return launch_rules<SNK_RULES_ADVERSARIAL>(p, plan, stream);
-    default: return launch_rules<SNK_RULES_CUT>(p, plan, stream);
-  }
-}
-
-#endif
-
-template <int S, int RULES, int K>
-static cudaError_t plan_lane(LaunchPlan& plan, int& occ) {
-  cudaError_t err;
-  if (plan.ws) {
-    if ((err = cudaFuncSetAttribute(k_step_lane_ws<S, RULES, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_lane_ws<S, RULES, K>, plan.block, plan.smem);
-  }
-  if (plan.split) {
-    if ((err = cudaFuncSetAttribute(k_lane_paint2<S, RULES, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_lane_paint2<S, RULES, K>, plan.block, plan.smem);
-  }
-  if ((err = cudaFuncSetAttribute(k_step_lane<S, RULES, K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
-  return cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_lane<S, RULES, K>, plan.block, plan.smem);
-}
-
-template <int RULES>
-cudaError_t plan_rules(LaunchPlan& plan, int n_sm, int S, int K) {
-  cudaError_t err = cudaErrorInvalidConfiguration;
+cudaError_t snk_plan(int rules, LaunchPlan& plan, int n_sm, int S, int K, long long work) {
+  cudaError_t err = rules == SNK_RULES_CLASSIC       ? resolve<SNK_RULES_CLASSIC>(plan, S, K)
+                    : rules == SNK_RULES_ADVERSARIAL ? resolve<SNK_RULES_ADVERSARIAL>(plan, S, K)
+                                                     : resolve<SNK_RULES_CUT>(plan, S, K);
+  if (err) return err;
+  // programmatic launches for the fused kernel and both kernels of the two-kernel forms; the warp-specialised, tile,
+  // dense and rows kernels launch without
+  plan.pdl = plan.form == FORM_LANE || plan.form == FORM_LANE_SPLIT || plan.form == FORM_LANE_GRID;
   int occ = 0;
-  if (plan.kind == KIND_LANE && plan.obs_grid) {
-#define X(s)                                                                                                                  \
-  if (S == s) {                                                                                                               \
-    if ((err = cudaFuncSetAttribute(k_lane_grid<s, RULES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err; \
-    err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_lane_grid<s, RULES>, plan.block, plan.smem);                  \
-  }
-    GRID_SNAKES(X)
-#undef X
-    if (err) return err;
-  } else if (plan.kind == KIND_LANE) {
-#define X(s, k) if (S == s && K == k) err = plan_lane<s, RULES, k>(plan, occ);
-    LANE_COMBOS(X)
-#undef X
-    if (err) return err;
-  } else if (plan.kind == KIND_ROWS && plan.obs_grid) {
-    if ((err = cudaFuncSetAttribute(k_step_rows<RULES, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
-    if ((err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_rows<RULES, true>, plan.block, plan.smem))) return err;
-  } else if (plan.kind == KIND_ROWS) {
-    if ((err = cudaFuncSetAttribute(k_step_rows<RULES, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
-    if ((err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_rows<RULES, false>, plan.block, plan.smem))) return err;
-  } else if (plan.kind == KIND_TILE && plan.block <= 256) {
-    if ((err = cudaFuncSetAttribute(k_step_tile<RULES, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
-    if ((err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_tile<RULES, 256>, plan.block, plan.smem))) return err;
-  } else if (plan.kind == KIND_TILE) {
-    if ((err = cudaFuncSetAttribute(k_step_tile<RULES, 512>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
-    if ((err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_tile<RULES, 512>, plan.block, plan.smem))) return err;
-  } else {
-    if ((err = cudaFuncSetAttribute(k_step_dense<RULES>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
-    if ((err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_step_dense<RULES>, plan.block, plan.smem))) return err;
-  }
+  if ((err = cudaFuncSetAttribute(plan.kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)plan.smem))) return err;
+  if ((err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, plan.kernel, plan.block, plan.smem))) return err;
   if (occ < 1) return cudaErrorInvalidConfiguration;
   plan.occupancy = occ;
   plan.max_grid = n_sm * occ;
+  plan.grid = (int)(work < plan.max_grid ? work : plan.max_grid);
+  if (plan.grid < 1) plan.grid = 1;
   return cudaSuccess;
 }
 
-#if SNK_TU >= 0 && SNK_TU <= 2
-template cudaError_t plan_rules<SNK_TU>(LaunchPlan&, int, int, int);
-#elif SNK_TU == 3
-extern template cudaError_t plan_rules<SNK_RULES_CLASSIC>(LaunchPlan&, int, int, int);
-extern template cudaError_t plan_rules<SNK_RULES_ADVERSARIAL>(LaunchPlan&, int, int, int);
-extern template cudaError_t plan_rules<SNK_RULES_CUT>(LaunchPlan&, int, int, int);
-#endif
-#if SNK_TU == -1 || SNK_TU == 3
-cudaError_t snk_plan(int rules, LaunchPlan& plan, int n_sm, int S, int K) {
-  switch (rules) {
-    case SNK_RULES_CLASSIC: return plan_rules<SNK_RULES_CLASSIC>(plan, n_sm, S, K);
-    case SNK_RULES_ADVERSARIAL: return plan_rules<SNK_RULES_ADVERSARIAL>(plan, n_sm, S, K);
-    default: return plan_rules<SNK_RULES_CUT>(plan, n_sm, S, K);
+cudaError_t snk_launch_step(const Params& p, const LaunchPlan& plan, cudaStream_t stream) {
+  // programmatic launches: a kernel's prologue overlaps the tail of the launch before it
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.stream = stream;
+  cfg.attrs = attr;
+  cfg.numAttrs = plan.pdl ? 1 : 0;
+  void* args[] = {const_cast<Params*>(&p)};
+  if (plan.logic && p.mode != MODE_OBSERVE) {  // thread per env
+    cfg.gridDim = dim3((unsigned)((p.N + 127) / 128));
+    cfg.blockDim = dim3(128);
+    cudaError_t err = cudaLaunchKernelExC(&cfg, plan.logic, args);
+    if (err != cudaSuccess) return err;
   }
+  cfg.gridDim = dim3(plan.grid);
+  cfg.blockDim = dim3(plan.block);
+  cfg.dynamicSmemBytes = plan.smem;
+  return cudaLaunchKernelExC(&cfg, plan.kernel, args);
 }
 
 cudaError_t snk_launch_upscale84(const uint8_t* native, uint8_t* out, long long N, int V, int C, int n_sm, cudaStream_t stream) {

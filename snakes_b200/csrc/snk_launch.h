@@ -7,24 +7,41 @@
 
 struct Params;
 struct PeerArgs;
-enum { KIND_LANE = 0, KIND_TILE = 1, KIND_DENSE = 2, KIND_ROWS = 3 };
 // k_step_lane_ws: paint warps (each owning a shared-memory image) and logic warps per CTA
 enum { WS_PAINT_WARPS = 2, WS_LOGIC_WARPS = 3 };
 
-struct LaunchPlan {
-  int kind;         // KIND_LANE (lane per env, chain bodies), KIND_TILE (warp per env), KIND_ROWS / KIND_DENSE (CTA per env)
-  bool ws;          // lane path as ONE warp-specialised kernel (k_step_lane_ws): paint warps + logic warps per CTA
-  bool split;       // lane path as two kernels: k_lane_logic (thread per env) + k_lane_paint2 (observation writer)
-  bool obs_grid;    // SNK_OBS_GRID: k_lane_logic + k_lane_grid (lane, always split) or k_step_rows<RULES, true> (rows)
-  int grid, block;
-  size_t smem;
-  int occupancy;    // resident CTAs per SM
-  int max_grid;     // SMs * occupancy: persistent grid size
+// The kernel sequences a step runs.  snk_api.cu's plan_launch picks one; resolve<RULES> in snk_kernels.cu is the only code
+// that names their kernels.  The lane family keeps bodies chain-coded with a lane per env; the others keep ring bodies.
+enum Form {
+  FORM_LANE,        // k_step_lane: a warp steps its batch, then streams its images
+  FORM_LANE_WS,     // k_step_lane_ws: paint warps + logic warps per CTA
+  FORM_LANE_SPLIT,  // k_lane_logic (thread per env) + k_lane_paint2 (observation writer)
+  FORM_LANE_GRID,   // SNK_OBS_GRID: k_lane_logic + k_lane_grid
+  FORM_TILE,        // k_step_tile, warp per env, instantiated for 256 and 512 threads (chosen by the block)
+  FORM_DENSE,       // k_step_dense, CTA per env
+  FORM_ROWS,        // k_step_rows<RULES, false>, CTA per env
+  FORM_ROWS_GRID,   // SNK_OBS_GRID: k_step_rows<RULES, true>
+  FORM_COUNT
 };
 
-cudaError_t snk_plan(int rules, LaunchPlan& plan, int n_sm, int S, int K);
+struct LaunchPlan {
+  int form;
+  const void* logic;   // k_lane_logic<S, RULES>, launched before `kernel` except in MODE_OBSERVE; NULL for one-kernel forms
+  const void* kernel;  // the step kernel, or the observation writer behind `logic`
+  bool pdl;            // programmatic stream serialization for `logic` and `kernel`
+  int grid, block;
+  size_t smem;
+  int occupancy;       // resident CTAs per SM
+  int max_grid;        // SMs * occupancy: persistent grid size
+  int envs_per_cta;
+  int restore_thr;     // Params::restore_thr under this plan
+};
+
+// Resolves plan.form (and plan.block) to its kernels, sets their shared-memory limit, and fills pdl, occupancy, max_grid
+// and grid = work clamped to [1, max_grid].  cudaErrorInvalidConfiguration: no kernel for this form, S and K.
+cudaError_t snk_plan(int rules, LaunchPlan& plan, int n_sm, int S, int K, long long work);
 bool snk_lane_supported(int S, int K);
-cudaError_t snk_launch_step(const Params& p, int rules, const LaunchPlan& plan, cudaStream_t stream);
+cudaError_t snk_launch_step(const Params& p, const LaunchPlan& plan, cudaStream_t stream);
 cudaError_t snk_launch_upscale84(const uint8_t* native, uint8_t* out, long long N, int V, int C, int n_sm, cudaStream_t stream);
 // env state (k_save_envs / k_restore_envs / k_copy_envs): entry j is env idx[j], or env first + j when idx is NULL
 cudaError_t snk_launch_save(const Params& p, const int64_t* idx, long long first, long long count, uint8_t* blob,

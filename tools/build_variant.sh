@@ -1,22 +1,16 @@
 #!/bin/bash
 # build_variant.sh NAME [GIT_REV] [extra nvcc flags]: compile the CUDA library of the working tree (GIT_REV = "-") or of a
 # commit into variants/libsnk_NAME.so for A/B timing on one box (SNK_LIB=variants/libsnk_NAME.so python tools/ab.py ...).
+# Either way the working tree's __graft_entry__.build_library compiles it.
 set -e
 cd "$(dirname "$0")/.."
 name=$1; rev=${2:--}; shift; shift || true
 src=$PWD
 if [ "$rev" != "-" ]; then
   src=$(mktemp -d /tmp/snk_variant_XXXX)
+  trap 'rm -rf "$src"' EXIT
   git archive "$rev" snakes_b200/csrc include | tar -x -C "$src"
 fi
-mkdir -p variants/_o_$name
-F="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC $*"
-C=$src/snakes_b200/csrc
-nvcc $F -c -o variants/_o_$name/api.o $C/snk_api.cu &
-for tu in 0 1 2 3; do nvcc $F -DSNK_TU=$tu -c -o variants/_o_$name/k$tu.o $C/snk_kernels.cu & done
-wait
-for o in api k0 k1 k2 k3; do [ -f variants/_o_$name/$o.o ] || { echo "FAILED: $o did not compile"; rm -rf variants/_o_$name; exit 1; }; done
-nvcc --shared -gencode arch=compute_100a,code=sm_100a -o variants/libsnk_$name.so variants/_o_$name/*.o
-rm -rf variants/_o_$name
-[ "$rev" != "-" ] && rm -rf "$src"
+mkdir -p variants
+python3 -c 'import sys, __graft_entry__ as g; g.build_library(sys.argv[1], sys.argv[2], sys.argv[3:])' "$src" "variants/libsnk_$name.so" "$@"
 echo built variants/libsnk_$name.so
