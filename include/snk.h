@@ -450,7 +450,13 @@ int snk_gen_actions(snk_handle* h, int8_t* d_actions, uint64_t step, uint64_t se
 /* Scripted policy for benchmarks (SURVEY.md section 8d second stream): every live snake turns toward
  * its nearest fruit unless the next cell is a wall or a body cell, else keeps going; with probability
  * eps_permille / 1000 a uniform random action instead (Philox stream 2).  Keeps snakes long (larger
- * SigmaL, fewer resets).  Lane-family configurations with classic fruit lists only. */
+ * SigmaL, fewer resets).  Lane-family configurations with classic fruit lists only; eps_permille outside 0..1000 is
+ * SNK_EINVAL.  Exactly, per env e and snake s: a dead snake gets 0.  The draw rnd is the Philox value of key (seed, global
+ * env id), stream 2, counter step * S + s (as for snk_gen_actions) bounded to [0, 5000); rnd / 5 < eps_permille gives
+ * action rnd % 5.  Otherwise action a = 1..4 is a candidate unless it reverses the velocity, its cell is on the border,
+ * or a segment of any snake (tails included) lies there; its distance is the least Manhattan distance from that cell to
+ * the first F fruits (with F = 0 all distances are equal).  The lowest a of strictly smallest distance wins; with no
+ * candidate left the action is 0, which keeps the snake going in its current direction. */
 int snk_gen_scripted_actions(snk_handle* h, int8_t* d_actions, uint64_t step, uint64_t seed,
                              int32_t eps_permille, void* stream);
 

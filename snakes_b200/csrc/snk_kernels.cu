@@ -1154,6 +1154,8 @@ static cudaError_t launch_upscale(const uint8_t* native, uint8_t* out, long long
 // outside the board exactly when the green byte of its pixel in view 0 is non-zero (snake_rgb / the white border; fruit
 // and empty cells have G = 0), so six byte loads replace the walk of both bodies -- which, one env per lane, cost every
 // warp its longest pair of snakes: 31 us per 131 072 envs under this policy, a third of the step it feeds.
+// The contract (draw, candidates, distances, tie-break) is stated at snk_gen_scripted_actions in include/snk.h;
+// tests/scripted_ref.py restates it in numpy and tests/test_gpu_scripted.py holds this kernel to it.
 template <int S>
 __global__ void __launch_bounds__(128) k_scripted_actions(const Params p, int8_t* actions, u64 step, u64 seed, int eps_permille,
                                                           const u8* __restrict__ occ_obs) {
