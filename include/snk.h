@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define SNK_VERSION 340 /* 0.3.4 */
+#define SNK_VERSION 350 /* 0.3.5 */
 
 /* error codes */
 #define SNK_OK 0
@@ -403,6 +403,16 @@ int snk_restore_envs(snk_handle* h, const int64_t* d_idx, int64_t count, const v
  * about 1/12 of the bytes of a save + restore through a blob at 2 snakes on 19x19.  d_src may repeat (1 -> many); d_dst
  * must be distinct and disjoint from d_src. */
 int snk_copy_envs(snk_handle* h, const int64_t* d_src, const int64_t* d_dst, int64_t count, void* stream);
+/* snk_copy_envs across handles: env d_dst[j] of `dst` <- env d_src[j] of `src`, private layout to private layout, one
+ * kernel.  `src` is only read.  Everything else is as for snk_copy_envs: d_src may repeat, d_dst must be distinct (and,
+ * when src == dst, disjoint from d_src); the RNG key stays (seed, global id) of the destination; the destination's
+ * observations are not re-encoded.  An index outside [0, N) of its own handle raises SNK_DEVERR_BAD_STATE on `dst` and
+ * that entry is skipped.  Rejected (SNK_EINVAL naming the field, before any CUDA call): a NULL argument, count < 1,
+ * handles on different devices, of another size, n_snakes, n_fruits or rules, or of another private layout (body family,
+ * record words, chain words, ring capacity, fruit grid stride or bitmap words).  The family follows the launch plan, which
+ * follows the observation size, so two handles of one configuration in different obs_modes may be rejected: states are
+ * not converted between layouts (save_envs / restore_envs do that through the canonical blob). */
+int snk_clone_envs(const snk_handle* src, const int64_t* d_src, snk_handle* dst, const int64_t* d_dst, int64_t count, void* stream);
 
 /* Episode statistics (Monitor's aggregate role).  snk_get_stats synchronises `stream`. */
 int snk_get_stats(snk_handle* h, double* h_stats /*[SNK_NSTATS]*/, void* stream);
@@ -494,6 +504,28 @@ int snk_gen_scripted_actions(snk_handle* h, int8_t* d_actions, uint64_t step, ui
 int snk_tally_layout(const snk_handle* h, size_t* out /*[2]*/);
 int snk_tally(snk_handle* h, const int32_t* d_group, int32_t n_groups, int32_t episodes_per_env, void* d_work,
               int64_t* d_counts, int64_t* d_envs_done, void* stream);
+
+/* Rollout search (DESIGN.md section 4.19): the bookkeeping of a search handle whose slots are clones of roots.  With
+ * A = n_actions and R = rollouts, slot j < n_roots * A * R belongs to root m = j / (A R) and candidate action
+ * a = (j / R) % A.  Slots at and beyond n_roots * A * R are never read or written.  The caller keeps d_ret (int32 [slots],
+ * 4-byte aligned) and d_active (uint8 [slots]) between the calls; each is one kernel, stream-ordered, without allocation
+ * or synchronisation.
+ *   snk_search_begin, before the search's first snk_step: seat `seat`'s action of slot j in d_actions (int8 [N][S], the
+ *     step's action array) <- a; d_ret[j] <- 0; d_active[j] <- 1.
+ *   snk_search_accumulate, after every snk_step: an active slot adds the handle's d_reward_all[j][seat] (an integer) to
+ *     d_ret[j].  The step where that reward is -1 (the seat died, the death rule of snk_tally) or where d_done[j] is set
+ *     is the slot's last counted step: d_active[j] <- 0 after it.
+ *   snk_search_pick: V[m][a] = sum of d_ret over the R slots of (m, a), written as float to d_value [n_roots][A]; the
+ *     lowest a of maximal V[m][a] is written to d_pick[m * pick_stride] (int8; pick_stride = S puts it straight into a
+ *     column of an [N][S] action array).  Every sum is of integers, so the result is the same bits in any order.
+ * Rejected (SNK_EINVAL, before any CUDA call): a NULL handle or array, seat outside [0, S), n_actions outside 1..127,
+ * rollouts < 1, n_roots < 1 or n_roots * A * R > N, pick_stride < 1, d_ret or d_value not 4-byte aligned. */
+int snk_search_begin(snk_handle* h, int8_t* d_actions, int32_t seat, int32_t n_actions, int32_t rollouts, int64_t n_roots,
+                     int32_t* d_ret, uint8_t* d_active, void* stream);
+int snk_search_accumulate(snk_handle* h, int32_t seat, int32_t n_actions, int32_t rollouts, int64_t n_roots, int32_t* d_ret,
+                          uint8_t* d_active, void* stream);
+int snk_search_pick(snk_handle* h, int32_t n_actions, int32_t rollouts, int64_t n_roots, const int32_t* d_ret, float* d_value,
+                    int8_t* d_pick, int64_t pick_stride, void* stream);
 
 /* Algorithmic bytes of one env-step (SURVEY.md section 8d): obs K*H*W*3 + state 19S + 2*SigmaL + 2F + 30. */
 int snk_algorithmic_bytes_per_step(const snk_config* cfg, double mean_sum_len, double* out);

@@ -12,7 +12,8 @@ from .vec_env import EnvStates, Infos, MonitorCSV, SnakeVecEnv, StepGraph, expan
 from .grid_conv import grid_conv84_in, grid_conv_in  # noqa: E402,F401
 from .sharding import all_reduce_stats, make_sharded_env, shard_range  # noqa: E402,F401
 from .rollout import gae  # noqa: E402,F401
-from . import arena  # noqa: E402,F401
+from . import arena, search  # noqa: E402,F401
+from .search import RolloutSearch  # noqa: E402,F401
 from .registration import ENV_IDS, SnakeGymEnv, make, make_basic_env, register  # noqa: E402,F401
 
-__version__ = "0.3.4"
+__version__ = "0.3.5"

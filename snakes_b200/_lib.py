@@ -109,6 +109,7 @@ _SIGNATURES = {
     "snk_save_envs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t, C.c_void_p]),
     "snk_restore_envs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t, C.c_void_p]),
     "snk_copy_envs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    "snk_clone_envs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     "snk_get_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "snk_reset_stats": (C.c_int, [C.c_void_p, C.c_void_p]),
     "snk_check_errors": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint32), C.c_void_p]),
@@ -136,6 +137,11 @@ _SIGNATURES = {
                                            C.c_void_p, C.c_void_p, C.c_size_t, C.c_int32, C.c_void_p]),
     "snk_tally_layout": (C.c_int, [C.c_void_p, C.POINTER(C.c_size_t)]),
     "snk_tally": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "snk_search_begin": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p,
+                                   C.c_void_p]),
+    "snk_search_accumulate": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "snk_search_pick": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,
+                                  C.c_void_p]),
     "snk_algorithmic_bytes_per_step":(C.c_int, [C.POINTER(SnkConfig), C.c_double, C.POINTER(C.c_double)]),
     "snk_launch_count": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
     "snk_launch_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),

@@ -14,9 +14,23 @@ import math
 import numpy as np
 import torch
 
-from . import _lib
+from . import _lib, search
 
 PLAYER_KINDS = ("scripted", "random")
+
+
+class Search(object):
+    """A rollout-search player (search.RolloutSearch): for every env of its block and its seat, each candidate action is
+    played from `rollouts` clones of the env, followed by `horizon` steps of the `rollout` policy ('scripted' with
+    `eps`, or 'random') keyed by `seed`, and the action of the largest summed return is taken.  It needs no training,
+    and with random rollouts it plays every rule-set and every step family."""
+
+    def __init__(self, rollouts=8, horizon=16, rollout="scripted", eps=0.05, seed=1):
+        self.rollouts, self.horizon, self.rollout, self.eps, self.seed = int(rollouts), int(horizon), rollout, float(eps), int(seed)
+
+    def __repr__(self):
+        return "Search(rollouts=%d, horizon=%d, rollout=%r, eps=%g, seed=%d)" % (
+            self.rollouts, self.horizon, self.rollout, self.eps, self.seed)
 POLL_STEPS = 32   # steps between two reads of the finished-env counter (one 8-byte copy)
 
 
@@ -52,6 +66,9 @@ def _check_player(env, p):
         if p == "scripted" and (env.cfg.rules != _lib.RULES["classic"] or env.launch_info()["kind"] != 0):
             raise ValueError("'scripted' needs a lane-family env with classic rules (snk_gen_scripted_actions)")
         return
+    if isinstance(p, Search):
+        search.check_args(env, p.rollouts, p.horizon, p.rollout)
+        return
     if not callable(getattr(p, "step", None)):
         raise ValueError("a player is a model (anything with .step(ob, view)), 'scripted' or 'random', got %r" % (p,))
     net = _net(p)
@@ -86,8 +103,9 @@ def play(env, matches, episodes=1, seed=1, eps=0.05):
     """Plays every match of `matches` (a list of tuples of env.S players) on `env`, `episodes` episodes per env, in every
     seat rotation.  A player is a model (anything whose .step(ob, view) returns the actions first: selfplay.Model or
     CnnPolicy, grid models on an obs_mode 'grid' env, RGB models otherwise), 'scripted' (the device's fruit-seeking
-    policy, gen_scripted_actions with `eps`; lane-family classic envs only) or 'random' (gen_actions).  `seed` keys the
-    scripted and random action streams.  The env is reset first and must auto-reset and keep its observations on the
+    policy, gen_scripted_actions with `eps`; lane-family classic envs only), 'random' (gen_actions) or a Search (rollout
+    search: one search.RolloutSearch per Search object of the call, sized to the largest block, acts for each of its
+    (block, seat) pairs on that block's envs before every step).  `seed` keys the scripted and random action streams.  The env is reset first and must auto-reset and keep its observations on the
     device; an RGB env needs one view per seat (n_views >= S).
 
     Returns one record per match: {'players': [per-player dict of episodes, wins, draws, losses, score = (wins +
@@ -129,17 +147,24 @@ def play(env, matches, episodes=1, seed=1, eps=0.05):
     # per (block, seat): who acts there; a model plays a block's seat with one forward call on that block
     kinds = sorted({p for m in matches for p in m if isinstance(p, str)})
     from_kind = {k: torch.zeros((N, S), dtype=torch.bool, device=dev) for k in kinds}
-    model_calls = []
+    model_calls, search_calls = [], []
     for m, r, b0, b1 in layout:
         for i, p in enumerate(matches[m]):
             s = seat_of(i, r, S)
             if isinstance(p, str):
                 from_kind[p][b0:b1, s] = True
+            elif isinstance(p, Search):
+                search_calls.append((p, b0, b1, s, torch.arange(b0, b1, dtype=torch.int64, device=dev)))
             else:
                 model_calls.append((p, b0, b1, s))
     scratch = {k: torch.empty((N, S), dtype=torch.int8, device=dev) for k in kinds}
     actions = torch.zeros((N, S), dtype=torch.int8, device=dev)
     grid = env.obs_mode == "grid"
+    largest = max(b1 - b0 for _, _, b0, b1 in layout)
+    searchers = {}
+    for p, _, _, _, _ in search_calls:
+        if p not in searchers:
+            searchers[p] = search.RolloutSearch(env, largest, p.rollouts, p.horizon, p.rollout, p.eps, p.seed)
 
     env.reset()
     stream = env._stream()
@@ -152,6 +177,8 @@ def play(env, matches, episodes=1, seed=1, eps=0.05):
         for p, b0, b1, s in model_calls:
             ob = obs[b0:b1] if grid else obs[b0:b1, ..., 3 * s:3 * s + 3]
             actions[b0:b1, s] = p.step(ob, s)[0].to(torch.int8)
+        for p, b0, b1, s, roots in search_calls:
+            searchers[p].act(s, roots, out=actions[b0:b1, s])
         if "scripted" in kinds:
             env.gen_scripted_actions(t, seed, eps, out=scratch["scripted"])
         if "random" in kinds:
@@ -167,6 +194,9 @@ def play(env, matches, episodes=1, seed=1, eps=0.05):
             if t > limit:
                 raise RuntimeError("%d of %d envs finished %d episodes in %d steps" % (int(envs_done.item()), N, episodes, t))
     env.check_errors()
+    for rs in searchers.values():
+        rs.search_env.check_errors()
+        rs.close()
     c = counts.cpu().numpy().reshape(len(matches), S, S, F)
     records = []
     for m, match in enumerate(matches):

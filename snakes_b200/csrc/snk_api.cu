@@ -1235,9 +1235,33 @@ extern "C" int snk_copy_envs(snk_handle* h, const int64_t* d_src, const int64_t*
   if (!h || !d_src || !d_dst) return fail(SNK_EINVAL, "NULL argument");
   if (count < 1) return fail(SNK_EINVAL, "count must be >= 1, got %lld", (long long)count);
   CUDA_TRY(cudaSetDevice(h->cfg.device));
-  CUDA_TRY(snk_launch_copy(h->p, d_src, d_dst, count, (cudaStream_t)stream));
+  CUDA_TRY(snk_launch_copy(h->p, h->p, d_src, d_dst, count, (cudaStream_t)stream));
   h->launches++;
   if (!stream_capturing((cudaStream_t)stream)) h->obs_current = nullptr;
+  return SNK_OK;
+}
+
+extern "C" int snk_clone_envs(const snk_handle* src, const int64_t* d_src, snk_handle* dst, const int64_t* d_dst, int64_t count,
+                              void* stream) {
+  if (!src || !dst || !d_src || !d_dst) return fail(SNK_EINVAL, "NULL argument");
+  if (count < 1) return fail(SNK_EINVAL, "count must be >= 1, got %lld", (long long)count);
+  const snk_config &a = src->cfg, &b = dst->cfg;
+  if (a.device != b.device) return fail(SNK_EINVAL, "device differs: %d vs %d", a.device, b.device);
+  if (a.size != b.size) return fail(SNK_EINVAL, "size differs: %d vs %d", a.size, b.size);
+  if (a.n_snakes != b.n_snakes) return fail(SNK_EINVAL, "n_snakes differs: %d vs %d", a.n_snakes, b.n_snakes);
+  if (a.n_fruits != b.n_fruits) return fail(SNK_EINVAL, "n_fruits differs: %d vs %d", a.n_fruits, b.n_fruits);
+  if (a.rules != b.rules) return fail(SNK_EINVAL, "rules differ: %d vs %d", a.rules, b.rules);
+  // the private layout: the family follows the launch plan (the image size), so one configuration can have two
+  const Params &ps = src->p, &pd = dst->p;
+  const struct { const char* name; int s, d; } layout[] = {
+      {"family", ps.family, pd.family}, {"RW", ps.RW, pd.RW}, {"CW", ps.CW, pd.CW}, {"cap", ps.cap, pd.cap},
+      {"grid_stride", ps.grid_stride, pd.grid_stride}, {"GBW", ps.GBW, pd.GBW}};
+  for (const auto& f : layout)
+    if (f.s != f.d) return fail(SNK_EINVAL, "private layout differs: %s %d vs %d", f.name, f.s, f.d);
+  CUDA_TRY(cudaSetDevice(b.device));
+  CUDA_TRY(snk_launch_copy(ps, pd, d_src, d_dst, count, (cudaStream_t)stream));
+  dst->launches++;
+  if (!stream_capturing((cudaStream_t)stream)) dst->obs_current = nullptr;
   return SNK_OK;
 }
 
@@ -1516,6 +1540,64 @@ extern "C" int snk_tally(snk_handle* h, const int32_t* d_group, int32_t n_groups
   a.counts = d_counts; a.envs_done = d_envs_done; a.err = p.err;
   a.N = p.N; a.S = p.S; a.n_groups = n_groups; a.episodes_per_env = episodes_per_env;
   CUDA_TRY(snk_launch_tally(a, (cudaStream_t)stream));
+  h->launches++;
+  return SNK_OK;
+}
+
+// rollout search bookkeeping (snk_search.cu): slots j < n_roots * n_actions * rollouts of the handle
+static int search_check(const snk_handle* h, int32_t seat, int32_t n_actions, int32_t rollouts, int64_t n_roots, const void* d_ret) {
+  if (!h) return fail(SNK_EINVAL, "handle is NULL");
+  if (!d_ret) return fail(SNK_EINVAL, "NULL argument");
+  if (seat < 0 || seat >= h->p.S) return fail(SNK_EINVAL, "seat %d outside [0, %d)", seat, h->p.S);
+  if (n_actions < 1 || n_actions > 127) return fail(SNK_EINVAL, "n_actions must be 1..127, got %d", n_actions);
+  if (rollouts < 1) return fail(SNK_EINVAL, "rollouts must be >= 1, got %d", rollouts);
+  if (n_roots < 1 || n_roots * n_actions * rollouts > h->p.N)
+    return fail(SNK_EINVAL, "n_roots %lld x %d actions x %d rollouts outside [1, num_envs = %lld]", (long long)n_roots, n_actions,
+                rollouts, h->p.N);
+  if (misaligned(d_ret, 4)) return fail(SNK_EINVAL, "d_ret must be 4-byte aligned");
+  return SNK_OK;
+}
+
+static SearchArgs search_args(const snk_handle* h, int32_t seat, int32_t n_actions, int32_t rollouts, int64_t n_roots,
+                              int32_t* d_ret, uint8_t* d_active) {
+  SearchArgs a;
+  a.reward_all = h->p.reward_all; a.done = h->p.done; a.ret = d_ret; a.active = d_active;
+  a.S = h->p.S; a.seat = seat; a.n_actions = n_actions; a.rollouts = rollouts; a.n_roots = n_roots;
+  return a;
+}
+
+extern "C" int snk_search_begin(snk_handle* h, int8_t* d_actions, int32_t seat, int32_t n_actions, int32_t rollouts, int64_t n_roots,
+                                int32_t* d_ret, uint8_t* d_active, void* stream) {
+  int rc = search_check(h, seat, n_actions, rollouts, n_roots, d_ret);
+  if (rc) return rc;
+  if (!d_actions || !d_active) return fail(SNK_EINVAL, "NULL argument");
+  CUDA_TRY(cudaSetDevice(h->cfg.device));
+  CUDA_TRY(snk_launch_search_begin(search_args(h, seat, n_actions, rollouts, n_roots, d_ret, d_active), d_actions, (cudaStream_t)stream));
+  h->launches++;
+  return SNK_OK;
+}
+
+extern "C" int snk_search_accumulate(snk_handle* h, int32_t seat, int32_t n_actions, int32_t rollouts, int64_t n_roots, int32_t* d_ret,
+                                     uint8_t* d_active, void* stream) {
+  int rc = search_check(h, seat, n_actions, rollouts, n_roots, d_ret);
+  if (rc) return rc;
+  if (!d_active) return fail(SNK_EINVAL, "NULL argument");
+  CUDA_TRY(cudaSetDevice(h->cfg.device));
+  CUDA_TRY(snk_launch_search_accumulate(search_args(h, seat, n_actions, rollouts, n_roots, d_ret, d_active), (cudaStream_t)stream));
+  h->launches++;
+  return SNK_OK;
+}
+
+extern "C" int snk_search_pick(snk_handle* h, int32_t n_actions, int32_t rollouts, int64_t n_roots, const int32_t* d_ret,
+                               float* d_value, int8_t* d_pick, int64_t pick_stride, void* stream) {
+  int rc = search_check(h, 0, n_actions, rollouts, n_roots, d_ret);
+  if (rc) return rc;
+  if (!d_value || !d_pick) return fail(SNK_EINVAL, "NULL argument");
+  if (pick_stride < 1) return fail(SNK_EINVAL, "pick_stride must be >= 1, got %lld", (long long)pick_stride);
+  if (misaligned(d_value, 4)) return fail(SNK_EINVAL, "d_value must be 4-byte aligned");
+  CUDA_TRY(cudaSetDevice(h->cfg.device));
+  SearchArgs a = search_args(h, 0, n_actions, rollouts, n_roots, (int32_t*)d_ret, nullptr);
+  CUDA_TRY(snk_launch_search_pick(a, d_value, d_pick, pick_stride, (cudaStream_t)stream));
   h->launches++;
   return SNK_OK;
 }

@@ -1466,40 +1466,42 @@ __global__ void __launch_bounds__(256) k_restore_envs(const Params p, const int6
 }
 
 // private -> private, one warp per (src, dst) pair: the record, the chain words >= 1 each body reaches (lane family) or the
-// whole ring row (ring family), the fruit count grid and the lane family's fruit bitmap; clears frame_ok[dst].
-__global__ void k_copy_envs(const Params p, const int64_t* __restrict__ src,
+// whole ring row (ring family), the fruit count grid and the lane family's fruit bitmap; clears frame_ok[dst].  Env src[j]
+// of handle `ps` into env dst[j] of handle `pd`: the same handle for snk_copy_envs, two handles of one private layout
+// (family, RW, CW, cap, grid_stride, GBW, checked by snk_clone_envs) otherwise.  `ps` is only read.
+__global__ void k_copy_envs(const Params ps, const Params pd, const int64_t* __restrict__ src,
                             const int64_t* __restrict__ dst, long long count) {
-  const int lane = threadIdx.x & 31, S = p.S;
+  const int lane = threadIdx.x & 31, S = pd.S;
   const long long j = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
   if (j >= count) return;
   const long long es = src[j], ed = dst[j];
-  if (es < 0 || es >= p.N || ed < 0 || ed >= p.N) {
-    if (lane == 0) atomicOr(p.err, SNK_DEVERR_BAD_STATE);
+  if (es < 0 || es >= ps.N || ed < 0 || ed >= pd.N) {
+    if (lane == 0) atomicOr(pd.err, SNK_DEVERR_BAD_STATE);
     return;
   }
-  const u32* rs = p.rec + es * p.RW;
-  u32* rd = p.rec + ed * p.RW;
-  for (int w = lane; w < p.RW; w += 32) rd[w] = rs[w];
-  if (p.family == 1) {
+  const u32* rs = ps.rec + es * pd.RW;
+  u32* rd = pd.rec + ed * pd.RW;
+  for (int w = lane; w < pd.RW; w += 32) rd[w] = rs[w];
+  if (pd.family == 1) {
     for (int s = 0; s < S; ++s) {
       const int len = rs[REC_SNAKE0 + 2 * s] >> 16;
       const int nw = len >= 2 ? ((len - 2) >> 4) + 1 : 0;  // words holding codes 0 .. len-2; word 0 is in the record
-      const u32* cs = p.chain + (es * S + s) * p.CW;
-      u32* cd = p.chain + (ed * S + s) * p.CW;
+      const u32* cs = ps.chain + (es * S + s) * pd.CW;
+      u32* cd = pd.chain + (ed * S + s) * pd.CW;
       for (int w = 1 + lane; w < nw; w += 32) cd[w] = cs[w];
     }
-    if (lane == 0) p.frame_ok[ed] = 0;
+    if (lane == 0) pd.frame_ok[ed] = 0;
   } else {
-    const uint4* bs = reinterpret_cast<const uint4*>(p.body + es * S * p.cap);
-    uint4* bd = reinterpret_cast<uint4*>(p.body + ed * S * p.cap);
-    for (int k = lane; k < S * p.cap / 8; k += 32) bd[k] = bs[k];
+    const uint4* bs = reinterpret_cast<const uint4*>(ps.body + es * S * pd.cap);
+    uint4* bd = reinterpret_cast<uint4*>(pd.body + ed * S * pd.cap);
+    for (int k = lane; k < S * pd.cap / 8; k += 32) bd[k] = bs[k];
   }
-  if (p.grid) {
-    const uint4* gs = reinterpret_cast<const uint4*>(p.grid + es * p.grid_stride);
-    uint4* gd = reinterpret_cast<uint4*>(p.grid + ed * p.grid_stride);
-    for (int k = lane; k < p.grid_stride / 16; k += 32) gd[k] = gs[k];
-    if (p.gbits)
-      for (int w = lane; w < p.GBW; w += 32) p.gbits[ed * p.GBW + w] = p.gbits[es * p.GBW + w];
+  if (pd.grid) {
+    const uint4* gs = reinterpret_cast<const uint4*>(ps.grid + es * pd.grid_stride);
+    uint4* gd = reinterpret_cast<uint4*>(pd.grid + ed * pd.grid_stride);
+    for (int k = lane; k < pd.grid_stride / 16; k += 32) gd[k] = gs[k];
+    if (pd.gbits)
+      for (int w = lane; w < pd.GBW; w += 32) pd.gbits[ed * pd.GBW + w] = ps.gbits[es * pd.GBW + w];
   }
 }
 
@@ -1781,8 +1783,9 @@ cudaError_t snk_launch_restore(const Params& p, const int64_t* idx, long long co
   return cudaGetLastError();
 }
 
-cudaError_t snk_launch_copy(const Params& p, const int64_t* src, const int64_t* dst, long long count, cudaStream_t stream) {
-  k_copy_envs<<<(unsigned)((count + 7) / 8), 256, 0, stream>>>(p, src, dst, count);
+cudaError_t snk_launch_copy(const Params& ps, const Params& pd, const int64_t* src, const int64_t* dst, long long count,
+                            cudaStream_t stream) {
+  k_copy_envs<<<(unsigned)((count + 7) / 8), 256, 0, stream>>>(ps, pd, src, dst, count);
   return cudaGetLastError();
 }
 

@@ -48,7 +48,9 @@ cudaError_t snk_launch_save(const Params& p, const int64_t* idx, long long first
                             const snk_state_layout& lay, cudaStream_t stream);
 cudaError_t snk_launch_restore(const Params& p, const int64_t* idx, long long count, const uint8_t* blob, const snk_state_layout& lay,
                                cudaStream_t stream);
-cudaError_t snk_launch_copy(const Params& p, const int64_t* src, const int64_t* dst, long long count, cudaStream_t stream);
+// k_copy_envs: env src[j] of `ps` -> env dst[j] of `pd` (one handle, or two of the same private layout)
+cudaError_t snk_launch_copy(const Params& ps, const Params& pd, const int64_t* src, const int64_t* dst, long long count,
+                            cudaStream_t stream);
 cudaError_t snk_launch_sum_inbox(const PeerArgs& a, const double* stats, double* glob, cudaStream_t stream);
 cudaError_t snk_launch_expand_views(const uint8_t* grid, long long n_cells, int first_view, int n_views, uint8_t* out, cudaStream_t stream);
 // snk_grid_conv.cu: the grid's first convolution layer (n_cells = n * V * V) and the CTA count of its weight gradient
@@ -93,3 +95,16 @@ struct TallyArgs {
   int S, n_groups, episodes_per_env;
 };
 cudaError_t snk_launch_tally(const TallyArgs& a, cudaStream_t stream);
+// snk_search.cu: rollout-search bookkeeping (snk_search_begin / _accumulate / _pick).  Slot j < n_roots * n_actions *
+// rollouts of the search handle is root j / (n_actions * rollouts), candidate action (j / rollouts) % n_actions.
+struct SearchArgs {
+  const float* reward_all;  // [N][S] the search handle's per-step outputs
+  const uint8_t* done;      // [N]
+  int32_t* ret;             // [slots] return of `seat` over the counted steps
+  uint8_t* active;          // [slots] 1 until the slot's last counted step has been added
+  int S, seat, n_actions, rollouts;
+  long long n_roots;
+};
+cudaError_t snk_launch_search_begin(const SearchArgs& a, int8_t* actions, cudaStream_t stream);
+cudaError_t snk_launch_search_accumulate(const SearchArgs& a, cudaStream_t stream);
+cudaError_t snk_launch_search_pick(const SearchArgs& a, float* value, int8_t* pick, long long pick_stride, cudaStream_t stream);

@@ -677,6 +677,25 @@ class SnakeVecEnv(object):
         if observe:
             self._observe()
 
+    def clone_envs_from(self, src_env, src, dst, observe=True):
+        """Env dst[j] of this env <- env src[j] of `src_env` on the device (snk_clone_envs): copy_envs across handles.
+        src_env is only read.  Both handles must be on one device with the same size, n_snakes, n_fruits and rules and
+        the same private layout (a grid-mode and a native handle of one configuration can differ there: SnkError).
+        src may repeat; dst must be distinct.  A clone keeps this env's RNG key, so it equals its source until the next
+        random draw.  `observe` as in restore_envs."""
+        if src_env is self:
+            raise ValueError("src_env is this env: use copy_envs")
+        s, ns, _ = src_env._env_index(src)
+        d, nd, _ = self._env_index(dst, distinct=True)
+        if ns != nd:
+            raise ValueError("%d sources for %d destinations" % (ns, nd))
+        if observe:
+            self._before_overwrite()
+        _lib.check(self._L.snk_clone_envs(src_env._h, C.c_void_p(s.data_ptr()), self._h, C.c_void_p(d.data_ptr()), ns,
+                                          self._stream()))
+        if observe:
+            self._observe()
+
     def save(self, path):
         """Checkpoint of the env state (the reference never checkpoints it; its learner only saves
         model parameters, ppo_multi_agent_new.py:104-106).  A .npz with the constructor arguments
