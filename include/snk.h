@@ -535,7 +535,8 @@ int snk_launch_count(const snk_handle* h, uint64_t* out);
 /* The launch plan of the step kernel (bench.py's config.kernel): kind (0 lane, 1 tile, 2 dense, 3 rows), grid, block,
  * dynamic shared memory bytes, resident CTAs per SM, envs per CTA. */
 int snk_launch_info(const snk_handle* h, int32_t* out /*[6]*/);
-/* Which form of the lane path the NEXT step will launch (it follows the body-length regime, DESIGN.md 4.8):
+/* Which form of the lane path the NEXT eager step will launch (it follows the body-length regime, DESIGN.md 4.8; a classic
+ * step recorded into a graph that stores sectors into the own buffer follows thresholds of its own, DESIGN.md 4.20):
  * out[0] = 0 fused kernel, 1 warp-specialised kernel, 3 two kernels (k_lane_logic + k_lane_paint2, or + k_lane_grid in
  * SNK_OBS_GRID, which always uses this form), -1 not a lane-family
  * configuration (2 is no longer reported); out[1] = envs stepped per warp batch of the fused kernel;

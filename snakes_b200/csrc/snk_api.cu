@@ -66,9 +66,9 @@ struct snk_handle {
   uint8_t* d_obs_own;     // native observations (the step kernels' output)
   // regime-adaptive lane path: `plan` is the fused kernel, `plan_alt` the two-kernel form (k_lane_logic + k_lane_paint2)
   LaunchPlan plan_alt;
-  bool have_alt, use_alt;
+  bool have_alt, use_alt, use_alt_sec;  // use_alt_sec: the form of a graph-captured step that stores sectors (regime_update)
   double* h_regime;            // mapped pinned host memory [2]: env-steps, body cells (Params::regime_out)
-  double reg_steps0, reg_cells0, alt_hi, alt_lo;
+  double reg_steps0, reg_cells0, alt_hi, alt_lo, sec_hi, sec_lo;
   const uint8_t* obs_current;  // where the native observations of the CURRENT state are (NULL: not encoded since the state changed)
   uint8_t* d_obs84_own;   // obs_mode atari84: the 84x84 images handed to the caller
   uint8_t* d_obs_user;    // what snk_get_buffers reports: own buffer or the caller's target
@@ -302,24 +302,42 @@ static int plan_launch(snk_handle* h) {
     plan.envs_per_cta = p.W;
     CUDA_TRY(finish(plan));
   }
-  // Regime-adaptive lane path.  With short bodies the fused kernel wins (2x19x19, 131 072 envs, random actions: 64.5 us
-  // against 73.3 us for the two-kernel form: the logic hides under the observation stream); with long bodies its warps
-  // -- ten per SM, each a serial chain through 78 KB of code, 2.4x the instruction cache -- fall behind and the two
-  // small kernels win.  Measured on one box, mean body cells per env 5.8 / 8.6 / 12.8 / 22.2 (fruit-seeking policy with
-  // 70 / 40 / 20 / 5 % random actions): fused 72.6 / 83.0 / 92.4 / 109.9 us, two kernels 75.9 / 79.8 / 85.6 / 93.4 us.  The host cannot know
-  // the regime without the statistics, so the first CTA of every step posts the running sums into mapped host memory
-  // (peer_push) and regime_update() reads them -- no synchronisation, a step or two late, which is early enough
-  // for a quantity that moves over hundreds of steps.  Results are bit-identical either way.  adaptive=0 turns it off.
+  // Regime-adaptive lane path: `plan` the fused kernel, `plan_alt` the two-kernel form (k_lane_logic + k_lane_paint2).  The
+  // fused kernel's warps are serial chains (logic of a batch, then its images, ten warps per SM); the two kernels run the
+  // logic at full occupancy in one wave and pay for a second launch.  Two pairs of thresholds in body cells per env, with
+  // hysteresis, pick between them (launch()):
+  //  * alt_hi / alt_lo: a step that stores whole images, or an eager step.  With short bodies the fused kernel wins
+  //    (2x19x19, 131 072 envs, random actions: 64.5 us against 73.3 us for the two-kernel form with whole images); with
+  //    long bodies its warps fall behind.  Measured on one box, body cells per env 5.8 / 8.6 / 12.8 / 22.2 (fruit-seeking
+  //    policy with 70 / 40 / 20 / 5 % random actions): fused 72.6 / 83.0 / 92.4 / 109.9 us, two kernels 75.9 / 79.8 /
+  //    85.6 / 93.4 us; 8 cells at 2646 bytes of image per env, scaled with the image.  Eager steps keep these thresholds
+  //    even when they store sectors: a second launch per step costs an eager loop with per-step copies more than the
+  //    two-kernel form saves (bench.py e2e_obs_resident, 131 072 envs: 4.09e9 against 4.54e9 agent-steps/s, §4.20).
+  //  * sec_hi / sec_lo: a classic step recorded into a graph that stores sectors into the own buffer (native
+  //    observations).  Both forms then store sectors.  Measured on B200 (2x19x19, same states and actions; body cells
+  //    4.3 random, then 5.0 / 6.0 / 7.6 / 11.2 fruit-seeking as above), two kernels / fused:
+  //      131 072 envs: 0.93 / 0.80 / 0.74 / 0.70 / 0.77     1 M envs: 0.96 / 0.79 / 0.68 / 0.70 / 0.83
+  //       32 768 envs: 1.04 / 0.96 / 0.92 / 0.90 / 0.95
+  //    So once the fused kernel's warps must step more than one batch each, the two-kernel form wins at every body
+  //    length (sec_hi = 0); with one batch per warp the forms cross near 5 body cells per env, scaled with the image.
+  // The host cannot know the regime without the statistics, so the first CTA of every step posts the running sums into
+  // mapped host memory (peer_push) and regime_update() reads them -- no synchronisation, a step or two late, which is
+  // early enough for a quantity that moves over hundreds of steps.  Results are bit-identical either way.  adaptive=0
+  // turns it off; alt_hi=<n> sets both thresholds.
   std::string lv;
   if (form == FORM_LANE && p.EPW == 32 && !dbg_get(dbg, "lane", &lv) && dbg_int(dbg, "adaptive", 1) != 0) {
+    const bool one_round = (N + 31) / 32 <= (long long)plan.max_grid * 2;  // every 32-env batch finds a resident warp
     // the alternative steps the same 32-env batches: p's lane geometry stays as it is
     h->have_alt = plan_lane(h->plan_alt, FORM_LANE_SPLIT, p.TE, 32, 64) == cudaSuccess;
     cudaGetLastError();
-    // thresholds in body cells per env, hysteresis between them; measured at 2646 bytes of image per env and scaled
-    // with the image (the larger the image, the longer the stream hides the fused kernel's logic)
     const int hi = dbg_int(dbg, "alt_hi", 0);
     h->alt_hi = hi > 0 ? (double)hi : 8.0 * (double)p.E / 2646.0;
+    h->sec_hi = hi > 0 ? (double)hi : one_round ? 5.0 * (double)p.E / 2646.0 : 0.0;
     h->alt_lo = 0.75 * h->alt_hi;
+    h->sec_lo = 0.75 * h->sec_hi;
+    // the forms for a fresh reset: every snake one cell long
+    h->use_alt = (double)S > h->alt_hi;
+    h->use_alt_sec = (double)S > h->sec_hi;
   }
   return SNK_OK;
 }
@@ -496,7 +514,7 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   if (h->cfg.max_steps == 0) h->cfg.max_steps = 2000;
   h->launches = 0;
   h->d_main_target = nullptr;
-  h->obs_current = nullptr; h->have_alt = false; h->use_alt = false; h->h_regime = nullptr; h->reg_steps0 = h->reg_cells0 = 0.0;
+  h->obs_current = nullptr; h->have_alt = false; h->use_alt = h->use_alt_sec = false; h->h_regime = nullptr; h->reg_steps0 = h->reg_cells0 = 0.0;
   h->d_obs_own = nullptr; h->d_actions_own = nullptr; h->d_blob = nullptr; h->blob_bytes = 0; h->d_views = nullptr; h->views_bytes = 0;
   h->d_tape_vals = h->d_tape_bounds = nullptr; h->d_tape_off = nullptr;
   h->comm = nullptr; h->comm_ranks = 1; h->comm_rank = 0; h->side = nullptr; h->cap_stream = nullptr;
@@ -555,16 +573,17 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   p.obs = h->d_obs_own;
   if (p.family == 1) {
     // frame_ok[e] = 1 <=> d_obs_own holds exactly the image of env e's record (cleared here and by every restore / copy, written
-    // by every lane-family kernel that writes a record).  With it the fused kernel's classic step stores only the sectors
-    // a step changes; delta=0 always stores whole images.  Sectors never cross env boundaries because the first and last
+    // by every lane-family kernel that writes a record).  With it the lane path's classic step (fused kernel and two-kernel
+    // form) stores only the sectors a step changes; delta=0 always stores whole images.  Sectors never cross env boundaries because the first and last
     // (V+1)*C bytes of an env image are border (needs >= 32) and the buffer is 32-byte aligned.  Default: 32-env batches
     // only.  A small shard (smaller batches, §4.10 of DESIGN.md) is bound by one warp's serial chain, not by the stream,
     // and there the sector loop is longer than one bulk-store issue (2x10x10, 4 096 envs on B200: 10.39 vs 9.86 us per
     // step); the headline shard gains 64.5 -> 52.7 us.  delta=0 / delta=1 turn it off / on regardless.
-    TRY(dev_alloc(h, &p.frame_ok, (size_t)N, true));
     const int dm = dbg_int(dbg, "delta", -1);
+    // Default: 32-env batches of the fused kernel and its adaptive pair.  The small-image two-kernel form (§4.8) keeps whole
+    // images: there the sector store is slower (3x10x10 classic, 65 536 envs on B200: 45.8 us per step with sectors, 41.9 us whole).
     p.delta = !grid && cfg->rules == SNK_RULES_CLASSIC && (V + 1) * p.C >= 32 && ((uintptr_t)h->d_obs_own & 31) == 0 &&
-              (dm < 0 ? p.EPW == 32 : dm != 0);
+              (dm < 0 ? p.EPW == 32 && h->plan.form != FORM_LANE_SPLIT : dm != 0);
   }
   h->d_obs84_own = nullptr;
   h->obs_out_env_bytes = (size_t)p.E;
@@ -589,6 +608,13 @@ extern "C" int snk_create_ex(const snk_config* cfg, const char* debug_opts, snk_
   TRY(dev_alloc(h, &p.err, (size_t)1, true));
   TRY(dev_alloc(h, &p.ticket, (size_t)1, true));
   TRY(dev_alloc(h, &h->d_actions_own, (size_t)N * S, true));
+  if (p.family == 1) {
+    // frame_ok, and the two-kernel form's writer learns the old state from k_lane_logic: DeltaPrev entries (8 words per env
+    // for S <= 2, 12 for S <= 4) from the first 256-byte boundary past the flags (delta_prev() in snk_lane.cuh).  Allocated
+    // whenever p.delta is set, whatever the form: a launch's Params::delta never exceeds the handle's, so every launch that
+    // may write or read the entries finds them.  Last of the per-env buffers, so that the entries move no other buffer.
+    TRY(dev_alloc(h, &p.frame_ok, p.delta ? (size_t)((N + 255) & ~255LL) + (size_t)N * 4 * ((2 * S + 6) & ~3) : (size_t)N, true));
+  }
 
   // lookup tables: padded id -> (outside?, y-major board index incl. the reference's aliasing), and back
   std::vector<uint32_t> cellinfo((size_t)p.VV);
@@ -672,6 +698,8 @@ static void regime_update(snk_handle* h) {
   h->reg_steps0 = steps; h->reg_cells0 = cells;
   if (mean > h->alt_hi) h->use_alt = true;
   else if (mean < h->alt_lo) h->use_alt = false;
+  if (mean > h->sec_hi) h->use_alt_sec = true;
+  else if (mean < h->sec_lo) h->use_alt_sec = false;
 }
 
 static int launch(snk_handle* h, int mode, const int8_t* d_actions, const uint8_t* d_mask, cudaStream_t stream,
@@ -719,7 +747,9 @@ static int launch(snk_handle* h, int mode, const int8_t* d_actions, const uint8_
   }
   p.snap = snap;
   if (mode == MODE_STEP) regime_update(h);
-  const bool alt = h->have_alt && h->use_alt;
+  // a graph-captured classic step that stores sectors into the own buffer follows sec_hi / sec_lo (plan_launch)
+  const bool sectors = capturing && p.delta && h->cfg.obs_mode == SNK_OBS_NATIVE;
+  const bool alt = h->have_alt && (sectors ? h->use_alt_sec : h->use_alt);
   const LaunchPlan& plan = alt ? h->plan_alt : h->plan;
   p.restore_thr = plan.restore_thr;
   CUDA_TRY(snk_launch_step(p, plan, stream));

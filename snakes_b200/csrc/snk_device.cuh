@@ -49,7 +49,7 @@ struct Params {
   int R;                        // rows kernel: image rows per chunk buffer
   u32 magicV, magicD;           // n / V == (n * magicV) >> 16 for n < V*V, n / D likewise for n < D*D (65536 / d + 1; exact while n * d < 65536)
   int restore_thr;              // lane kernel: un-paint an image by zero-fill + border redraw when a lane would walk more segments than this (0 = always walk)
-  int delta;                    // fused lane kernel, classic step into the own buffer: an image whose envs all have frame_ok stores only the 32-byte sectors the step can change
+  int delta;                    // lane family (fused and two-kernel form), classic step into the own buffer: an image whose envs all have frame_ok stores only the 32-byte sectors the step can change
   int frame_own;                // this launch writes a complete image of every env into the handle's own observation buffer (lane_store writes it to frame_ok)
   int max_steps, auto_reset, rng_mode, mode;
   long long N, env_id_base, n_groups;
@@ -63,6 +63,7 @@ struct Params {
   const u8* mask;
   u8* obs;
   u8* frame_ok;                 // [N] lane family: 1 = the own observation buffer holds exactly the image of the env's record
+                                // (with `delta`, followed by the two-kernel form's DeltaPrev entries: delta_prev(); allocated whenever the handle's `delta` is set)
   float* reward;
   float* reward_all;
   u8* done;

@@ -306,7 +306,11 @@ __global__ void __launch_bounds__(128, (S <= 2 ? 7 : 1)) k_lane_logic(const Para
     const FruitSet grid = fruit_set(p, e);
     LaneRaw<S> raw;
     raw.act = 0;
-    if (valid) { raw = lane_fetch<S>(p, e, p.mode == MODE_STEP); lane_unpack<S>(raw, env); }
+    if (valid) {
+      raw = lane_fetch<S>(p, e, p.mode == MODE_STEP);
+      if (RULES == SNK_RULES_CLASSIC && p.delta) delta_prev_store<S>(p, e, raw);  // for the writer's sector store
+      lane_unpack<S>(raw, env);
+    }
     if (p.mode == MODE_STEP) {
       lane_step<S, RULES, true>(p, e, valid, env, raw.act, rng, grid, s_bm[tid >> 5], errs, st, s_hop);
     } else if (valid && (!p.mask || p.mask[e])) {
@@ -416,7 +420,7 @@ __device__ __forceinline__ void cta_paint(const Params& p, const PaintEnv<S>& pe
       }
     }
   }
-  __syncthreads();
+  if (paint) __syncthreads();  // un-painting writes zeros only: its groups need no order
 #pragma unroll
   for (int s = 0; s < S; ++s) {
     if (runs.i[s] < runs.i1[s]) {
@@ -433,12 +437,14 @@ __device__ __forceinline__ void cta_paint(const Params& p, const PaintEnv<S>& pe
         if ((i & 15) == 0) w = ch[i >> 4];
       }
     }
-    if (s + 1 < S) __syncthreads();
+    if (paint && s + 1 < S) __syncthreads();
   }
 }
 
 // Un-paint.  Short bodies: the same walk writes zeros.  Long bodies (`restore`): the threads zero-fill the buffer and
 // redraw the border (cta_restore).  A CTA's last image is not un-painted at all.
+// With Params::delta (classic RGB step) an image whose envs all qualify (delta_eligible, on the old state k_lane_logic left
+// at delta_prev()) goes out as its changed sectors (delta_store) instead of one bulk store.
 // GRID: the same writer for SNK_OBS_GRID (k_lane_grid), images of TE cell-code grids of V*V bytes.
 template <int S, int RULES, int K, bool GRID>
 __device__ __forceinline__ void lane_paint2_body(const Params& p, u8* smem, u64& s_bar) {
@@ -457,31 +463,41 @@ __device__ __forceinline__ void lane_paint2_body(const Params& p, u8* smem, u64&
   const long long n_items = (p.N + TE - 1) / TE;
   const long long stride = gridDim.x;
   long long item = blockIdx.x;
+  const bool delta = !GRID && RULES == SNK_RULES_CLASSIC && p.delta;
   asm volatile("griddepcontrol.wait;" ::: "memory");  // the records of this step come from k_lane_logic
   PaintEnv<S> cur = paint_env_from_memory<S>(p, item < n_items ? item * TE + slot : p.N);
+  DeltaOld<S> cur_old;
+  bool cur_frame = false;
+  if (delta && cur.valid) cur_old = delta_prev_load<S>(p, item * TE + slot, cur_frame);
   bool have_image = false;  // the border image has arrived in the buffer
   const int sh = 31 - __clz(LPE);
   while (item < n_items) {
     const long long next = item + stride;
     const PaintEnv<S> nxt = paint_env_from_memory<S>(p, next < n_items ? next * TE + slot : p.N);
+    DeltaOld<S> nxt_old;
+    bool nxt_frame = false;
+    if (delta && nxt.valid) nxt_old = delta_prev_load<S>(p, next * TE + slot, nxt_frame);
     const long long e0 = item * TE;
     int trips = 0;
 #pragma unroll
     for (int s = 0; s < S; ++s) trips += (cur.len[s] + LPE - 1) >> sh;
     const PaintRuns<S> runs = cta_paint_prepare<S>(p, cur, e0 + slot, sub, LPE);
-    const bool restore = __syncthreads_or(p.restore_thr > 0 && trips > p.restore_thr);
+    const bool ok = delta && (!cur.valid || delta_eligible<S>(cur_old, cur_frame, cur.len));
     if (!have_image) { mbar_wait(&s_bar, 0); have_image = true; }
     cta_paint<S, RULES, K, GRID>(p, cur, runs, e0 + slot, sub, LPE, img, true);
     fence_async_smem();
-    __syncthreads();
-    store_image(p, tile, tile_bytes, e0, tid, NT);
+    // the barriers that order the phases also take the CTA's votes
+    const bool sectors = __syncthreads_and(ok);
+    if (!GRID && RULES == SNK_RULES_CLASSIC && sectors) delta_store<S, K, true>(p, cur, cur_old, slot, sub, LPE, tile, (int)min((long long)TE, p.N - e0) * E, e0);
+    else store_image(p, tile, tile_bytes, e0, tid, NT);
     if (next < n_items) {  // the last image of a CTA leaves its buffer as it is
-      __syncthreads();
-      if (restore) cta_restore<GRID ? 1 : 3 * K>(tile, tile_bytes >> 4, img, p.V, sub, LPE, tid, NT);
+      if (__syncthreads_or(p.restore_thr > 0 && trips > p.restore_thr)) cta_restore<GRID ? 1 : 3 * K>(tile, tile_bytes >> 4, img, p.V, sub, LPE, tid, NT);
       else cta_paint<S, RULES, K, GRID>(p, cur, runs, e0 + slot, sub, LPE, img, false);
       __syncthreads();
     }
     cur = nxt;
+    cur_old = nxt_old;
+    cur_frame = nxt_frame;
     item = next;
   }
   if (!have_image) mbar_wait(&s_bar, 0);  // never leave with a bulk copy into our shared memory in flight
@@ -674,7 +690,7 @@ __global__ void __launch_bounds__(64, (S >= 3 ? 4 : 0)) k_step_lane(const Params
     u32 whole = ~0u;
     if (delta) {
       old = delta_old<S>(raw);
-      whole = __ballot_sync(FULL, valid && !delta_eligible<S>(old, raw.frame, env));
+      whole = __ballot_sync(FULL, valid && !delta_eligible<S>(old, raw.frame, env.len));
     }
     // records + actions of this warp's NEXT batch: in flight while the current one is painted
     if (b + stride < n_batches && lane < EPW && (b + stride) * EPW + lane < p.N) raw = lane_fetch<S>(p, (b + stride) * EPW + lane, stepping);
@@ -696,7 +712,7 @@ __global__ void __launch_bounds__(64, (S >= 3 ? 4 : 0)) k_step_lane(const Params
 #endif
       if (((whole >> (q * TE)) & tile_mask) == 0) {
         const DeltaOld<S> po = delta_old_from_lane<S>(old, q * TE + slot);
-        delta_store<S, K>(p, pe, po, slot, sub, LPE, tile, (int)min((long long)TE, p.N - e0) * E, e0);
+        delta_store<S, K, false>(p, pe, po, slot, sub, LPE, tile, (int)min((long long)TE, p.N - e0) * E, e0);
       } else {
         store_image(p, tile, tile_bytes, e0, lane, 32);
       }

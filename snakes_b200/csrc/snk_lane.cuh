@@ -834,13 +834,59 @@ __device__ __forceinline__ DeltaOld<S> delta_old(const LaneRaw<S>& raw) {
   return o;
 }
 
-// the owner lane's verdict: the old frame is in the buffer and every old and new body fits the first chain word
+// the verdict for one env: the old frame is in the buffer and every old and new body fits the first chain word
 template <int S>
-__device__ __forceinline__ bool delta_eligible(const DeltaOld<S>& o, bool frame, const LaneEnv<S>& env) {
+__device__ __forceinline__ bool delta_eligible(const DeltaOld<S>& o, bool frame, const int (&len)[S]) {
   bool ok = frame;
 #pragma unroll
-  for (int s = 0; s < S; ++s) ok = ok && (o.hl[s] >> 16) <= DELTA_MAX_LEN && env.len[s] <= DELTA_MAX_LEN;
+  for (int s = 0; s < S; ++s) ok = ok && (o.hl[s] >> 16) <= DELTA_MAX_LEN && len[s] <= DELTA_MAX_LEN;
   return ok;
+}
+
+// The two-kernel form: k_lane_logic keeps the old state's paint items and frame_ok of every env (W words: hl[S], c0[S],
+// fr[2], frame), written right after lane_fetch, for the observation writer behind it.  They live in the frame_ok
+// allocation, from the first 256-byte boundary past its N flags; snk_create_ex allocates them whenever the handle's
+// Params::delta is set, and no launch sets it otherwise.
+template <int S>
+struct DeltaPrev {
+  static constexpr int W = (2 * S + 3 + 3) & ~3;  // 32 bytes for S <= 2, 48 for S <= 4
+};
+__device__ __forceinline__ u32* delta_prev(const Params& p) { return reinterpret_cast<u32*>(p.frame_ok + ((p.N + 255) & ~255LL)); }
+
+template <int S>
+__device__ __forceinline__ void delta_prev_store(const Params& p, long long e, const LaneRaw<S>& raw) {
+  constexpr int RW = LaneRec<S>::RW, W = DeltaPrev<S>::W;
+  u32 r[RW], q[W];
+#pragma unroll
+  for (int i = 0; i < RW / 4; ++i) { r[4 * i] = raw.v[i].x; r[4 * i + 1] = raw.v[i].y; r[4 * i + 2] = raw.v[i].z; r[4 * i + 3] = raw.v[i].w; }
+#pragma unroll
+  for (int i = 0; i < W; ++i) q[i] = 0;
+#pragma unroll
+  for (int s = 0; s < S; ++s) { q[s] = r[REC_SNAKE0 + 2 * s]; q[S + s] = r[LaneRec<S>::c0_word(s)]; }
+  q[2 * S] = r[REC_SNAKE0 + 2 * S]; q[2 * S + 1] = r[REC_SNAKE0 + 2 * S + 1]; q[2 * S + 2] = raw.frame;
+  uint4* g = reinterpret_cast<uint4*>(delta_prev(p) + e * W);
+  u64 pol;  // read once by the writer right behind, then rewritten by the next step: keep it in the L2 like the records
+  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
+#pragma unroll
+  for (int i = 0; i < W / 4; ++i)
+    asm volatile("st.global.L2::cache_hint.v4.u32 [%0], {%1, %2, %3, %4}, %5;" ::"l"(g + i), "r"(q[4 * i]), "r"(q[4 * i + 1]),
+                 "r"(q[4 * i + 2]), "r"(q[4 * i + 3]), "l"(pol) : "memory");
+}
+
+// the writer's read of it (at the L2: k_lane_logic wrote it a moment ago); `frame` = the old frame_ok
+template <int S>
+__device__ __forceinline__ DeltaOld<S> delta_prev_load(const Params& p, long long e, bool& frame) {
+  constexpr int W = DeltaPrev<S>::W;
+  const uint4* g = reinterpret_cast<const uint4*>(delta_prev(p) + e * W);
+  u32 q[W];
+#pragma unroll
+  for (int i = 0; i < W / 4; ++i) { const uint4 v = __ldcg(g + i); q[4 * i] = v.x; q[4 * i + 1] = v.y; q[4 * i + 2] = v.z; q[4 * i + 3] = v.w; }
+  DeltaOld<S> o;
+#pragma unroll
+  for (int s = 0; s < S; ++s) { o.hl[s] = q[s]; o.c0[s] = q[S + s]; }
+  o.fr[0] = q[2 * S]; o.fr[1] = q[2 * S + 1];
+  frame = q[2 * S + 2] != 0;
+  return o;
 }
 
 template <int S>
@@ -870,11 +916,21 @@ __device__ __forceinline__ void delta_pixel(u8* g, const u8* tile, int bytes, in
   if (r1 != r0 && (u32)r1 <= (u32)(bytes - 32)) store_sector(g + r1, tile + r1, pol);
 }
 
-// Store the sectors of one env of the image.  Its paint items -- the new and the old classic fruits, then per snake the
-// segments of the new and of the old body -- are dealt round-robin to the env's LPE lanes; one loop with one store site
-// keeps the code small (the kernel lives off the instruction cache, see lane_reset).  `bytes` = bytes of the image that
-// belong to valid envs.
-template <int S, int K>
+// Store the sectors of one env of the image: the paint items whose pixel can differ between the two frames.
+//  * Every new fruit and the old cell of a fruit that moved; TIGHT: only a fruit whose cell changed, new and old cell (a
+//    fruit that stayed paints the same pixel in both frames).
+//  * A snake that moved (`shifted`: neither killed nor reset) has new segment i + 1 = old segment i for i < k =
+//    min(old length, new length - 1): of its old body only the segments from k on (the popped tail).  Every new segment;
+//    TIGHT: only new segments 0 and 1 (the new head, the old head turned body) and those past k -- the others are
+//    body-coloured in both frames.
+//  * Any other snake: every old and every new segment.
+// A cell where none of these lies holds the same items in the same paint order in both frames, so its pixel is unchanged
+// (tests/test_delta_rule_cpu.py checks both rules on oracle trajectories).  The fused kernel keeps the wider rule: there
+// the tight one's extra instructions cost more than its 42 % fewer stores save (2x19x19, 131 072 envs on B200: 54.7 vs
+// 52.8 us per step); in the observation writer of the two-kernel form the tight rule wins (49.3 vs 51.7 us).
+// The items are dealt round-robin to the env's LPE lanes; one loop with one store site keeps the code small (the fused
+// kernel lives off the instruction cache, see lane_reset).  `bytes` = bytes of the image that belong to valid envs.
+template <int S, int K, bool TIGHT>
 __device__ __forceinline__ void delta_store(const Params& p, const PaintEnv<S>& pe, const DeltaOld<S>& po, int slot, int sub, int LPE,
                                             const u8* tile, int bytes, long long e0) {
   constexpr int C = 3 * K;
@@ -885,37 +941,52 @@ __device__ __forceinline__ void delta_store(const Params& p, const PaintEnv<S>& 
   const int a = (int)(t0 & 31), base = slot * p.E;
   u64 pol;
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
-  // A snake that moved (and was neither killed nor reset) has old segment i = new segment i + 1: of its old body only the
-  // segments from new length - 1 on (the popped tail) are not in the new one.  `skip[s]` old segments are left out.
-  int n = 2 * F, skip[S];
+  u32 fm = 0;  // TIGHT: the fruits whose cell changed
+  if (TIGHT) {
+#pragma unroll
+    for (int f = 0; f < 4; ++f)
+      if (f < F && (int)((po.fr[f >> 1] >> (16 * (f & 1))) & 0xffffu) != pe.fruit[f]) fm |= 1u << f;
+  }
+  const int nf = TIGHT ? 2 * __popc(fm) : 2 * F;
+  // per snake: k[s] matched segments, of which the old ones are left out; TIGHT also leaves out the d[s] = k - 1 new
+  // segments 2..k
+  int n = nf, k[S], d[S];
 #pragma unroll
   for (int s = 0; s < S; ++s) {
     const int nl = pe.len[s], oh = (int)(po.hl[s] & 0xffffu), ol = (int)(po.hl[s] >> 16);
     const u32 m = ol >= 17 ? ~0u : (1u << (2 * max(ol - 1, 0))) - 1u;  // the codes of the old body
     const bool shifted = nl >= 1 && pe.head[s] - codes_disp(pe.c0[s], V, 1) == oh && (((pe.c0[s] >> 2) ^ po.c0[s]) & m) == 0;
-    skip[s] = shifted ? min(ol, nl - 1) : 0;
-    n += nl + ol - skip[s];
+    k[s] = shifted ? min(ol, nl - 1) : 0;
+    d[s] = TIGHT ? max(k[s] - 1, 0) : 0;
+    n += nl - d[s] + ol - k[s];
   }
   for (int j = sub; j < n; j += LPE) {
     int pid = 0;
-    if (j < 2 * F) {
+    if (j < nf) {
+      if (TIGHT) {
+        const int f = (int)__fns(fm, 0, (j >> 1) + 1);
 #pragma unroll
-      for (int f = 0; f < 4; ++f) {
-        const int of = (int)((po.fr[f >> 1] >> (16 * (f & 1))) & 0xffffu);
-        if (f < F && j == f) pid = pe.fruit[f];
-        if (f < F && j == F + f) pid = of == pe.fruit[f] ? -1 : of;  // a fruit that stayed is one of the new items
+        for (int q = 0; q < 4; ++q)
+          if (q == f) pid = (j & 1) ? (int)((po.fr[q >> 1] >> (16 * (q & 1))) & 0xffffu) : pe.fruit[q];
+      } else {
+#pragma unroll
+        for (int f = 0; f < 4; ++f) {
+          const int of = (int)((po.fr[f >> 1] >> (16 * (f & 1))) & 0xffffu);
+          if (f < F && j == f) pid = pe.fruit[f];
+          if (f < F && j == F + f) pid = of == pe.fruit[f] ? -1 : of;  // a fruit that stayed is one of the new items
+        }
       }
     } else {
-      int i = j - 2 * F, head = 0;
+      int i = j - nf, head = 0;
       u32 w = 0;
       bool found = false;
 #pragma unroll
       for (int s = 0; s < S; ++s) {
-        const int nl = pe.len[s], ol = (int)(po.hl[s] >> 16) - skip[s];
-        if (!found && i < nl) { head = pe.head[s]; w = pe.c0[s]; found = true; }
-        else if (!found) i -= nl;
-        if (!found && i < ol) { head = (int)(po.hl[s] & 0xffffu); w = po.c0[s]; i += skip[s]; found = true; }
-        else if (!found) i -= ol;
+        const int nn = pe.len[s] - d[s], on = (int)(po.hl[s] >> 16) - k[s];
+        if (!found && i < nn) { head = pe.head[s]; w = pe.c0[s]; if (TIGHT && i >= 2) i += d[s]; found = true; }
+        else if (!found) i -= nn;
+        if (!found && i < on) { head = (int)(po.hl[s] & 0xffffu); w = po.c0[s]; i += k[s]; found = true; }
+        else if (!found) i -= on;
       }
       pid = head - codes_disp(w, V, i);
     }

@@ -2,6 +2,8 @@
 (one launch per measurement, CUDA events), so Python is out of the numbers.
 
     python tools/ab.py short long c3 c2 1m atari rows      # any subset; default: short long
+    extra lines: c3c (3 snakes classic 10x10), adv (adversarial 2x19x19), grid (obs_mode grid 2x19x19), roll (graph with
+    per-step observation outputs, 2x19x19), e2e (eager step_scalars_async loop, 2x19x19)
 """
 import os
 import sys
@@ -40,6 +42,42 @@ def short(N, T=400, reps=3, tag="short", **kw):
     us = timed_graph(env, g, reps) / T * 1e3
     report("%s N=%d %s" % (tag, N, kw), env, us, N)
     g.close(); env.close()
+
+
+def roll(N, T=16, reps=3, **kw):
+    """A graph that writes every step's observations into its own [T] output (rollout slots): whole images."""
+    env = snakes_b200.SnakeVecEnv(N, **kw); env.reset()
+    acts = torch.stack([env.gen_actions(t, 1).clone() for t in range(T)])
+    obs = torch.empty((T,) + tuple(env.obs.shape), dtype=torch.uint8, device="cuda")
+    g = env.make_graph(acts, T=T, obs_out=obs)
+    g.launch()
+    env.reset_stats()
+    us = timed_graph(env, g, reps) / T * 1e3
+    report("roll N=%d %s" % (N, kw), env, us, N)
+    g.close(); env.close()
+
+
+def e2e(N, K=320, **kw):
+    """Eager steps with numpy actions in and per-env scalars out, four in flight (bench.py's e2e_obs_resident)."""
+    import time
+    import numpy as np
+    env = snakes_b200.SnakeVecEnv(N, **kw); env.reset()
+    acts = [np.random.RandomState(t).randint(0, 5, size=(N, env.S)).astype(np.int8) for t in range(8)]
+    for t in range(8):
+        env.wait_scalars(env.step_scalars_async(acts[t]))
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    tickets = []
+    for t in range(K):
+        tickets.append(env.step_scalars_async(acts[t % 8]))
+        if t >= 2:
+            env.wait_scalars(tickets[t - 2])
+    for tk in tickets[-2:]:
+        env.wait_scalars(tk)
+    torch.cuda.synchronize()
+    us = (time.perf_counter() - t0) / K * 1e6
+    report("e2e N=%d %s" % (N, kw), env, us, N)
+    env.close()
 
 
 def long_(N, warm=400, T=100, eps=0.05, **kw):
@@ -83,3 +121,7 @@ if __name__ == "__main__":
     if "1m" in which: short(1048576, T=60, reps=1, tag="1m", size=19, n_snakes=2)
     if "atari" in which: short(131072, T=40, reps=2, tag="atari84", size=19, n_snakes=2, obs_mode="atari84")
     if "rows" in which: short(32768, T=30, reps=2, tag="rows", size=64, n_snakes=16, rules="cut")
+    if "adv" in which: short(131072, tag="adv", size=19, n_snakes=2, rules="adversarial")
+    if "grid" in which: short(131072, tag="grid", size=19, n_snakes=2, obs_mode="grid")
+    if "roll" in which: roll(131072, size=19, n_snakes=2)
+    if "e2e" in which: e2e(131072, size=19, n_snakes=2)
